@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload target|c2|c3|c3_buried|c4|c5|sample] [--chains C]
     python bench.py --impl reference ...      # the CPU restatement of the reference algorithm on the host cores
+    python bench.py --dump-outputs DIR ...    # also writes the logL of the last timed step as DIR/logl.npy
 
 A step = one pass of the hot path (format_model -> propagator -> filter/FFT -> misfit -> correlated-noise
 likelihood) over one batch of `--chains` models per GPU.  `value` is measured with the models resident in HBM
@@ -57,7 +58,24 @@ def parse():
     ap.add_argument("--pt-iters", type=int, default=200, help="timed PT-MCMC iterations (0 = skip the PT leg)")
     ap.add_argument("--no-configs", action="store_true", help="skip the side workloads (configs sub-keys), sustained leg and k sweep")
     ap.add_argument("--sustain-s", type=float, default=2.5, help="seconds of back-to-back steps in the sustained leg")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path returned in its last step (logL per model, float64) as DIR/logl.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes every array as out_dir/<name>.npy.  Above DUMP_LIMIT bytes in all, each keeps the same fixed, evenly spaced
+    subset of its models, so that two runs with the same arguments still compare entry for entry."""
+    stride = -(-sum(a.nbytes for a in arrays.values()) // DUMP_LIMIT)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a[::stride])
 
 
 def workload_desc(cfg, name, chains, k_mean):
@@ -112,13 +130,15 @@ def make_inputs(cfg, chains, seed, k_fixed=None):
     return workloads.draw_models(cfg, chains, seed=seed, dvs_scale=0.3, k_fixed=k_fixed)
 
 
-def attach_obs_via_cuda(cfg, Evaluator):
-    """Observed traces = CUDA forward of the data-generating model + noise, rounded to float32 like a SAC file."""
+def attach_obs(cfg):
+    """Observed traces = forward of the data-generating model + noise, rounded to float32 like a SAC file.  The forward is
+    the C restatement's (oracle/), so the inputs of a run do not depend on the build of the library being measured."""
+    sys.path.insert(0, os.path.join(ROOT, "oracle"))
+    import oracle_c
     tm = workloads.true_model(cfg)
     cfg.obs = np.zeros((cfg.ntrc, cfg.nsmp))
     cfg.r_inv = workloads.lapack_r_inv(cfg)
-    with Evaluator(cfg) as ev:
-        _, rft, _ = ev.calc_likelihood(tm["k"], tm["z"], tm["dvp"], tm["dvs"], tm["sig"], want_rft=True)
+    _, rft, _ = oracle_c.eval_batch(cfg, tm["k"], tm["z"], tm["dvp"], tm["dvs"], tm["sig"])
     obs = rft[0, :, :cfg.nsmp] + np.random.default_rng(7).normal(0.0, 0.01, (cfg.ntrc, cfg.nsmp))
     cfg.obs = obs.astype(np.float32).astype(np.float64)
     return cfg
@@ -148,7 +168,8 @@ def cpu_sample_size(cfg, models, target_s, cap):
 
 
 def cpu_arm(cfg, models, n_sample, steps, warmup):
-    """Times the C restatement of the reference algorithm (oracle/) on all host cores: evals/s."""
+    """Times the C restatement of the reference algorithm (oracle/) on all host cores: evals/s, cores, seconds per pass and
+    the logL of the last pass."""
     sys.path.insert(0, os.path.join(ROOT, "oracle"))
     import oracle_c
     cores = host_cores()
@@ -156,10 +177,10 @@ def cpu_arm(cfg, models, n_sample, steps, warmup):
     times = []
     for i in range(warmup + steps):
         t0 = time.perf_counter()
-        oracle_c.eval_batch(cfg, sub["k"], sub["z"], sub["dvp"], sub["dvs"], sub["sig"], want_rft=False, nthreads=cores)
+        ll, _, _ = oracle_c.eval_batch(cfg, sub["k"], sub["z"], sub["dvp"], sub["dvs"], sub["sig"], want_rft=False, nthreads=cores)
         if i >= warmup:
             times.append(time.perf_counter() - t0)
-    return n_sample / float(np.mean(times)), cores, float(np.mean(times))
+    return n_sample / float(np.mean(times)), cores, float(np.mean(times)), ll
 
 
 def run_reference(args):
@@ -174,13 +195,15 @@ def run_reference(args):
     import helpers
     cfg = helpers.attach_obs_and_rinv(cfg, noise=0.01)
     cores = host_cores()
-    steps, warmup = max(1, min(args.steps, 5)), max(1, min(args.warmup, 1))
+    steps, warmup = args.steps, max(1, min(args.warmup, 1))
     models = make_inputs(cfg, min(chains, 16384), seed=100)
     # bounded sample: about 20 s of CPU work over the whole --steps/--warmup run
     n_sample = args.cpu_sample or cpu_sample_size(cfg, models, 20.0 / (steps + warmup), len(models["k"]))
     models = {k: v[:n_sample] for k, v in models.items()}
     k_mean = float(np.mean(models["k"]))
-    val, cores, sec = cpu_arm(cfg, models, n_sample, steps, warmup)
+    val, cores, sec, ll = cpu_arm(cfg, models, n_sample, steps, warmup)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"logl": ll})
     line = {"impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus, "steps": steps,
             "warmup": warmup, "ms_per_step": sec * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
             "dtype": "f64", "data": "synthetic", "config": workload_desc(cfg, args.workload, chains, k_mean),
@@ -364,10 +387,9 @@ def main():
         return float(t.item())
 
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
-    mk_eval = lambda c: Evaluator(c, device=local_rank)
 
     # ================= primary workload =================
-    cfg = attach_obs_via_cuda(workloads.make_config(args.workload), mk_eval)
+    cfg = attach_obs(workloads.make_config(args.workload))
     chains = args.chains or (FIXED_TOTAL[args.workload] // world if args.workload in FIXED_TOTAL else DEFAULT_CHAINS.get(args.workload, 4096))
     leg = Leg(torch, Evaluator, capi, cfg, chains, local_rank, seed=100 + rank)
     steps, warmup = args.steps, max(args.warmup, 3)
@@ -386,6 +408,14 @@ def main():
     clocks = sampler.stop()
     total_ms = allmax(float(np.sum(step_ms)))
     value = world * chains * steps / (total_ms * 1e-3)
+    out_logl = None
+    if args.dump_outputs:
+        # the logL every step writes into leg.logl, as the last timed step left it (the passes below write it again)
+        out_logl = leg.logl
+        if world > 1:
+            out_logl = torch.empty(world * chains, dtype=torch.float64, device=dev)
+            dist.all_gather_into_tensor(out_logl, leg.logl)
+        out_logl = out_logl.cpu().numpy()
     km = leg.kernel_split(5, flush)          # [prep + forward, quadratic form + logL] ms, separate pass
 
     # ---- end-to-end arms: host buffers through the C-ABI calls a Fortran host would make ----
@@ -511,7 +541,7 @@ def main():
         for name in SIDE_CONFIGS:
             if name == args.workload:
                 continue
-            c = attach_obs_via_cuda(workloads.make_config(name), mk_eval)
+            c = attach_obs(workloads.make_config(name))
             fixed = name in FIXED_TOTAL
             n_c = FIXED_TOTAL[name] // world if fixed else DEFAULT_CHAINS[name]
             lc = Leg(torch, Evaluator, capi, c, n_c, local_rank, seed=500 + rank)
@@ -610,10 +640,12 @@ def main():
         if world == 1 and not args.no_cpu_baseline:
             sys.path.insert(0, os.path.join(ROOT, "oracle"))
             n_sample = args.cpu_sample or cpu_sample_size(cfg, leg.models, 5.0, chains)   # ~15 s of CPU work in 3 passes
-            val, cores, sec = cpu_arm(cfg, leg.models, min(n_sample, chains), 2, 1)
+            val, cores, sec, _ = cpu_arm(cfg, leg.models, min(n_sample, chains), 2, 1)
             line["cpu_baseline"] = {"value": val, "unit": UNIT, "cores": cores, "kind": "port",
                                     "sample": f"first {min(n_sample, chains)} models of the same batch, {sec:.2f} s per pass, "
                                               "C restatement of the reference algorithm (OpenMP over models)"}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"logl": out_logl})
         print(json.dumps(line), flush=True)
     leg.close()
     if world > 1:

@@ -1,6 +1,6 @@
 """ctypes loader for the C restatement ``oracle/rfinv_oracle.c`` (TEST INFRASTRUCTURE ONLY).
 
-Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / --impl reference legs import this.
+Only tests/, __graft_entry__.smoke() and bench.py (observed traces, cpu_baseline / --impl reference legs) import this.
 """
 from __future__ import annotations
 

@@ -23,7 +23,7 @@ SMALL = {
     "three_traces_mixed": dict(ntrc=3, rayps=[0.05, 0.06, 0.11], a_gus=[2.0, 4.0, 8.0], ipha=[1, 1, -1],
                                sig_min=[0.01, 0.02, 0.03], sig_max=[0.01, 0.02, 0.03], sdep=1.5),
 }
-N_SMALL = 64
+N_SMALL = 32          # models kept per small variant: the first 32 of a 64-model draw (keeps the fixture below 1 MB)
 
 
 def variant_config(name):
@@ -35,7 +35,7 @@ def variant_config(name):
 
 def variant_models(name, cfg):
     if name != "c4":
-        return workloads.draw_models(cfg, N_SMALL, seed=3, dvs_scale=0.3)
+        return {k: v[:N_SMALL] for k, v in workloads.draw_models(cfg, 64, seed=3, dvs_scale=0.3).items()}
     # the worst-conditioned S traces of a 2048-model sample (max|rx| / maxval(rx) > 1e3) plus ordinary models
     m = workloads.draw_models(cfg, 2048, seed=21, dvs_scale=0.3)
     _, _, _, cond = oracle_c.eval_batch(cfg, m["k"], m["z"], m["dvp"], m["dvs"], m["sig"], want_cond=True)

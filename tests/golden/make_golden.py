@@ -1,8 +1,8 @@
-"""Generates tests/golden/*.npz.  Run in the build container (needs /root/reference and scipy):
+"""Generates tests/golden/sample_syn.npz and oracle_vectors.npz (needs the reference's source tree and scipy):
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py <reference>/sample_syn
 
-1. sample_syn.npz   -- the reference's own fixtures, extracted verbatim from /root/reference/sample_syn:
+1. sample_syn.npz   -- the reference's own fixtures, extracted verbatim from its sample_syn directory:
                        the two SAC traces (float32 samples + header words), true/true.velmod, model/sample.velmod
                        and the values of params.in.  These PIN the forward path (land, P, deconv_mode 0).
 2. oracle_vectors.npz -- outputs of the numpy restatement (oracle/rfinv_oracle.py) for variants the reference
@@ -17,7 +17,6 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path[:0] = [ROOT, os.path.join(ROOT, "oracle"), os.path.join(ROOT, "tests")]
-REF = "/root/reference/sample_syn"
 
 
 def read_sac(path):
@@ -37,12 +36,12 @@ def read_params(path):
     return vals
 
 
-def main():
-    s1 = read_sac(os.path.join(REF, "data/sample_1.trc"))
-    s2 = read_sac(os.path.join(REF, "data/sample_2.trc"))
-    true_vm = np.loadtxt(os.path.join(REF, "true/true.velmod"), comments="#")
-    ref_vm = np.loadtxt(os.path.join(REF, "model/sample.velmod"))
-    params = read_params(os.path.join(REF, "params.in"))
+def main(sample_syn):
+    s1 = read_sac(os.path.join(sample_syn, "data/sample_1.trc"))
+    s2 = read_sac(os.path.join(sample_syn, "data/sample_2.trc"))
+    true_vm = np.loadtxt(os.path.join(sample_syn, "true/true.velmod"), comments="#")
+    ref_vm = np.loadtxt(os.path.join(sample_syn, "model/sample.velmod"))
+    params = read_params(os.path.join(sample_syn, "params.in"))
     np.savez(os.path.join(HERE, "sample_syn.npz"),
              trc1=s1["data"], trc2=s2["data"], delta=np.float32(s1["delta"]), b=np.float32(s1["b"]), npts=s1["npts"],
              true_velmod=true_vm, ref_velmod=ref_vm, params=np.array(params))
@@ -79,4 +78,4 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1])
