@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define RFINV_ABI_VERSION 3
+#define RFINV_ABI_VERSION 4
 
 /* status codes */
 #define RFINV_OK 0
@@ -255,6 +255,20 @@ int32_t rfinv_pt_get_hist(rfinv_handle* h, int64_t* nmod, int64_t* nk, int64_t* 
                           double* vpvs_mean);
 /* Recorded models (all_models): vp_model/vs_model [n_models][nbin_z]. */
 int32_t rfinv_pt_get_models(rfinv_handle* h, int64_t max_models, double* vp_model, double* vs_model, int64_t* n_models);
+
+/* ---- checkpoint / resume (ABI version 4) ---------------------------------------------------------------------------
+ * Writes this handle's complete PT state to `path` (atomically: path + ".tmp", fsync, rename): mt19937 streams, chain state
+ * and RF buffers, swap table, counters, likelihood history and, with the bookkeeping on, histograms, means and recorded
+ * models.  Per-iteration logs are not saved.  A distributed run writes one file per process (its own virtual ranks).
+ * RFINV_ERR_STATE between rfinv_pt_local_step and rfinv_pt_apply_swap, and after rfinv_pt_reduce_outputs. */
+int32_t rfinv_pt_save(rfinv_handle* h, const char* path);
+/* Loads a state written by rfinv_pt_save into a handle on which rfinv_pt_init(h, nproc_total, rank_begin, rank_count)
+ * was called with the same arguments and no iteration has run since.  Continues at iterations_done = the saved count;
+ * the continued run is bit-identical to an uninterrupted one.  The configuration must be the one the file was written
+ * with, except that cfg.niter may be larger.  Logging is switched off (call rfinv_pt_set_logging again).
+ * RFINV_ERR_IO: unreadable, short, bad magic / version / checksum.  RFINV_ERR_ARG: other rank layout, nchains, a smaller
+ * niter, or a configuration group that differs (named in rfinv_last_error()).  RFINV_ERR_STATE: not fresh from pt_init. */
+int32_t rfinv_pt_restore(rfinv_handle* h, const char* path);
 
 /* ---- file formats either side of the path (host only, no CUDA) ---------------------------------------
  * params.in (positional, '#' comment lines; src/params.f90:101-405), SAC traces cut to [T_START, T_END]

@@ -190,6 +190,19 @@ module rfinv_b200_capi
        real(c_double), intent(out) :: out(*)
      end function rfinv_filter_traces
 
+     ! checkpoint / resume (ABI version 4): path is a NUL-terminated string, e.g. trim(fname)//c_null_char
+     integer(c_int32_t) function rfinv_pt_save(handle, path) bind(C, name="rfinv_pt_save")
+       import :: c_int32_t, c_ptr, c_char
+       type(c_ptr), value :: handle
+       character(kind=c_char), intent(in) :: path(*)
+     end function rfinv_pt_save
+
+     integer(c_int32_t) function rfinv_pt_restore(handle, path) bind(C, name="rfinv_pt_restore")
+       import :: c_int32_t, c_ptr, c_char
+       type(c_ptr), value :: handle
+       character(kind=c_char), intent(in) :: path(*)
+     end function rfinv_pt_restore
+
      function rfinv_last_error() bind(C, name="rfinv_last_error") result(msg)
        import :: c_ptr
        type(c_ptr) :: msg

@@ -13,7 +13,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 SO = os.path.join(HERE, "librfinv_b200.so")
-SOURCES = ["capi.cu", "forward.cu", "forward_general.cu", "likelihood.cu", "pt.cu", "comm.cu", "fp64_peak.cu", "host_io.cu"]
+SOURCES = ["capi.cu", "forward.cu", "forward_general.cu", "likelihood.cu", "pt.cu", "comm.cu", "checkpoint.cu", "fp64_peak.cu", "host_io.cu"]
 HEADERS = ["rfinv_common.cuh", "rfinv_handle.h", "rfinv_pt.h", os.path.join("..", "..", "include", "rfinv_b200.h")]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

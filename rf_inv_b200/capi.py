@@ -67,6 +67,8 @@ SIGNATURES = {
     "rfinv_pt_get_log": (C.c_int32, [C.c_void_p, i8p, i8p, i32p, i32p]),
     "rfinv_pt_get_hist": (C.c_int32, [C.c_void_p, i64p, i64p, i64p, i64p, i64p, i64p, i64p, i64p, dp, dp, dp]),
     "rfinv_pt_get_models": (C.c_int32, [C.c_void_p, C.c_int64, dp, dp, i64p]),
+    "rfinv_pt_save": (C.c_int32, [C.c_void_p, C.c_char_p]),
+    "rfinv_pt_restore": (C.c_int32, [C.c_void_p, C.c_char_p]),
     "rfinv_problem_load": (C.c_int32, [C.c_char_p, C.c_char_p, C.POINTER(C.c_void_p)]),
     "rfinv_problem_free": (None, [C.c_void_p]),
     "rfinv_problem_config": (C.POINTER(RfinvConfigC), [C.c_void_p]),

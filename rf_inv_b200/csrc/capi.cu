@@ -22,6 +22,12 @@ int rfinv_pdl_mode() {
   return mode;
 }
 
+int rfinv_arith_switches() {
+  auto on = [](const char* name) { return getenv(name) && atoi(getenv(name)) != 0; };
+  static const int bits = (on("RFINV_FULL_BAND") ? 1 : 0) | (on("RFINV_QF_DENSE") ? 2 : 0) | (on("RFINV_QF_NOSPLIT") ? 4 : 0);
+  return bits;
+}
+
 void rfinv_set_error(const char* fmt, ...) {
   va_list ap;
   va_start(ap, fmt);
@@ -54,7 +60,7 @@ void build_filter(const rfinv_config& c, std::vector<double>& flt) {
 // deconvolution is on (its water level is the maximum over all bins) or RFINV_FULL_BAND=1.
 void band_limits(DevConfig& d, const std::vector<double>& flt) {
   const int nh = d.nh, jfull = rfinv_forward_bins_per_thread(d.nfft_p2), nthr = (d.nfft_p2 / 2) / jfull;
-  static const bool full_band = getenv("RFINV_FULL_BAND") && atoi(getenv("RFINV_FULL_BAND")) != 0;
+  const bool full_band = (rfinv_arith_switches() & 1) != 0;
   const int allowed[6] = {1, 2, 3, 4, 6, 8};
   d.jb_max = 1;
   for (int t = 0; t < d.ntrc; ++t) {
@@ -491,8 +497,8 @@ int32_t rfinv_create(const rfinv_config* cfg, int32_t device, rfinv_handle** out
   // forward_kernel then writes (s | a) instead of m into the misfit rows (DevConfig::qf_split).
   std::vector<double> wfac;
   {
-    static const bool force_dense = getenv("RFINV_QF_DENSE") && atoi(getenv("RFINV_QF_DENSE")) != 0;
-    static const bool no_split = getenv("RFINV_QF_NOSPLIT") && atoi(getenv("RFINV_QF_NOSPLIT")) != 0;
+    const bool force_dense = (rfinv_arith_switches() & 2) != 0;
+    const bool no_split = (rfinv_arith_switches() & 4) != 0;
     const int ntile_dense = Sp / 64;
     std::vector<std::vector<double>> Wt(T);      // per trace: [wrows_t][Sp], row = one column of W, K contiguous
     std::vector<int> wrows_t(T, 0);

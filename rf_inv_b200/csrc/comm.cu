@@ -219,6 +219,7 @@ int32_t rfinv_comm_info(rfinv_handle* h, int32_t* world, int32_t* rank, int32_t*
 // recorded models of every process in process order (rfinv_pt_get_models).  Collective; call once, after the last iteration.
 int32_t rfinv_pt_reduce_outputs(rfinv_handle* h) {
   if (!h || !h->pt) { rfinv_set_error("rfinv_pt_reduce_outputs: call rfinv_pt_init first"); return RFINV_ERR_STATE; }
+  h->pt->reduced = true;
   if (!h->comm || h->comm_world == 1) return RFINV_OK;   // a single process already holds the job-wide sums
   NcclApi* api = nccl_api();
   PtState* s = h->pt;

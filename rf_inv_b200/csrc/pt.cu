@@ -1224,7 +1224,9 @@ int32_t rfinv_pt_local_step(rfinv_handle* h) {
   if (st != RFINV_OK) return st;
   RFINV_CUDA_CHECK(cudaSetDevice(h->device));
   if ((st = pt_reserve_lhist(h, h->pt->it_done + 1)) != RFINV_OK) return st;
-  return pt_enqueue_local(h, pt_records(h->pt));
+  if ((st = pt_enqueue_local(h, pt_records(h->pt))) != RFINV_OK) return st;
+  h->pt->step_pending = true;
+  return RFINV_OK;
 }
 
 int32_t rfinv_pt_swap_table(rfinv_handle* h, uint64_t* dev_ptr, int32_t* n_doubles) {
@@ -1247,6 +1249,7 @@ int32_t rfinv_pt_apply_swap(rfinv_handle* h, uint64_t gathered_dev_ptr, int32_t 
   pt_swap_kernel<<<1, 32, 0, h->stream>>>(s->dev, reinterpret_cast<const double*>(gathered_dev_ptr), world, s->table_len);
   RFINV_CUDA_CHECK(cudaGetLastError());
   s->it_done++;
+  s->step_pending = false;
   return RFINV_OK;
 }
 
@@ -1481,3 +1484,5 @@ int32_t rfinv_pt_get_log(rfinv_handle* h, int8_t* flags, int8_t* itypes, int32_t
 }
 
 }  // extern "C"
+
+int rfinv_pt_reserve_lhist(rfinv_handle* h, int upto) { return pt_reserve_lhist(h, upto); }

@@ -79,3 +79,8 @@ int rfinv_comm_peer_setup(rfinv_handle* h);
 void rfinv_comm_peer_release(rfinv_handle* h);
 // pt.cu: after the job-wide sum, the bins whose means the reference assigns go back to the assigned value
 int rfinv_pt_fix_assigned_bins(rfinv_handle* h);
+// pt.cu: room in the likelihood history for iterations [0, upto)
+int rfinv_pt_reserve_lhist(rfinv_handle* h, int upto);
+// capi.cu: the environment switches that change the arithmetic, as read once per process: bit 0 RFINV_FULL_BAND, bit 1
+// RFINV_QF_DENSE, bit 2 RFINV_QF_NOSPLIT
+int rfinv_arith_switches();

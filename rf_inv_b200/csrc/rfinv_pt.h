@@ -104,4 +104,6 @@ struct PtState {
   int log_cap = 0, log_base = 0;
   long long n_eval = 0;
   bool record = false;
+  bool step_pending = false;   // rfinv_pt_local_step has run, rfinv_pt_apply_swap not yet: no checkpoint in between
+  bool reduced = false;        // rfinv_pt_reduce_outputs has run: the bookkeeping may hold job-wide sums
 };

@@ -8,6 +8,7 @@ all-gather (NCCL over NVLink on GPUs); every process then evaluates the same swa
 from __future__ import annotations
 
 import ctypes as C
+import os
 from typing import Dict, Optional
 
 import numpy as np
@@ -104,6 +105,18 @@ class ParallelTempering:
         """output_results' mpi_reduce / mpi_gather (src/mcmc_out.f90:52-93): afterwards process 0's hist() / counters() / models()
         are job-wide.  Collective; call once after the last iteration."""
         capi.check(self._lib.rfinv_pt_reduce_outputs(self.ev.handle))
+
+    # -- checkpoint / resume ----------------------------------------------------------------------
+    def save(self, path) -> None:
+        """Writes this process's complete PT state to `path` (atomically).  Not between local_step and the swap, and not
+        after reduce_outputs()."""
+        capi.check(self._lib.rfinv_pt_save(self.ev.handle, os.fsencode(path)))
+
+    def restore(self, path) -> None:
+        """Loads a state written by save() into this freshly initialised object (same configuration -- niter may be larger --
+        and the same nproc_total / world / rank).  The run continues at the saved iteration, bit-identical to an
+        uninterrupted run.  Logging is switched off: call set_logging() again."""
+        capi.check(self._lib.rfinv_pt_restore(self.ev.handle, os.fsencode(path)))
 
     # -- results ----------------------------------------------------------------------------------
     def set_logging(self, cap_iters: int) -> None:
