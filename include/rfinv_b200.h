@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define RFINV_ABI_VERSION 4
+#define RFINV_ABI_VERSION 5
 
 /* status codes */
 #define RFINV_OK 0
@@ -269,6 +269,24 @@ int32_t rfinv_pt_save(rfinv_handle* h, const char* path);
  * RFINV_ERR_IO: unreadable, short, bad magic / version / checksum.  RFINV_ERR_ARG: other rank layout, nchains, a smaller
  * niter, or a configuration group that differs (named in rfinv_last_error()).  RFINV_ERR_STATE: not fresh from pt_init. */
 int32_t rfinv_pt_restore(rfinv_handle* h, const char* path);
+
+/* ---- several runs advanced together on one GPU (ABI version 5) -------------------------------------------------------
+ * A study inverts many stations, each an independent PT run of its own handle.  A group advances n such handles by one
+ * iteration in ONE graph launch with n parallel branches, so the small kernels of many runs share the GPU instead of taking
+ * turns.  Members stay ordinary handles: rfinv_pt_get_*, rfinv_pt_set_logging, rfinv_pt_save / _restore and a solo rfinv_pt_run
+ * keep working between group runs.  A group iteration lasts as long as its slowest member's. */
+typedef struct rfinv_pt_group rfinv_pt_group;
+/* n >= 1 distinct handles on the same device, each after rfinv_pt_init as a single process (rank_count == nproc_total).  The
+ * handles must outlive the group.  RFINV_ERR_ARG: NULL or duplicate handles, members on different devices; RFINV_ERR_STATE:
+ * a member without rfinv_pt_init or with a distributed layout.  The message names the member index. */
+int32_t rfinv_pt_group_create(rfinv_handle* const* handles, int32_t n, rfinv_pt_group** out);
+/* n_iter iterations of every member, as if each had called rfinv_pt_run(member, n_iter): every member ends with the same bits
+ * (state, RF buffers, counters, likelihood history, histograms, recorded models, logs; the profile means are summed with fp64
+ * atomics and agree to rounding).  Synchronous.  RFINV_ERR_STATE, naming the member, when the members differ in nburn, ncorr
+ * or iterations done, or a member is between rfinv_pt_local_step and rfinv_pt_apply_swap or after rfinv_pt_reduce_outputs. */
+int32_t rfinv_pt_group_run(rfinv_pt_group* g, int32_t n_iter);
+/* Frees the group; the member handles are untouched. */
+void rfinv_pt_group_destroy(rfinv_pt_group* g);
 
 /* ---- file formats either side of the path (host only, no CUDA) ---------------------------------------
  * params.in (positional, '#' comment lines; src/params.f90:101-405), SAC traces cut to [T_START, T_END]

@@ -203,6 +203,25 @@ module rfinv_b200_capi
        character(kind=c_char), intent(in) :: path(*)
      end function rfinv_pt_restore
 
+     ! several stations advanced together (ABI version 5): handles(n) are the c_ptr of n handles after rfinv_pt_init
+     integer(c_int32_t) function rfinv_pt_group_create(handles, n, group) bind(C, name="rfinv_pt_group_create")
+       import :: c_int32_t, c_ptr
+       type(c_ptr), intent(in) :: handles(*)
+       integer(c_int32_t), value :: n
+       type(c_ptr), intent(out) :: group
+     end function rfinv_pt_group_create
+
+     integer(c_int32_t) function rfinv_pt_group_run(group, n_iter) bind(C, name="rfinv_pt_group_run")
+       import :: c_int32_t, c_ptr
+       type(c_ptr), value :: group
+       integer(c_int32_t), value :: n_iter
+     end function rfinv_pt_group_run
+
+     subroutine rfinv_pt_group_destroy(group) bind(C, name="rfinv_pt_group_destroy")
+       import :: c_ptr
+       type(c_ptr), value :: group
+     end subroutine rfinv_pt_group_destroy
+
      function rfinv_last_error() bind(C, name="rfinv_last_error") result(msg)
        import :: c_ptr
        type(c_ptr) :: msg

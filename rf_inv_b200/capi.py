@@ -69,6 +69,9 @@ SIGNATURES = {
     "rfinv_pt_get_models": (C.c_int32, [C.c_void_p, C.c_int64, dp, dp, i64p]),
     "rfinv_pt_save": (C.c_int32, [C.c_void_p, C.c_char_p]),
     "rfinv_pt_restore": (C.c_int32, [C.c_void_p, C.c_char_p]),
+    "rfinv_pt_group_create": (C.c_int32, [C.POINTER(C.c_void_p), C.c_int32, C.POINTER(C.c_void_p)]),
+    "rfinv_pt_group_run": (C.c_int32, [C.c_void_p, C.c_int32]),
+    "rfinv_pt_group_destroy": (None, [C.c_void_p]),
     "rfinv_problem_load": (C.c_int32, [C.c_char_p, C.c_char_p, C.POINTER(C.c_void_p)]),
     "rfinv_problem_free": (None, [C.c_void_p]),
     "rfinv_problem_config": (C.POINTER(RfinvConfigC), [C.c_void_p]),

@@ -1594,7 +1594,7 @@ int launch_forward_t(const DevConfig& cfg, const ModelBatch& mb, const EvalOutpu
   static const size_t extra = getenv("RFINV_FWD_EXTRA_SMEM") ? (size_t)atoi(getenv("RFINV_FWD_EXTRA_SMEM")) : 0;  // occupancy experiments
   const size_t smem = forward_smem_bytes(cfg, nthr) + extra;
   if (nthr != BMAX) { rfinv_set_error("forward_kernel<%d,%d>: launched with %d threads", J, BMAX, nthr); return RFINV_ERR_ARG; }
-  RFINV_CUDA_CHECK(cudaFuncSetAttribute(forward_kernel<J, BMAX, MINB, MIXED, BURIED, GEN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  RFINV_CUDA_CHECK(rfinv_raise_smem_limit((const void*)forward_kernel<J, BMAX, MINB, MIXED, BURIED, GEN>, smem));
   int dev = 0, n_sm = 0, per_sm = 0;
   RFINV_CUDA_CHECK(cudaGetDevice(&dev));
   RFINV_CUDA_CHECK(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev));
@@ -1698,7 +1698,7 @@ int rfinv_launch_prep(const DevConfig& cfg, const ModelBatch& mb, uint8_t* is_va
   const size_t prep_smem = sizeof(double) * (prep_smem_model_doubles(cfg.k_max) + (size_t)rays_per_cta * prep_smem_ray_doubles(cfg.k_max));
 #define PREP(BUR, HOST)                                                                                                    \
   do {                                                                                                                     \
-    RFINV_CUDA_CHECK(cudaFuncSetAttribute(prep_kernel<BUR, HOST>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prep_smem)); \
+    RFINV_CUDA_CHECK(rfinv_raise_smem_limit((const void*)prep_kernel<BUR, HOST>, prep_smem));                                \
     prep_kernel<BUR, HOST><<<(unsigned)m_count * n_groups, 32 * rays_per_cta, prep_smem, stream>>>(cfg, mb, lc, rc, is_valid, counter, m_begin + m_count, ntr_eff, nthr, rays_per_cta, m_begin); \
   } while (0)
   if (cfg.bdep > 0.0) { if (mb.chain_major) PREP(true, true); else PREP(true, false); }
@@ -1748,10 +1748,10 @@ int rfinv_launch_filter_traces(const DevConfig& cfg, int n_series, const double*
   const size_t smem = sizeof(double2) * (2 * fft_buf_elems(cfg.fft_len) + (cfg.fft_general ? 0 : fft_twiddle_entries(cfg.fft_len))) + sizeof(double) * 64;
   const int nthr = cfg.fft_len / 8 < 32 ? 32 : (cfg.fft_len / 8 > 128 ? 128 : cfg.fft_len / 8);
   if (cfg.fft_general) {
-    RFINV_CUDA_CHECK(cudaFuncSetAttribute(filter_traces_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    RFINV_CUDA_CHECK(rfinv_raise_smem_limit((const void*)filter_traces_kernel<true>, smem));
     filter_traces_kernel<true><<<n_series, nthr, smem, stream>>>(cfg, in, trace_of, out);
   } else {
-    RFINV_CUDA_CHECK(cudaFuncSetAttribute(filter_traces_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    RFINV_CUDA_CHECK(rfinv_raise_smem_limit((const void*)filter_traces_kernel<false>, smem));
     filter_traces_kernel<false><<<n_series, nthr, smem, stream>>>(cfg, in, trace_of, out);
   }
   RFINV_CUDA_CHECK(cudaGetLastError());

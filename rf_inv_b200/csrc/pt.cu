@@ -955,9 +955,15 @@ int rfinv_pt_fix_assigned_bins(rfinv_handle* h) {
   return RFINV_OK;
 }
 
+// drops the captured iterations: something baked into their launches changed.  A new generation tells the groups the handle
+// is in (rfinv_pt_group_run) to capture theirs again.
+static void pt_drop_graphs(PtState* s) {
+  for (cudaGraphExec_t& g : s->graph) { if (g) cudaGraphExecDestroy(g); g = nullptr; }
+  s->generation = rfinv_pt_next_generation();
+}
+
 void rfinv_handle::invalidate_pt_graphs() {
-  if (!pt) return;
-  for (cudaGraphExec_t& g : pt->graph) { if (g) cudaGraphExecDestroy(g); g = nullptr; }
+  if (pt) pt_drop_graphs(pt);
 }
 
 void rfinv_handle::free_pt() {
@@ -1116,10 +1122,6 @@ int32_t rfinv_pt_draw(rfinv_handle* h, int32_t local_rank, int32_t kind, int32_t
 
 int32_t rfinv_pt_ntype(rfinv_handle* h) { return (h && h->pt) ? h->pt->dev.ntype : -1; }
 
-static void pt_drop_graphs(PtState* s) {
-  for (cudaGraphExec_t& g : s->graph) { if (g) cudaGraphExecDestroy(g); g = nullptr; }
-}
-
 int32_t rfinv_pt_set_logging(rfinv_handle* h, int32_t cap_iters) {
   int st = pt_require(h, "rfinv_pt_set_logging");
   if (st != RFINV_OK) return st;
@@ -1178,9 +1180,9 @@ static int pt_enqueue_local(rfinv_handle* h, bool record, bool peer_exchange = f
     const size_t per_warp = sizeof(double) * pt_propose_smem_doubles(h->dc.k_max, h->dc.ntrc, d.nchains);
     if (per_warp <= 48 * 1024) {
       const int warps = per_warp <= 12 * 1024 ? 4 : (per_warp <= 24 * 1024 ? 2 : 1);
-      RFINV_CUDA_CHECK(cudaFuncSetAttribute(pt_propose_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(per_warp * warps)));
+      RFINV_CUDA_CHECK(rfinv_raise_smem_limit((const void*)pt_propose_kernel<true, false>, per_warp * warps));
       const bool peer = s->peer_state == 1 && peer_exchange;
-      RFINV_CUDA_CHECK(cudaFuncSetAttribute(pt_propose_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(per_warp * warps)));
+      RFINV_CUDA_CHECK(rfinv_raise_smem_limit((const void*)pt_propose_kernel<true, true>, per_warp * warps));
       if (peer) pt_propose_kernel<true, true><<<(d.G + warps - 1) / warps, 32 * warps, per_warp * warps, q>>>(h->dc, d, s->d_table, s->peers);
       else pt_propose_kernel<true, false><<<(d.G + warps - 1) / warps, 32 * warps, per_warp * warps, q>>>(h->dc, d, s->d_table, s->peers);
     } else {
@@ -1272,6 +1274,12 @@ static int pt_enqueue_iteration(rfinv_handle* h, int world, bool record) {
   return RFINV_OK;
 }
 
+// RFINV_PT_GRAPH=0: plain launches instead of replaying captured iterations
+static bool pt_use_graph() {
+  static const bool use = !(getenv("RFINV_PT_GRAPH") && atoi(getenv("RFINV_PT_GRAPH")) == 0);
+  return use;
+}
+
 // pt_control's loop (src/pt_mcmc.f90:488-572) for n_iter iterations over `world` processes.  The launch sequence of an
 // iteration -- five kernels; with several processes also the two kernels of the peer-memory exchange on a side branch, or one
 // ncclAllGather and the swap kernel -- is captured once per variant (with / without the bookkeeping kernels) in a CUDA graph and
@@ -1302,7 +1310,7 @@ static int pt_iterate(rfinv_handle* h, int n_iter, int world) {
     RFINV_CUDA_CHECK(cudaStreamCreateWithFlags(&s->side_stream, cudaStreamNonBlocking));
     for (cudaEvent_t& e : s->ev_side) RFINV_CUDA_CHECK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
   }
-  static const bool use_graph = !(getenv("RFINV_PT_GRAPH") && atoi(getenv("RFINV_PT_GRAPH")) == 0);
+  const bool use_graph = pt_use_graph();
   if (s->graph_world != world) { pt_drop_graphs(s); s->graph_world = world; }
   for (int it = 0; it < n_iter; ++it) {
     const bool record = pt_records(s);
@@ -1486,3 +1494,178 @@ int32_t rfinv_pt_get_log(rfinv_handle* h, int8_t* flags, int8_t* itypes, int32_t
 }  // extern "C"
 
 int rfinv_pt_reserve_lhist(rfinv_handle* h, int upto) { return pt_reserve_lhist(h, upto); }
+
+// ---------------- several single-process runs advanced together (rfinv_pt_group_*) ----------------
+// One iteration of every member is ONE graph: the group's stream forks to the members' capture streams, each member's own
+// launch sequence (pt_enqueue_iteration) is captured on its branch, and the branches join again.  The members' kernels then
+// run side by side, so many small runs fill the GPU that one of them leaves mostly idle.  Variant [0]: nobody records the
+// posterior bookkeeping in this iteration, [1]: the members with the bookkeeping on record (equal nburn / ncorr /
+// iterations_done make that decision the same for all of them).
+struct rfinv_pt_group {
+  std::vector<rfinv_handle*> h;
+  int device = 0;
+  cudaStream_t stream = nullptr;
+  cudaEvent_t fork = nullptr;
+  std::vector<cudaEvent_t> join;
+  cudaGraphExec_t graph[2] = {nullptr, nullptr};
+  // per member: the PtState and its generation the graphs were captured with (a new one, or a new generation, means the
+  // member's buffers may have moved: capture again)
+  std::vector<PtState*> cap_state;
+  std::vector<uint64_t> cap_gen;
+};
+
+static void group_drop_graphs(rfinv_pt_group* g) {
+  for (cudaGraphExec_t& e : g->graph) { if (e) cudaGraphExecDestroy(e); e = nullptr; }
+}
+
+// the members' iterations of variant `v` as one fork-join graph on the group's stream
+static int group_capture(rfinv_pt_group* g, cudaGraphExec_t* out) {
+  const int n = (int)g->h.size();
+  for (rfinv_handle* h : g->h)   // (created outside the capture)
+    if (!h->pt->capture_stream) RFINV_CUDA_CHECK(cudaStreamCreateWithFlags(&h->pt->capture_stream, cudaStreamNonBlocking));
+  cudaGraph_t graph = nullptr;
+  cudaError_t e = cudaStreamBeginCapture(g->stream, cudaStreamCaptureModeThreadLocal);
+  if (e != cudaSuccess) { rfinv_set_error("rfinv_pt_group_run: cudaStreamBeginCapture: %s", cudaGetErrorString(e)); return RFINV_ERR_CUDA; }
+  int st = RFINV_OK;
+  e = cudaEventRecord(g->fork, g->stream);
+  for (int i = 0; i < n && e == cudaSuccess && st == RFINV_OK; ++i) {
+    rfinv_handle* h = g->h[i];
+    PtState* s = h->pt;
+    e = cudaStreamWaitEvent(s->capture_stream, g->fork, 0);
+    if (e != cudaSuccess) break;
+    cudaStream_t user_stream = h->stream;   // the member's launch code enqueues on h->stream: its branch of the capture
+    h->stream = s->capture_stream;
+    st = pt_enqueue_iteration(h, 1, pt_records(s));
+    h->stream = user_stream;
+    if (st != RFINV_OK) break;
+    e = cudaEventRecord(g->join[i], s->capture_stream);
+    if (e == cudaSuccess) e = cudaStreamWaitEvent(g->stream, g->join[i], 0);
+  }
+  const cudaError_t e_end = cudaStreamEndCapture(g->stream, &graph);
+  if (st != RFINV_OK) { if (graph) cudaGraphDestroy(graph); return st; }
+  if (e == cudaSuccess) e = e_end;
+  if (e != cudaSuccess) {
+    if (graph) cudaGraphDestroy(graph);
+    rfinv_set_error("rfinv_pt_group_run: capture of the group's iteration: %s", cudaGetErrorString(e));
+    return RFINV_ERR_CUDA;
+  }
+  e = cudaGraphInstantiate(out, graph, 0);
+  cudaGraphDestroy(graph);
+  if (e != cudaSuccess) { *out = nullptr; rfinv_set_error("rfinv_pt_group_run: cudaGraphInstantiate: %s", cudaGetErrorString(e)); return RFINV_ERR_CUDA; }
+  return RFINV_OK;
+}
+
+extern "C" {
+
+int32_t rfinv_pt_group_create(rfinv_handle* const* handles, int32_t n, rfinv_pt_group** out) {
+  static const char* who = "rfinv_pt_group_create";
+  if (!out) { rfinv_set_error("%s: out is NULL", who); return RFINV_ERR_ARG; }
+  *out = nullptr;
+  if (!handles || n < 1) { rfinv_set_error("%s: need at least one handle (n = %d)", who, n); return RFINV_ERR_ARG; }
+  for (int i = 0; i < n; ++i) {
+    rfinv_handle* h = handles[i];
+    if (!h) { rfinv_set_error("%s: member %d is NULL", who, i); return RFINV_ERR_ARG; }
+    for (int j = 0; j < i; ++j)
+      if (handles[j] == h) { rfinv_set_error("%s: member %d is the same handle as member %d", who, i, j); return RFINV_ERR_ARG; }
+    if (!h->pt) { rfinv_set_error("%s: member %d: call rfinv_pt_init first", who, i); return RFINV_ERR_STATE; }
+    if (h->pt->dev.G != h->pt->dev.nproc_total) {
+      rfinv_set_error("%s: member %d holds %d of %d ranks (a distributed layout); a group advances single-process runs", who, i,
+                      h->pt->dev.G, h->pt->dev.nproc_total);
+      return RFINV_ERR_STATE;
+    }
+    if (h->device != handles[0]->device) {
+      rfinv_set_error("%s: member %d is on device %d, member 0 on device %d", who, i, h->device, handles[0]->device);
+      return RFINV_ERR_ARG;
+    }
+  }
+  RFINV_CUDA_CHECK(cudaSetDevice(handles[0]->device));
+  rfinv_pt_group* g = new rfinv_pt_group();
+  g->h.assign(handles, handles + n);
+  g->device = handles[0]->device;
+  g->join.assign(n, nullptr);
+  g->cap_state.assign(n, nullptr);
+  g->cap_gen.assign(n, 0);
+  cudaError_t e = cudaStreamCreateWithFlags(&g->stream, cudaStreamNonBlocking);
+  if (e == cudaSuccess) e = cudaEventCreateWithFlags(&g->fork, cudaEventDisableTiming);
+  for (int i = 0; i < n && e == cudaSuccess; ++i) e = cudaEventCreateWithFlags(&g->join[i], cudaEventDisableTiming);
+  if (e != cudaSuccess) {
+    rfinv_set_error("%s: %s", who, cudaGetErrorString(e));
+    rfinv_pt_group_destroy(g);
+    return RFINV_ERR_CUDA;
+  }
+  *out = g;
+  return RFINV_OK;
+}
+
+int32_t rfinv_pt_group_run(rfinv_pt_group* g, int32_t n_iter) {
+  static const char* who = "rfinv_pt_group_run";
+  if (!g) { rfinv_set_error("%s: group is NULL", who); return RFINV_ERR_ARG; }
+  if (n_iter < 0) { rfinv_set_error("%s: n_iter = %d", who, n_iter); return RFINV_ERR_ARG; }
+  const int n = (int)g->h.size();
+  for (int i = 0; i < n; ++i) {
+    rfinv_handle* h = g->h[i];
+    const PtState* s = h->pt;
+    if (!s) { rfinv_set_error("%s: member %d: call rfinv_pt_init first", who, i); return RFINV_ERR_STATE; }
+    if (s->dev.G != s->dev.nproc_total) {
+      rfinv_set_error("%s: member %d holds %d of %d ranks (a distributed layout)", who, i, s->dev.G, s->dev.nproc_total);
+      return RFINV_ERR_STATE;
+    }
+    if (s->step_pending) {
+      rfinv_set_error("%s: member %d is between rfinv_pt_local_step and rfinv_pt_apply_swap", who, i);
+      return RFINV_ERR_STATE;
+    }
+    if (s->reduced) { rfinv_set_error("%s: member %d: rfinv_pt_reduce_outputs has run", who, i); return RFINV_ERR_STATE; }
+    const PtState* s0 = g->h[0]->pt;
+    if (s->dev.nburn != s0->dev.nburn || s->dev.ncorr != s0->dev.ncorr || s->it_done != s0->it_done) {
+      rfinv_set_error("%s: member %d has nburn %d, ncorr %d and %d iterations done, member 0 has %d, %d and %d: the members must "
+                      "agree on all three", who, i, s->dev.nburn, s->dev.ncorr, s->it_done, s0->dev.nburn, s0->dev.ncorr, s0->it_done);
+      return RFINV_ERR_STATE;
+    }
+  }
+  if (n_iter == 0) return RFINV_OK;
+  int st;
+  RFINV_CUDA_CHECK(cudaSetDevice(g->device));
+  for (rfinv_handle* h : g->h) {
+    RFINV_CUDA_CHECK(cudaStreamSynchronize(h->stream));   // the caller may have queued work on the member's own stream
+    if ((st = pt_reserve_lhist(h, h->pt->it_done + n_iter)) != RFINV_OK) return st;
+  }
+  const bool use_graph = pt_use_graph();
+  if (use_graph) {
+    bool stale = false;
+    for (int i = 0; i < n; ++i) stale = stale || g->cap_state[i] != g->h[i]->pt || g->cap_gen[i] != g->h[i]->pt->generation;
+    if (stale) {
+      group_drop_graphs(g);
+      for (int i = 0; i < n; ++i) { g->cap_state[i] = g->h[i]->pt; g->cap_gen[i] = g->h[i]->pt->generation; }
+    }
+  }
+  for (int it = 0; it < n_iter; ++it) {
+    const PtState* s0 = g->h[0]->pt;
+    const int next = s0->it_done + 1;   // pt_records without a member's bookkeeping switch
+    const int variant = next > s0->dev.nburn && next % s0->dev.ncorr == 0 ? 1 : 0;
+    if (use_graph) {
+      cudaGraphExec_t& ge = g->graph[variant];
+      if (!ge && (st = group_capture(g, &ge)) != RFINV_OK) return st;
+      RFINV_CUDA_CHECK(cudaGraphLaunch(ge, g->stream));
+    } else {
+      for (rfinv_handle* h : g->h)   // round robin over the members' own streams
+        if ((st = pt_enqueue_iteration(h, 1, pt_records(h->pt))) != RFINV_OK) return st;
+    }
+    for (rfinv_handle* h : g->h) h->pt->it_done++;
+  }
+  if (use_graph) RFINV_CUDA_CHECK(cudaStreamSynchronize(g->stream));
+  else for (rfinv_handle* h : g->h) RFINV_CUDA_CHECK(cudaStreamSynchronize(h->stream));
+  return RFINV_OK;
+}
+
+void rfinv_pt_group_destroy(rfinv_pt_group* g) {
+  if (!g) return;
+  cudaSetDevice(g->device);
+  if (g->stream) cudaStreamSynchronize(g->stream);
+  group_drop_graphs(g);
+  for (cudaEvent_t e : g->join) if (e) cudaEventDestroy(e);
+  if (g->fork) cudaEventDestroy(g->fork);
+  if (g->stream) cudaStreamDestroy(g->stream);
+  delete g;
+}
+
+}  // extern "C"

@@ -3,6 +3,9 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <math.h>
+#include <map>
+#include <mutex>
+#include <utility>
 #include "../../include/rfinv_b200.h"
 
 #define RFINV_MAX_TRC 16     // traces per model (kernel parameter arrays)
@@ -110,6 +113,23 @@ __device__ __forceinline__ bool layer_velocity(const DevConfig& cfg, double zc, 
   } while (0)
 
 void rfinv_set_error(const char* fmt, ...);
+
+// cudaFuncAttributeMaxDynamicSharedMemorySize of `kernel` on the current device raised to at least `bytes`, never lowered.  The
+// attribute is process-wide per kernel while the size a launch needs depends on the handle's shape (nfft, k_max, ntrc, nchains):
+// a handle of another shape that set a smaller value would invalidate the launches another handle has captured in a graph.
+inline cudaError_t rfinv_raise_smem_limit(const void* kernel, size_t bytes) {
+  static std::mutex mu;
+  static std::map<std::pair<int, const void*>, size_t> limit;   // (device, kernel) -> largest value set
+  int dev = 0;
+  cudaError_t e = cudaGetDevice(&dev);
+  if (e != cudaSuccess) return e;
+  std::lock_guard<std::mutex> lock(mu);
+  size_t& cur = limit[{dev, kernel}];
+  if (bytes <= cur) return cudaSuccess;
+  e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+  if (e == cudaSuccess) cur = bytes;
+  return e;
+}
 
 // Programmatic dependent launch (sm_90+): a kernel launched with rfinv_launch_pdl may start while the kernel before it on the
 // stream is still draining -- its CTAs take the SM slots the predecessor's last CTAs free, run their prologue, and block in

@@ -1,5 +1,6 @@
 // Device-resident parallel-tempering state (pt.cu).
 #pragma once
+#include <atomic>
 #include "rfinv_common.cuh"
 
 // Passed to the PT kernels by value.  Arrays are chain-fastest: x[i*Cl + c].
@@ -78,12 +79,19 @@ struct PtPeers {
 // words of 8 bytes behind the gather buffer
 inline size_t pt_peer_tail_words(int world) { return (size_t)world + 2 + 8; }
 
+// unique over the process: a PtState that rfinv_pt_init creates again at the same address still gets a new generation
+inline uint64_t rfinv_pt_next_generation() {
+  static std::atomic<uint64_t> n{0};
+  return ++n;
+}
+
 struct PtState {
   PtDev dev;
   int it_done = 0;
   // one iteration as a CUDA graph: [0] plain, [1] with the posterior bookkeeping kernels (every ncorr-th iteration after
   // the burn-in); invalidated when something that is baked into the launches changes (logging, capacity)
   cudaGraphExec_t graph[2] = {nullptr, nullptr};
+  uint64_t generation = rfinv_pt_next_generation();   // renewed whenever the graphs are dropped (groups capture again)
   int graph_world = 0;
   cudaStream_t capture_stream = nullptr;
   cudaStream_t side_stream = nullptr;      // side branch of the iteration (peer-memory exchange)

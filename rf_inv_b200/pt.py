@@ -175,6 +175,45 @@ class ParallelTempering:
         return flags[:n.value], itypes[:n.value], swaps[:n.value]
 
 
+class PtGroup:
+    """Several single-process runs (one per station) advanced together on one GPU: ``PtGroup([pt_a, pt_b, ...]).run(n)``
+    leaves every member with the bits ``member.run(n)`` alone would give, in one graph launch per iteration for all of them
+    (rfinv_pt_group_run).  The members stay usable on their own between group runs."""
+
+    def __init__(self, pts):
+        self._g = None
+        self.pts = list(pts)                          # keeps the handles alive as long as the group
+        if not self.pts:
+            raise ValueError("a group needs at least one ParallelTempering")
+        self._lib = self.pts[0]._lib
+        handles = (C.c_void_p * len(self.pts))(*[p.ev.handle for p in self.pts])
+        g = C.c_void_p()
+        capi.check(self._lib.rfinv_pt_group_create(C.cast(handles, C.POINTER(C.c_void_p)), len(self.pts), C.byref(g)))
+        self._g = g
+
+    def run(self, n_iter: int) -> None:
+        if self._g is None:
+            raise RuntimeError("the group is closed")
+        capi.check(self._lib.rfinv_pt_group_run(self._g, int(n_iter)))
+
+    def close(self) -> None:
+        if self._g is not None:
+            self._lib.rfinv_pt_group_destroy(self._g)
+            self._g = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
 def build_table(temps, logl, peeks, pair=(-1, -1)) -> np.ndarray:
     """Host-side layout of one process's swap table (what pt_finish_kernel / pt_propose_kernel write)."""
     return np.concatenate([np.asarray(temps, dtype=np.float64), np.asarray(logl, dtype=np.float64),

@@ -7,7 +7,13 @@ into OUT_DIR.
 
 ``--checkpoint PATH`` saves the complete chain state as the run goes (under torchrun one file per process,
 ``PATH.<rank>-of-<world>``); ``--resume`` continues from it if it exists, so the same command can be resubmitted after an
-interruption, or with a larger N_ITER in params.in.  A resumed run writes exactly the files an uninterrupted run writes."""
+interruption, or with a larger N_ITER in params.in.  A resumed run writes exactly the files an uninterrupted run writes.
+
+Several params files (``python -m rf_inv_b200.run a/params.in b/params.in ... --nproc N``), one per station, run side by
+side on one GPU as one group (rfinv_pt_group_run): every station writes into its own OUT_DIR exactly the files a run of its
+params file alone writes.  The stations must agree on N_BURN, N_ITER and N_CORR and write to different OUT_DIRs.  Station i
+(its position on the command line) checkpoints to ``PATH.<i>``.  Under torchrun process r runs the stations i with
+i % world == r as its group on its own GPU; the processes do not communicate."""
 from __future__ import annotations
 
 import argparse
@@ -18,12 +24,25 @@ import numpy as np
 
 from . import io as rio
 from . import workloads
-from .pt import ParallelTempering
+from .pt import ParallelTempering, PtGroup
 
 
 def checkpoint_path(path: str, world: int, rank: int) -> str:
     """The file of this process: `path` itself for one process, `path.<rank>-of-<world>` under torchrun."""
     return path if world == 1 else f"{path}.{rank}-of-{world}"
+
+
+def print_summary(cfg, hist, cnt) -> None:
+    """The acceptance summary of src/mcmc_out.f90:99-107."""
+    labels = ["Birth proposal", "Death proposal", "Moving interface depth proposal", "Perturbing dVs proposal"]
+    if cfg.vp_mode == 1:
+        labels.append("Perturbing dVs proposal")  # sic: the reference labels the dVp proposal like this (pt_mcmc.f90:386)
+    if any(cfg.sig_mode):
+        labels.append("Perturbing sigma proposal")
+    print(" --- Summary ---")
+    print(f" # of sampled models: {hist['nmod']}")
+    for lab, a, n in zip(labels, cnt["naccept"], cnt["nprop"]):
+        print(f" # of {lab}: {int(a)} / {int(n)}")
 
 
 def run(params_path: str, nproc: int, verbose: bool = True, n_iter: int = None, checkpoint: str = None,
@@ -88,16 +107,8 @@ def run(params_path: str, nproc: int, verbose: bool = True, n_iter: int = None, 
     vp_model, vs_model = pt.models()
     lh = cnt["likelihood_hist"]
     if rank == 0:
-        if verbose:                                       # summary, src/mcmc_out.f90:99-107
-            labels = ["Birth proposal", "Death proposal", "Moving interface depth proposal", "Perturbing dVs proposal"]
-            if cfg.vp_mode == 1:
-                labels.append("Perturbing dVs proposal")  # sic: the reference labels the dVp proposal like this (pt_mcmc.f90:386)
-            if any(cfg.sig_mode):
-                labels.append("Perturbing sigma proposal")
-            print(" --- Summary ---")
-            print(f" # of sampled models: {hist['nmod']}")
-            for lab, a, n in zip(labels, cnt["naccept"], cnt["nprop"]):
-                print(f" # of {lab}: {int(a)} / {int(n)}")
+        if verbose:
+            print_summary(cfg, hist, cnt)
         rio.write_outputs(cfg, cfg.out_dir, nproc, hist, lh, vp_model, vs_model)
     pt.close()
     if world > 1:
@@ -105,13 +116,108 @@ def run(params_path: str, nproc: int, verbose: bool = True, n_iter: int = None, 
     return hist, cnt
 
 
+def station_checkpoint_path(path: str, station: int) -> str:
+    """The checkpoint file of station `station` (its position on the command line) of a group run."""
+    return f"{path}.{station}"
+
+
+def load_stations(params_paths):
+    """The configurations of the stations of a group run, refused before any GPU work when two stations write to the same
+    OUT_DIR or when they differ in N_BURN, N_ITER or N_CORR (a group advances its stations in lock step)."""
+    cfgs = [rio.load_problem(p) for p in params_paths]
+    seen = {}
+    for i, (p, c) in enumerate(zip(params_paths, cfgs)):
+        d = os.path.realpath(c.out_dir)
+        if d in seen:
+            j = seen[d]
+            raise ValueError(f"stations {j} ({params_paths[j]}) and {i} ({p}) write to the same OUT_DIR {c.out_dir}")
+        seen[d] = i
+    for key, name in (("nburn", "N_BURN"), ("niter", "N_ITER"), ("ncorr", "N_CORR")):
+        vals = [getattr(c, key) for c in cfgs]
+        if len(set(vals)) > 1:
+            raise ValueError(f"the stations of a group must have equal {name}: "
+                             + ", ".join(f"{p}: {v}" for p, v in zip(params_paths, vals)))
+    return cfgs
+
+
+def run_group(params_paths, nproc: int, verbose: bool = True, n_iter: int = None, checkpoint: str = None,
+              checkpoint_every: int = None, resume: bool = False):
+    """Several stations (one params file each) as one group on one GPU; arguments as in run().  Under torchrun process r
+    takes the stations i with i % world == r.  Returns {station index: (hist, counters)} of this process's stations."""
+    if resume and not checkpoint:
+        raise ValueError("resume needs a checkpoint path")
+    if checkpoint_every is not None and checkpoint_every < 1:
+        raise ValueError("checkpoint_every must be at least 1")
+    params_paths = list(params_paths)
+    cfgs = load_stations(params_paths)
+    world = int(os.environ.get("WORLD_SIZE", "1"))
+    rank = int(os.environ.get("RANK", "0"))
+    local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    mine = [i for i in range(len(params_paths)) if i % world == rank]
+    cks = [station_checkpoint_path(checkpoint, i) for i in range(len(params_paths))] if checkpoint else None
+    restore = False
+    if resume:                                            # every station restores, or none does (all processes see all files)
+        found = [os.path.exists(p) for p in cks]
+        if any(found) and not all(found):
+            raise FileNotFoundError(f"checkpoint files of {checkpoint} exist for some stations only: {found}")
+        restore = all(found)
+    if not mine:
+        return {}
+    for i in mine:
+        os.makedirs(cfgs[i].out_dir, exist_ok=True)
+        rio.write_side_copies(params_paths[i], cfgs[i].out_dir, os.path.dirname(os.path.abspath(params_paths[i])))
+        cfgs[i].r_inv = workloads.lapack_r_inv(cfgs[i])
+    pts = [ParallelTempering(cfgs[i], nproc, device=local_rank) for i in mine]
+    try:
+        if restore:
+            for i, pt in zip(mine, pts):
+                pt.restore(cks[i])
+            if verbose:
+                print(f" Resuming at iteration {pts[0].iterations_done} from {checkpoint}.<station>", flush=True)
+        cfg0 = cfgs[mine[0]]
+        n_tot = cfg0.nburn + cfg0.niter if n_iter is None else n_iter
+        done = pts[0].iterations_done
+        if done > n_tot:
+            raise ValueError(f"the checkpoints are at iteration {done}, beyond the {n_tot} iterations asked for")
+        step_len = max(cfg0.ncorr, 1) * 100
+        every = step_len if checkpoint_every is None else checkpoint_every
+        saved = done
+        with PtGroup(pts) as group:
+            while done < n_tot:                           # the progress steps of run()
+                step = min(step_len - done % step_len, n_tot - done)
+                group.run(step)
+                done += step
+                if verbose:
+                    print(f" Iteration #: {done} / {n_tot}", flush=True)
+                if cks and (done - saved >= every or done == n_tot):
+                    for i, pt in zip(mine, pts):
+                        pt.save(cks[i])
+                    saved = done
+        out = {}
+        for i, pt in zip(mine, pts):
+            cfg = cfgs[i]
+            hist, cnt = pt.hist(), pt.counters()
+            vp_model, vs_model = pt.models()
+            if verbose:
+                print(f" === {params_paths[i]} ===")
+                print_summary(cfg, hist, cnt)
+            rio.write_outputs(cfg, cfg.out_dir, nproc, hist, cnt["likelihood_hist"], vp_model, vs_model)
+            out[i] = (hist, cnt)
+        return out
+    finally:
+        for pt in pts:
+            pt.close()
+
+
 def main(argv=None):
     ap = argparse.ArgumentParser(description=__doc__)
-    ap.add_argument("params", nargs="?", default="params.in")
+    ap.add_argument("params", nargs="*", default=["params.in"],
+                    help="params.in of the run; several files (one per station) run side by side as one group")
     ap.add_argument("--nproc", type=int, default=20, help="number of virtual MPI ranks (mpirun -np of the reference)")
     ap.add_argument("--iters", type=int, default=None, help="override N_BURN + N_ITER (testing)")
     ap.add_argument("--checkpoint", default=None, metavar="PATH",
-                    help="save the chain state to PATH (under torchrun: PATH.<rank>-of-<world>) during and at the end of the run")
+                    help="save the chain state to PATH (under torchrun: PATH.<rank>-of-<world>; station i of a group: "
+                         "PATH.<i>) during and at the end of the run")
     ap.add_argument("--checkpoint-every", type=int, default=None, metavar="N",
                     help="save every N iterations, rounded up to the progress steps (default: every progress step)")
     ap.add_argument("--resume", action="store_true",
@@ -119,7 +225,11 @@ def main(argv=None):
     a = ap.parse_args(argv)
     if a.resume and not a.checkpoint:
         ap.error("--resume needs --checkpoint")
-    run(a.params, a.nproc, n_iter=a.iters, checkpoint=a.checkpoint, checkpoint_every=a.checkpoint_every, resume=a.resume)
+    if len(a.params) == 1:
+        run(a.params[0], a.nproc, n_iter=a.iters, checkpoint=a.checkpoint, checkpoint_every=a.checkpoint_every, resume=a.resume)
+    else:
+        run_group(a.params, a.nproc, n_iter=a.iters, checkpoint=a.checkpoint, checkpoint_every=a.checkpoint_every,
+                  resume=a.resume)
 
 
 if __name__ == "__main__":
