@@ -203,6 +203,21 @@ module rfinv_b200_capi
        character(kind=c_char), intent(in) :: path(*)
      end function rfinv_pt_restore
 
+     ! even/odd temperature swaps inside every virtual rank (ABI version 6): mode 0 the reference, 1 the sweep
+     integer(c_int32_t) function rfinv_pt_set_rank_swaps(handle, mode) bind(C, name="rfinv_pt_set_rank_swaps")
+       import :: c_int32_t, c_ptr
+       type(c_ptr), value :: handle
+       integer(c_int32_t), value :: mode
+     end function rfinv_pt_set_rank_swaps
+
+     ! mode, then swaps proposed / accepted per neighbour pair: n_prop(nchains-1), n_acc(nchains-1)
+     integer(c_int32_t) function rfinv_pt_get_rank_swaps(handle, mode, n_prop, n_acc) bind(C, name="rfinv_pt_get_rank_swaps")
+       import :: c_int32_t, c_int64_t, c_ptr
+       type(c_ptr), value :: handle
+       integer(c_int32_t), intent(out) :: mode
+       integer(c_int64_t), intent(out) :: n_prop(*), n_acc(*)
+     end function rfinv_pt_get_rank_swaps
+
      ! several stations advanced together (ABI version 5): handles(n) are the c_ptr of n handles after rfinv_pt_init
      integer(c_int32_t) function rfinv_pt_group_create(handles, n, group) bind(C, name="rfinv_pt_group_create")
        import :: c_int32_t, c_ptr

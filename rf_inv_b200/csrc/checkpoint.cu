@@ -150,6 +150,10 @@ std::vector<Part> parts(rfinv_handle* h, int it_done, long long n_models) {
   return v;
 }
 
+// The rank sweep's section (rfinv_pt_set_rank_swaps), written only in mode 1 -- a file written in mode 0 has the sections of
+// a library without the sweep: int64 [mode | n_prop per level | n_acc per level, summed over the ranks]
+constexpr const char* RS_SECTION = "rank_swaps";
+
 int io_error(const char* who, const std::string& path, const char* what) {
   rfinv_set_error("%s: %s: %s", who, path.c_str(), what);
   return RFINV_ERR_IO;
@@ -190,9 +194,19 @@ int32_t rfinv_pt_save(rfinv_handle* h, const char* path) {
   hd.ntrc = h->cfg.ntrc; hd.nsmp = h->cfg.nsmp; hd.k_max = h->cfg.k_max; hd.niter = h->cfg.niter;
   hd.it_done = s->it_done; hd.record = s->record ? 1 : 0; hd.n_eval_host = s->n_eval; hd.cap_models = d.vp_model ? d.cap_models : 0;
   fingerprints(h, hd.fp);
-  hd.n_sections = (uint32_t)ps.size();
+  std::vector<int64_t> rs;
+  if (s->rank_swaps == 1) {
+    const int nl = d.nchains > 1 ? d.nchains - 1 : 0;
+    rs.assign(1 + 2 * (size_t)nl, 0);
+    int32_t mode = 0;
+    int st;
+    if ((st = rfinv_pt_get_rank_swaps(h, &mode, rs.data() + 1, rs.data() + 1 + nl)) != RFINV_OK) return st;
+    rs[0] = mode;
+  }
+  hd.n_sections = (uint32_t)(ps.size() + (rs.empty() ? 0 : 1));
   size_t total = sizeof(CkHeader) + sizeof(uint64_t);
   for (const Part& p : ps) total += sizeof(CkSection) + (size_t)p.elem * p.count;
+  if (!rs.empty()) total += sizeof(CkSection) + sizeof(int64_t) * rs.size();
   std::unique_ptr<uint8_t[]> buf(new (std::nothrow) uint8_t[total]);
   if (!buf) { rfinv_set_error("%s: cannot allocate %zu bytes of host memory", who, total); return RFINV_ERR_IO; }
   size_t off = 0;
@@ -206,6 +220,14 @@ int32_t rfinv_pt_save(rfinv_handle* h, const char* path) {
     const size_t n = (size_t)p.elem * p.count;
     if (n) RFINV_CUDA_CHECK(cudaMemcpy(buf.get() + off, p.dev, n, cudaMemcpyDeviceToHost));
     off += n;
+  }
+  if (!rs.empty()) {
+    CkSection sc;
+    std::memset(&sc, 0, sizeof(sc));
+    std::snprintf(sc.name, sizeof(sc.name), "%s", RS_SECTION);
+    sc.elem_size = sizeof(int64_t); sc.count = rs.size();
+    std::memcpy(buf.get() + off, &sc, sizeof(sc)); off += sizeof(sc);
+    std::memcpy(buf.get() + off, rs.data(), sizeof(int64_t) * rs.size()); off += sizeof(int64_t) * rs.size();
   }
   const uint64_t sum = xxh64(buf.get(), off);
   std::memcpy(buf.get() + off, &sum, sizeof(sum));
@@ -336,6 +358,16 @@ int32_t rfinv_pt_restore(rfinv_handle* h, const char* path) {
       return RFINV_ERR_ARG;
     }
   }
+  // the rank sweep: the mode is part of the run (set it with rfinv_pt_set_rank_swaps before restoring)
+  const auto rs_it = found.find(RS_SECTION);
+  const int nl = d.nchains > 1 ? d.nchains - 1 : 0;
+  if ((rs_it != found.end()) != (s->rank_swaps == 1)) {
+    rfinv_set_error("%s: %s was written with the rank swaps %s, this handle has them %s (rfinv_pt_set_rank_swaps before restore)", who,
+                    path, rs_it != found.end() ? "on (mode 1)" : "off (mode 0)", s->rank_swaps == 1 ? "on (mode 1)" : "off (mode 0)");
+    return RFINV_ERR_ARG;
+  }
+  if (rs_it != found.end() && (rs_it->second.second.elem_size != sizeof(int64_t) || rs_it->second.second.count != 1 + 2 * (uint64_t)nl))
+    return io_error(who, file, "section 'rank_swaps' is malformed");
   if (hd.it_done < 0) return io_error(who, file, "negative iteration count");
   const std::vector<Part> ps = parts(h, hd.it_done, n_models);
   for (const Part& p : ps) {
@@ -357,6 +389,14 @@ int32_t rfinv_pt_restore(rfinv_handle* h, const char* path) {
   for (const Part& p : dst) {
     const size_t n = (size_t)p.elem * p.count;
     if (n) RFINV_CUDA_CHECK(cudaMemcpy(p.dev, buf.data() + found[p.name].first, n, cudaMemcpyHostToDevice));
+  }
+  if (rs_it != found.end() && nl > 0) {   // the per-level sums go into the row of local rank 0, the other rows start at zero
+    std::vector<int64_t> rs(1 + 2 * (size_t)nl);
+    std::memcpy(rs.data(), buf.data() + rs_it->second.first, sizeof(int64_t) * rs.size());
+    std::vector<int64_t> rows((size_t)d.G * nl, 0);
+    std::memcpy(rows.data(), rs.data() + 1 + nl, sizeof(int64_t) * nl);
+    RFINV_CUDA_CHECK(cudaMemcpy(d.rs_nprop, rs.data() + 1, sizeof(int64_t) * nl, cudaMemcpyHostToDevice));
+    RFINV_CUDA_CHECK(cudaMemcpy(d.rs_nacc, rows.data(), sizeof(int64_t) * rows.size(), cudaMemcpyHostToDevice));
   }
   s->it_done = hd.it_done;
   s->n_eval = hd.n_eval_host;

@@ -215,7 +215,7 @@ int32_t rfinv_comm_info(rfinv_handle* h, int32_t* world, int32_t* rank, int32_t*
 
 // output_results' reductions (src/mcmc_out.f90:52-79) on the device-resident bookkeeping: afterwards process 0 holds the
 // job-wide sums of nmod, nprop, naccept, nk, namp, nvpz, nvsz, nvpvsz, nz, nsig, likelihood_hist, vp/vs/vpvs_mean (the getters
-// rfinv_pt_get_hist / _get_counters then return what mpi_reduce delivers on rank 0) and, like mpi_gather (:86-93), the
+// rfinv_pt_get_hist / _get_counters then return what mpi_reduce delivers on rank 0; with the rank sweep on, also its counters) and, like mpi_gather (:86-93), the
 // recorded models of every process in process order (rfinv_pt_get_models).  Collective; call once, after the last iteration.
 int32_t rfinv_pt_reduce_outputs(rfinv_handle* h) {
   if (!h || !h->pt) { rfinv_set_error("rfinv_pt_reduce_outputs: call rfinv_pt_init first"); return RFINV_ERR_STATE; }
@@ -231,6 +231,8 @@ int32_t rfinv_pt_reduce_outputs(rfinv_handle* h) {
   struct Arr { void* p; size_t n; int type; };
   std::vector<Arr> arrs = {{d.nprop, (size_t)d.ntype, ncclUint64}, {d.naccept, (size_t)d.ntype, ncclUint64},
                            {s->d_lhist, (size_t)s->it_done, ncclFloat64}};
+  if (s->rank_swaps == 1 && d.rs_nprop)   // every process holds G rows of the same shape: their sum sums over all ranks
+    arrs.insert(arrs.end(), {{d.rs_nprop, (size_t)d.nchains - 1, ncclUint64}, {d.rs_nacc, (size_t)d.G * (d.nchains - 1), ncclUint64}});
   if (s->record) {
     const size_t T = c.ntrc, S = c.nsmp;
     arrs.insert(arrs.end(), {{d.nk, (size_t)c.k_max, ncclUint64}, {d.nz, (size_t)c.nbin_z, ncclUint64}, {d.nsig, (size_t)c.nbin_sig * T, ncclUint64},

@@ -724,6 +724,71 @@ __global__ void pt_swap_kernel(const PtDev p, const double* gathered, int world,
   pt_swap_decide(p, gathered, world, table_len);
 }
 
+// ---------------- even/odd temperature swaps inside every virtual rank (rfinv_pt_set_rank_swaps, DESIGN.md 7c) ----------------
+// Philox4x64-10 (Salmon, Moraes, Dror & Shaw, SC 2011), output word 0: a counter-based generator without state, so the sweep
+// leaves the mt19937 streams -- and with them every draw of the reference -- exactly as they are.
+__device__ __forceinline__ uint64_t philox4x64_w0(uint64_t c0, uint64_t c1, uint64_t c2, uint64_t c3, uint64_t k0, uint64_t k1) {
+  constexpr uint64_t M0 = 0xD2E7470EE14C6C93ULL, M1 = 0xCA5A826395121157ULL;
+#pragma unroll
+  for (int round = 0; round < 10; ++round) {
+    if (round) { k0 += 0x9E3779B97F4A7C15ULL; k1 += 0xBB67AE8584CAA73BULL; }
+    const uint64_t hi0 = __umul64hi(M0, c0), lo0 = M0 * c0, hi1 = __umul64hi(M1, c2), lo1 = M1 * c2;
+    c0 = hi1 ^ c1 ^ k0; c1 = lo1; c2 = hi0 ^ c3 ^ k1; c3 = lo0;
+  }
+  return c0;
+}
+
+// One WARP per virtual rank, after acceptance and bookkeeping, before the global swap.  Level of a chain = its place in the
+// rank's chains sorted by (temperature, chain index), found by counting; levels l = i (mod 2) and l + 1 are proposed a swap
+// with judge_pt's test (src/pt_mcmc.f90:580-595) and the Philox uniform of counter (i, global rank, l, 0).  Accepted pairs
+// exchange their temperatures in temps and in the swap table.  peer: the peer-memory exchange, where pt_finish_kernel has
+// already advanced *it_dev and the table alternates.  DECIDE (single process): the last CTA then takes the global swap
+// decision that pt_finish_kernel<false, true> takes without the sweep.
+constexpr int PT_RS_WARPS = 4;
+template <bool DECIDE>
+__global__ void __launch_bounds__(32 * PT_RS_WARPS) pt_rank_swap_kernel(const PtDev p, double* __restrict__ table, int table_len,
+                                                                        int peer) {
+  extern __shared__ int rs_at[];   // [warps][nchains]: chain at each level
+  __shared__ int s_last;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, n = p.nchains;
+  const int r = blockIdx.x * (blockDim.x >> 5) + warp;
+  const int it = *p.it_dev - peer;
+  if (peer) table += (size_t)(it & 1) * table_len;
+  if (r < p.G) {
+    int* at = rs_at + (size_t)warp * n;
+    const int c0 = r * n;
+    for (int a = lane; a < n; a += 32) {
+      const double ta = p.temps[c0 + a];
+      int lvl = 0;
+      for (int b = 0; b < n; ++b) { const double tb = p.temps[c0 + b]; lvl += tb < ta || (tb == ta && b < a); }
+      at[lvl] = a;
+    }
+    __syncwarp();
+    const uint64_t grank = (uint64_t)(p.rank_begin + r), key = (uint64_t)(uint32_t)p.iseed;
+    for (int l = (it & 1) + 2 * lane; l + 1 < n; l += 64) {
+      const int a = c0 + at[l], b = c0 + at[l + 1];
+      const double ta = p.temps[a], tb = p.temps[b];
+      const uint64_t w = philox4x64_w0((uint64_t)it, grank, (uint64_t)l, 0, key, 0);
+      const double u = (double)(w >> 11) * 0x1p-53;
+      const double del_s = __dmul_rn(__dsub_rn(p.logl[b], p.logl[a]), __dsub_rn(__ddiv_rn(1.0, ta), __ddiv_rn(1.0, tb)));
+      const int yn = log(u) <= del_s;
+      if (yn) { p.temps[a] = tb; p.temps[b] = ta; table[a] = tb; table[b] = ta; }
+      p.rs_nacc[(size_t)r * (n - 1) + l] += (unsigned long long)yn;
+    }
+    if (r == 0 && lane == 0)
+      for (int l = it & 1; l + 1 < n; l += 2) p.rs_nprop[l] += (unsigned long long)p.G;
+  }
+  if (!DECIDE) return;
+  __threadfence();   // this CTA's table entries are ordered before its arrival
+  __syncthreads();
+  if (threadIdx.x == 0) s_last = atomicAdd(p.rs_arrived, 1) == (int)gridDim.x - 1;
+  __syncthreads();
+  if (!s_last || threadIdx.x != 0) return;
+  __threadfence();
+  *p.rs_arrived = 0;
+  pt_swap_decide(p, table, 1, table_len);
+}
+
 // Peer-memory exchange, side branch of the iteration (rfinv_pt.h).  pt_pairpush_kernel: one warp; the owner of virtual rank 0
 // takes the pair pt_propose_kernel has just drawn (local table, parity it & 1) to every process.
 __global__ void pt_pairpush_kernel(const PtDev p, const double* __restrict__ table, const PtPeers px) {
@@ -973,7 +1038,7 @@ void rfinv_handle::free_pt() {
   cudaFree(d.logl); cudaFree(d.temps); cudaFree(d.phi); cudaFree(d.slot); cudaFree(d.rft_smp[0]); cudaFree(d.rft_smp[1]);
   cudaFree(d.pk); cudaFree(d.pz); cudaFree(d.pdvp); cudaFree(d.pdvs); cudaFree(d.psig); cudaFree(d.pphi); cudaFree(d.log_r);
   cudaFree(d.log_prior12); cudaFree(d.itype); cudaFree(d.pflag); cudaFree(d.active); cudaFree(d.n_active);
-  cudaFree(d.nprop); cudaFree(d.naccept); cudaFree(d.n_eval);
+  cudaFree(d.nprop); cudaFree(d.naccept); cudaFree(d.n_eval); cudaFree(d.rs_nprop); cudaFree(d.rs_nacc); cudaFree(d.rs_arrived);
   cudaFree(d.log_flags); cudaFree(d.log_itypes); cudaFree(d.log_swaps);
   cudaFree(d.nk); cudaFree(d.nz); cudaFree(d.nsig); cudaFree(d.namp); cudaFree(d.nvpz); cudaFree(d.nvsz); cudaFree(d.nvpvsz); cudaFree(d.nmod);
   cudaFree(d.vp_mean); cudaFree(d.vs_mean); cudaFree(d.vpvs_mean); cudaFree(d.vp_model); cudaFree(d.vs_model); cudaFree(d.cold_ordinal); cudaFree(d.cold_count); cudaFree(d.ocean_bin);
@@ -1142,6 +1207,52 @@ int32_t rfinv_pt_set_logging(rfinv_handle* h, int32_t cap_iters) {
   return RFINV_OK;
 }
 
+int32_t rfinv_pt_set_rank_swaps(rfinv_handle* h, int32_t mode) {
+  int st = pt_require(h, "rfinv_pt_set_rank_swaps");
+  if (st != RFINV_OK) return st;
+  PtState* s = h->pt;
+  PtDev& d = s->dev;
+  if (mode != 0 && mode != 1) { rfinv_set_error("rfinv_pt_set_rank_swaps: mode %d (0: off, 1: even/odd swaps inside every rank)", mode); return RFINV_ERR_ARG; }
+  if (s->step_pending) {
+    rfinv_set_error("rfinv_pt_set_rank_swaps: an iteration is half done (rfinv_pt_local_step without rfinv_pt_apply_swap)");
+    return RFINV_ERR_STATE;
+  }
+  if (s->reduced) { rfinv_set_error("rfinv_pt_set_rank_swaps: rfinv_pt_reduce_outputs has run"); return RFINV_ERR_STATE; }
+  RFINV_CUDA_CHECK(cudaSetDevice(h->device));
+  RFINV_CUDA_CHECK(cudaStreamSynchronize(h->stream));
+  if (mode == 1 && d.nchains >= 2 && !d.rs_nprop) {   // counters start at zero and survive later switches
+    if ((st = dalloc(&d.rs_nprop, (size_t)d.nchains - 1)) != RFINV_OK) return st;
+    if ((st = dalloc(&d.rs_nacc, (size_t)d.G * (d.nchains - 1))) != RFINV_OK) return st;
+    if ((st = dalloc(&d.rs_arrived, 1)) != RFINV_OK) return st;
+  }
+  pt_drop_graphs(s);   // the captured launch sequence depends on the mode
+  s->rank_swaps = mode;
+  return RFINV_OK;
+}
+
+int32_t rfinv_pt_get_rank_swaps(rfinv_handle* h, int32_t* mode, int64_t* n_prop, int64_t* n_acc) {
+  int st = pt_require(h, "rfinv_pt_get_rank_swaps");
+  if (st != RFINV_OK) return st;
+  PtState* s = h->pt;
+  PtDev& d = s->dev;
+  if (mode) *mode = s->rank_swaps;
+  const int nl = d.nchains - 1;
+  if (nl < 1) return RFINV_OK;
+  RFINV_CUDA_CHECK(cudaStreamSynchronize(h->stream));
+  std::vector<unsigned long long> prop(nl, 0ULL), rows((size_t)d.G * nl, 0ULL);
+  if (d.rs_nprop) {
+    RFINV_CUDA_CHECK(cudaMemcpy(prop.data(), d.rs_nprop, sizeof(unsigned long long) * nl, cudaMemcpyDeviceToHost));
+    RFINV_CUDA_CHECK(cudaMemcpy(rows.data(), d.rs_nacc, sizeof(unsigned long long) * rows.size(), cudaMemcpyDeviceToHost));
+  }
+  for (int l = 0; l < nl; ++l) {
+    unsigned long long acc = 0ULL;
+    for (int r = 0; r < d.G; ++r) acc += rows[(size_t)r * nl + l];
+    if (n_prop) n_prop[l] = (int64_t)prop[l];
+    if (n_acc) n_acc[l] = (int64_t)acc;
+  }
+  return RFINV_OK;
+}
+
 // room in the likelihood history for iterations [0, upto); never called while a launch sequence is being captured
 static int pt_reserve_lhist(rfinv_handle* h, int upto) {
   PtState* s = h->pt;
@@ -1162,7 +1273,7 @@ static int pt_reserve_lhist(rfinv_handle* h, int upto) {
 // The launches of one iteration except the swap decision: proposal pass, batched evaluation, acceptance, likelihood
 // history, (posterior bookkeeping,) and this process's swap table.  Nothing here depends on the host's iteration counter.
 // fuse_swap: a single process -- the swap decision is taken by the last CTA of pt_finish_kernel (unless bookkeeping kernels
-// have to run in between)
+// have to run in between) or, with the rank sweep on, by the last CTA of pt_rank_swap_kernel
 static int pt_enqueue_local(rfinv_handle* h, bool record, bool peer_exchange = false, bool fuse_swap = false) {
   PtState* s = h->pt;
   PtDev& d = s->dev;
@@ -1199,17 +1310,30 @@ static int pt_enqueue_local(rfinv_handle* h, bool record, bool peer_exchange = f
   }
   if ((st = pt_eval(h, /*proposal=*/true, /*all=*/false)) != RFINV_OK) return st;
   if (peer_side) RFINV_CUDA_CHECK(cudaStreamWaitEvent(q, s->ev_side[2], 0));   // the side branch joins in front of pt_finish_kernel
+  const bool peer = s->peer_state == 1 && peer_exchange;
+  const bool sweep = pt_sweeps(s);
   {
     const unsigned nb = (unsigned)((d.Cl + PT_FIN_CHAINS - 1) / PT_FIN_CHAINS);
-    const bool peer = s->peer_state == 1 && peer_exchange;
     if (peer) pt_finish_kernel<true, false><<<nb, PT_FIN_THREADS, 0, q>>>(h->dc, d, s->d_table, s->peers, s->d_lhist, s->d_lh_part, s->d_lh_cnt);
-    else if (fuse_swap && !record) pt_finish_kernel<false, true><<<nb, PT_FIN_THREADS, 0, q>>>(h->dc, d, s->d_table, s->peers, s->d_lhist, s->d_lh_part, s->d_lh_cnt);
+    else if (fuse_swap && !record && !sweep) pt_finish_kernel<false, true><<<nb, PT_FIN_THREADS, 0, q>>>(h->dc, d, s->d_table, s->peers, s->d_lhist, s->d_lh_part, s->d_lh_cnt);
     else pt_finish_kernel<false, false><<<nb, PT_FIN_THREADS, 0, q>>>(h->dc, d, s->d_table, s->peers, s->d_lhist, s->d_lh_part, s->d_lh_cnt);
   }
   if (record) {   // posterior bookkeeping of the state after acceptance, before the swap (src/pt_mcmc.f90:204-286)
     pt_coldscan_kernel<<<1, 1024, 0, q>>>(d);
     pt_record_kernel<<<d.Cl, 128, 0, q>>>(h->dc, d);
     pt_record_finish_kernel<<<1, 1, 0, q>>>(d);
+  }
+  if (sweep) {   // after the bookkeeping (it sees the temperatures at acceptance), before the global swap reads the table
+    const int warps = d.nchains <= 3072 ? PT_RS_WARPS : 1;
+    const size_t smem = sizeof(int) * (size_t)d.nchains * warps;
+    const unsigned nb = (unsigned)((d.G + warps - 1) / warps);
+    if (fuse_swap && !peer) {
+      RFINV_CUDA_CHECK(rfinv_raise_smem_limit((const void*)pt_rank_swap_kernel<true>, smem));
+      pt_rank_swap_kernel<true><<<nb, 32 * warps, smem, q>>>(d, s->d_table, s->table_len, 0);
+    } else {
+      RFINV_CUDA_CHECK(rfinv_raise_smem_limit((const void*)pt_rank_swap_kernel<false>, smem));
+      pt_rank_swap_kernel<false><<<nb, 32 * warps, smem, q>>>(d, s->d_table, s->table_len, peer ? 1 : 0);
+    }
   }
   RFINV_CUDA_CHECK(cudaGetLastError());
   return RFINV_OK;
@@ -1262,7 +1386,7 @@ static int pt_enqueue_iteration(rfinv_handle* h, int world, bool record) {
   int st;
   const bool peer = world > 1 && s->peer_state == 1;
   if ((st = pt_enqueue_local(h, record, peer, world == 1)) != RFINV_OK) return st;
-  if (world == 1 && !record) return RFINV_OK;   // pt_finish_kernel took the swap decision
+  if (world == 1 && (!record || pt_sweeps(s))) return RFINV_OK;   // pt_finish_kernel or pt_rank_swap_kernel took the swap decision
   if (peer) return RFINV_OK;   // pair and table went to every process from inside the kernels; the swap is applied an iteration later
   const double* gathered = s->d_table;
   if (world > 1) {

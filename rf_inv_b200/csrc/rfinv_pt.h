@@ -43,6 +43,10 @@ struct PtDev {
   // (likelihood history, logs) -- nothing of an iteration's launch sequence depends on the host's counter, so the sequence
   // can be captured once in a CUDA graph and replayed
   int* it_dev;
+  // even/odd swaps inside every virtual rank (rfinv_pt_set_rank_swaps, DESIGN.md 7c); allocated by the first switch to mode 1
+  unsigned long long* rs_nprop;   // [nchains - 1] proposals per level, summed over the local ranks
+  unsigned long long* rs_nacc;    // [G][nchains - 1] accepted swaps per rank and level (rows: no same-address atomics)
+  int* rs_arrived;                // arrival counter of pt_rank_swap_kernel
 };
 
 struct ncclComm;   // NCCL communicator (comm.cu)
@@ -114,4 +118,8 @@ struct PtState {
   bool record = false;
   bool step_pending = false;   // rfinv_pt_local_step has run, rfinv_pt_apply_swap not yet: no checkpoint in between
   bool reduced = false;        // rfinv_pt_reduce_outputs has run: the bookkeeping may hold job-wide sums
+  int rank_swaps = 0;          // rfinv_pt_set_rank_swaps: 0 the reference's global swap only, 1 the rank sweep before it
 };
+
+// does an iteration of this state run the rank sweep?  (nothing to pair with fewer than two chains per rank)
+inline bool pt_sweeps(const PtState* s) { return s->rank_swaps == 1 && s->dev.nchains >= 2; }

@@ -118,6 +118,21 @@ class ParallelTempering:
         uninterrupted run.  Logging is switched off: call set_logging() again."""
         capi.check(self._lib.rfinv_pt_restore(self.ev.handle, os.fsencode(path)))
 
+    # -- even/odd swaps inside every virtual rank (DESIGN.md 7c) -----------------------------------
+    def set_rank_swaps(self, mode: int) -> None:
+        """0: the reference's one global swap per iteration (default); 1: also a sweep of swaps between neighbouring
+        temperature levels inside every virtual rank, before the global swap.  Between runs; every process the same."""
+        capi.check(self._lib.rfinv_pt_set_rank_swaps(self.ev.handle, int(mode)))
+
+    def rank_swaps(self) -> Dict[str, object]:
+        """{mode, n_prop, n_acc}: swaps the sweep proposed and accepted per neighbour pair l = 0 .. nchains-2, summed over
+        this process's ranks (over the job on process 0 after reduce_outputs() in mode 1)."""
+        n = max(self.cfg.nchains - 1, 0)
+        mode = C.c_int32(0)
+        n_prop = np.zeros(n, dtype=np.int64); n_acc = np.zeros(n, dtype=np.int64)
+        capi.check(self._lib.rfinv_pt_get_rank_swaps(self.ev.handle, C.byref(mode), _p(n_prop, capi.i64p), _p(n_acc, capi.i64p)))
+        return dict(mode=int(mode.value), n_prop=n_prop, n_acc=n_acc)
+
     # -- results ----------------------------------------------------------------------------------
     def set_logging(self, cap_iters: int) -> None:
         capi.check(self._lib.rfinv_pt_set_logging(self.ev.handle, int(cap_iters)))

@@ -13,7 +13,10 @@ Several params files (``python -m rf_inv_b200.run a/params.in b/params.in ... --
 side on one GPU as one group (rfinv_pt_group_run): every station writes into its own OUT_DIR exactly the files a run of its
 params file alone writes.  The stations must agree on N_BURN, N_ITER and N_CORR and write to different OUT_DIRs.  Station i
 (its position on the command line) checkpoints to ``PATH.<i>``.  Under torchrun process r runs the stations i with
-i % world == r as its group on its own GPU; the processes do not communicate."""
+i % world == r as its group on its own GPU; the processes do not communicate.
+
+``--rank-swaps`` adds even/odd temperature swaps between neighbouring levels inside every virtual rank (DESIGN.md 7c).  The
+reference's files are written as without it, plus OUT_DIR/rank_swaps with the acceptance of each neighbour pair."""
 from __future__ import annotations
 
 import argparse
@@ -45,10 +48,25 @@ def print_summary(cfg, hist, cnt) -> None:
         print(f" # of {lab}: {int(a)} / {int(n)}")
 
 
+def write_rank_swaps(out_dir: str, rs) -> None:
+    """OUT_DIR/rank_swaps: one line per neighbour pair l = 1 .. nchains-1 (levels l-1 and l, level 0 the coldest):
+    l, swaps accepted, swaps proposed, acceptance rate."""
+    with open(os.path.join(out_dir, "rank_swaps"), "w") as f:
+        for l, (a, n) in enumerate(zip(rs["n_acc"], rs["n_prop"]), start=1):
+            f.write(f"{l:5d} {int(a):12d} {int(n):12d} {a / n if n else 0.0:12.6f}\n")
+
+
+def print_rank_swaps(rs) -> None:
+    print(" --- Swaps between neighbouring temperature levels inside the ranks ---")
+    for l, (a, n) in enumerate(zip(rs["n_acc"], rs["n_prop"]), start=1):
+        print(f" # of swaps between levels {l - 1} and {l}: {int(a)} / {int(n)} ({a / n if n else 0.0:.4f})")
+
+
 def run(params_path: str, nproc: int, verbose: bool = True, n_iter: int = None, checkpoint: str = None,
-        checkpoint_every: int = None, resume: bool = False):
+        checkpoint_every: int = None, resume: bool = False, rank_swaps: bool = False):
     """checkpoint: save the state to this path every `checkpoint_every` iterations (rounded up to the progress steps; default:
-    every progress step) and at the end.  resume: restore it first if it exists and continue from its iteration count."""
+    every progress step) and at the end.  resume: restore it first if it exists and continue from its iteration count.
+    rank_swaps: the even/odd sweep inside every virtual rank (ParallelTempering.set_rank_swaps(1)); adds OUT_DIR/rank_swaps."""
     if resume and not checkpoint:
         raise ValueError("resume needs a checkpoint path")
     if checkpoint_every is not None and checkpoint_every < 1:
@@ -70,6 +88,8 @@ def run(params_path: str, nproc: int, verbose: bool = True, n_iter: int = None, 
         os.makedirs(cfg.out_dir, exist_ok=True)
         rio.write_side_copies(params_path, cfg.out_dir, os.path.dirname(os.path.abspath(params_path)))
     pt = ParallelTempering(cfg, nproc, device=local_rank, world=world, rank=rank)
+    if rank_swaps:                                        # before a restore: the checkpoint holds the sweep's counters
+        pt.set_rank_swaps(1)
     n_tot = cfg.nburn + cfg.niter if n_iter is None else n_iter
     ck = checkpoint_path(checkpoint, world, rank) if checkpoint else None
     if resume:
@@ -105,11 +125,16 @@ def run(params_path: str, nproc: int, verbose: bool = True, n_iter: int = None, 
         pt.reduce_outputs()                               # ncclReduce / ncclSend+Recv inside the library: process 0 is job-wide now
     hist, cnt = pt.hist(), pt.counters()
     vp_model, vs_model = pt.models()
+    rs = pt.rank_swaps() if rank_swaps else None
     lh = cnt["likelihood_hist"]
     if rank == 0:
         if verbose:
             print_summary(cfg, hist, cnt)
+            if rs:
+                print_rank_swaps(rs)
         rio.write_outputs(cfg, cfg.out_dir, nproc, hist, lh, vp_model, vs_model)
+        if rs:
+            write_rank_swaps(cfg.out_dir, rs)
     pt.close()
     if world > 1:
         dist.destroy_process_group()
@@ -141,7 +166,7 @@ def load_stations(params_paths):
 
 
 def run_group(params_paths, nproc: int, verbose: bool = True, n_iter: int = None, checkpoint: str = None,
-              checkpoint_every: int = None, resume: bool = False):
+              checkpoint_every: int = None, resume: bool = False, rank_swaps: bool = False):
     """Several stations (one params file each) as one group on one GPU; arguments as in run().  Under torchrun process r
     takes the stations i with i % world == r.  Returns {station index: (hist, counters)} of this process's stations."""
     if resume and not checkpoint:
@@ -169,6 +194,9 @@ def run_group(params_paths, nproc: int, verbose: bool = True, n_iter: int = None
         cfgs[i].r_inv = workloads.lapack_r_inv(cfgs[i])
     pts = [ParallelTempering(cfgs[i], nproc, device=local_rank) for i in mine]
     try:
+        if rank_swaps:
+            for pt in pts:
+                pt.set_rank_swaps(1)
         if restore:
             for i, pt in zip(mine, pts):
                 pt.restore(cks[i])
@@ -201,7 +229,11 @@ def run_group(params_paths, nproc: int, verbose: bool = True, n_iter: int = None
             if verbose:
                 print(f" === {params_paths[i]} ===")
                 print_summary(cfg, hist, cnt)
+                if rank_swaps:
+                    print_rank_swaps(pt.rank_swaps())
             rio.write_outputs(cfg, cfg.out_dir, nproc, hist, cnt["likelihood_hist"], vp_model, vs_model)
+            if rank_swaps:
+                write_rank_swaps(cfg.out_dir, pt.rank_swaps())
             out[i] = (hist, cnt)
         return out
     finally:
@@ -222,14 +254,18 @@ def main(argv=None):
                     help="save every N iterations, rounded up to the progress steps (default: every progress step)")
     ap.add_argument("--resume", action="store_true",
                     help="continue from the checkpoint if it exists (a missing file starts a fresh run)")
+    ap.add_argument("--rank-swaps", action="store_true",
+                    help="also swap temperatures between neighbouring levels inside every virtual rank, even and odd pairs "
+                         "in turn (writes OUT_DIR/rank_swaps)")
     a = ap.parse_args(argv)
     if a.resume and not a.checkpoint:
         ap.error("--resume needs --checkpoint")
     if len(a.params) == 1:
-        run(a.params[0], a.nproc, n_iter=a.iters, checkpoint=a.checkpoint, checkpoint_every=a.checkpoint_every, resume=a.resume)
+        run(a.params[0], a.nproc, n_iter=a.iters, checkpoint=a.checkpoint, checkpoint_every=a.checkpoint_every, resume=a.resume,
+            rank_swaps=a.rank_swaps)
     else:
         run_group(a.params, a.nproc, n_iter=a.iters, checkpoint=a.checkpoint, checkpoint_every=a.checkpoint_every,
-                  resume=a.resume)
+                  resume=a.resume, rank_swaps=a.rank_swaps)
 
 
 if __name__ == "__main__":

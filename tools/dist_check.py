@@ -3,6 +3,9 @@ the accept / reject flags, proposal types, swap decisions, final state and job-w
 rfinv_pt_run_distributed (in-library ncclAllGather, CUDA graph) equal those of ONE process holding every virtual rank.
 
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29511 tools/dist_check.py
+
+--rank-swaps runs both sides with the even/odd sweep inside every virtual rank (set_rank_swaps(1)) and also compares its
+job-wide counters.
 """
 import faulthandler, hashlib, json, os, signal, sys
 faulthandler.register(signal.SIGTERM, all_threads=True, chain=False)
@@ -16,7 +19,7 @@ from rf_inv_b200.evaluator import Evaluator
 from rf_inv_b200.pt import ParallelTempering
 
 
-def identity_check(cfg, nproc_total, n_iter, world, rank, local_rank, dist, torch):
+def identity_check(cfg, nproc_total, n_iter, world, rank, local_rank, dist, torch, rank_swaps=0):
     """Returns (ok, detail) on every process."""
     dev = torch.device("cuda", local_rank)
     # distributed run
@@ -24,6 +27,8 @@ def identity_check(cfg, nproc_total, n_iter, world, rank, local_rank, dist, torc
         print(f"[rank {rank}] {msg}", file=sys.stderr, flush=True)
     pt = ParallelTempering(cfg, nproc_total, device=local_rank, world=world, rank=rank)
     pt.set_logging(n_iter)
+    if rank_swaps:
+        pt.set_rank_swaps(rank_swaps)
     pt.init_comm(dist, torch)
     say("communicator up")
     pt.run_distributed(n_iter, dist, torch)
@@ -35,6 +40,7 @@ def identity_check(cfg, nproc_total, n_iter, world, rank, local_rank, dist, torc
     say("outputs reduced")
     cnt = pt.counters()
     hist = pt.hist() if cfg.niter > 0 else None
+    rsw = pt.rank_swaps() if rank_swaps else None
     say("getters done")
     pt.close()
     say("closed")
@@ -42,11 +48,14 @@ def identity_check(cfg, nproc_total, n_iter, world, rank, local_rank, dist, torc
     if rank == 0:
         ref = ParallelTempering(cfg, nproc_total, device=local_rank)
         ref.set_logging(n_iter)
+        if rank_swaps:
+            ref.set_rank_swaps(rank_swaps)
         ref.run(n_iter)
         rf, ri, rs = ref.log(n_iter)
         rst = ref.state()
         rcnt = ref.counters()
         rhist = ref.hist() if cfg.niter > 0 else None
+        rrsw = ref.rank_swaps() if rank_swaps else None
         ref.close()
         say("reference run done")
         box = [dict(flags=rf, itypes=ri, swaps=rs, state=rst)]
@@ -65,6 +74,9 @@ def identity_check(cfg, nproc_total, n_iter, world, rank, local_rank, dist, torc
     if rank == 0:
         parts["nprop"] = np.array_equal(cnt["nprop"], rcnt["nprop"]); parts["naccept"] = np.array_equal(cnt["naccept"], rcnt["naccept"])
         # likelihood_hist is a sum over processes of per-process tree sums: equal up to the order of additions
+        if rank_swaps:
+            parts["rank_swaps"] = (rsw["mode"] == rrsw["mode"] == 1 and np.array_equal(rsw["n_prop"], rrsw["n_prop"])
+                                   and np.array_equal(rsw["n_acc"], rrsw["n_acc"]) and int(rrsw["n_acc"].sum()) > 0)
         parts["likelihood_hist"] = bool(np.allclose(cnt["likelihood_hist"], rcnt["likelihood_hist"], rtol=1e-12, atol=0))
         if hist is not None:
             parts["nmod"] = hist["nmod"] == rhist["nmod"]
@@ -88,6 +100,7 @@ if __name__ == "__main__":
     torch.cuda.set_device(local_rank)
     os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
     dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
+    rank_swaps = 1 if "--rank-swaps" in sys.argv[1:] else 0
     out = {}
     for name, nproc, iters, kw in (("sample", 4 * world, 300, dict(nburn=100, niter=200)), ("c4", 8 * world, 120, dict()), ("target", 16 * world, 60, dict())):
         cfg = workloads.make_config(name)
@@ -101,7 +114,7 @@ if __name__ == "__main__":
         with Evaluator(cfg, device=local_rank) as ev:
             _, rft, _ = ev.calc_likelihood(tm["k"], tm["z"], tm["dvp"], tm["dvs"], tm["sig"], want_rft=True)
         cfg.obs = (rft[0, :, :cfg.nsmp] + np.random.default_rng(7).normal(0.0, 0.01, (cfg.ntrc, cfg.nsmp))).astype(np.float32).astype(np.float64)
-        ok, detail = identity_check(cfg, nproc, iters, world, rank, local_rank, dist, torch)
+        ok, detail = identity_check(cfg, nproc, iters, world, rank, local_rank, dist, torch, rank_swaps)
         out[name] = dict(identical=ok, world=world, virtual_ranks=nproc, iterations=iters, **detail)
     if rank == 0:
         print(json.dumps(out), flush=True)
