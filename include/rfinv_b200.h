@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define RFINV_ABI_VERSION 6
+#define RFINV_ABI_VERSION 7
 
 /* status codes */
 #define RFINV_OK 0
@@ -303,6 +303,21 @@ int32_t rfinv_pt_set_rank_swaps(rfinv_handle* h, int32_t mode);
  * (after rfinv_pt_reduce_outputs in mode 1: over the job, on process 0).  n_prop / n_acc have nchains - 1 entries; any
  * pointer may be NULL. */
 int32_t rfinv_pt_get_rank_swaps(rfinv_handle* h, int32_t* mode, int64_t* n_prop, int64_t* n_acc);
+
+/* ---- ladder tuning during the burn-in (ABI version 7, DESIGN.md 7d) --------------------------------------------------------
+ * On top of the rank sweep (mode 1): at the tuning points e = 64, 128, 256, ... <= nburn (inside iteration e - 1, after its
+ * sweep, before its global swap) every virtual rank moves the temperatures of its levels above the cold ones so that the
+ * rejection rates its neighbour pairs showed in the round [e/2, e) (from 0 for e = 64) would be equal: the ladder of equal
+ * rejection rates of Syed, Bouchard-Cote, Deligiannidis & Doucet (JRSS-B 2021).  The coldest level, the hottest and every cold
+ * chain keep their temperatures; models, logL and every random stream are untouched.  After the burn-in the ladders stay
+ * fixed.  Off (the default) leaves the mode-1 run bit for bit as it is.  A checkpoint restores only into a handle with the same
+ * setting; a distributed run needs it on every process.
+ * RFINV_ERR_ARG: a value other than 0 or 1.  RFINV_ERR_STATE: switching it on without rfinv_pt_init, after an iteration has
+ * run, or while the rank swaps are not mode 1; either way between rfinv_pt_local_step and rfinv_pt_apply_swap or after
+ * rfinv_pt_reduce_outputs.  rfinv_pt_set_rank_swaps(h, 0) switches the tuning off as well. */
+int32_t rfinv_pt_set_ladder_tuning(rfinv_handle* h, int32_t on);
+/* The setting and the number of tuning points passed with it on; either pointer may be NULL. */
+int32_t rfinv_pt_get_ladder_tuning(rfinv_handle* h, int32_t* on, int32_t* n_points);
 
 /* ---- file formats either side of the path (host only, no CUDA) ---------------------------------------
  * params.in (positional, '#' comment lines; src/params.f90:101-405), SAC traces cut to [T_START, T_END]

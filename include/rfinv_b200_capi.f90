@@ -218,6 +218,20 @@ module rfinv_b200_capi
        integer(c_int64_t), intent(out) :: n_prop(*), n_acc(*)
      end function rfinv_pt_get_rank_swaps
 
+     ! ladder tuning during the burn-in on top of the rank swaps (ABI version 7): on 0 or 1, before the first iteration
+     integer(c_int32_t) function rfinv_pt_set_ladder_tuning(handle, on) bind(C, name="rfinv_pt_set_ladder_tuning")
+       import :: c_int32_t, c_ptr
+       type(c_ptr), value :: handle
+       integer(c_int32_t), value :: on
+     end function rfinv_pt_set_ladder_tuning
+
+     ! the setting, and the tuning points passed with it on
+     integer(c_int32_t) function rfinv_pt_get_ladder_tuning(handle, on, n_points) bind(C, name="rfinv_pt_get_ladder_tuning")
+       import :: c_int32_t, c_ptr
+       type(c_ptr), value :: handle
+       integer(c_int32_t), intent(out) :: on, n_points
+     end function rfinv_pt_get_ladder_tuning
+
      ! several stations advanced together (ABI version 5): handles(n) are the c_ptr of n handles after rfinv_pt_init
      integer(c_int32_t) function rfinv_pt_group_create(handles, n, group) bind(C, name="rfinv_pt_group_create")
        import :: c_int32_t, c_ptr

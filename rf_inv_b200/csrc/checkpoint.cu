@@ -153,6 +153,11 @@ std::vector<Part> parts(rfinv_handle* h, int it_done, long long n_models) {
 // The rank sweep's section (rfinv_pt_set_rank_swaps), written only in mode 1 -- a file written in mode 0 has the sections of
 // a library without the sweep: int64 [mode | n_prop per level | n_acc per level, summed over the ranks]
 constexpr const char* RS_SECTION = "rank_swaps";
+// The ladder tuning's section (rfinv_pt_set_ladder_tuning), written only with the tuning on: int64 [on | per local rank and
+// level pair, the acceptances since the last tuning point].  The rank_swaps section keeps only sums over the ranks, so the
+// restore rebuilds the snapshot rows as (restored rows) - (acceptances of the round): the next tuning point sees the counts
+// of an uninterrupted run.
+constexpr const char* LT_SECTION = "ladder_tuning";
 
 int io_error(const char* who, const std::string& path, const char* what) {
   rfinv_set_error("%s: %s: %s", who, path.c_str(), what);
@@ -203,10 +208,23 @@ int32_t rfinv_pt_save(rfinv_handle* h, const char* path) {
     if ((st = rfinv_pt_get_rank_swaps(h, &mode, rs.data() + 1, rs.data() + 1 + nl)) != RFINV_OK) return st;
     rs[0] = mode;
   }
-  hd.n_sections = (uint32_t)(ps.size() + (rs.empty() ? 0 : 1));
+  std::vector<int64_t> lt;
+  if (d.rs_tune) {
+    const size_t nr = d.nchains > 1 ? (size_t)d.G * (d.nchains - 1) : 0;
+    lt.assign(1 + nr, 0);
+    lt[0] = 1;
+    if (nr) {
+      std::vector<unsigned long long> acc(nr), base(nr);
+      RFINV_CUDA_CHECK(cudaMemcpy(acc.data(), d.rs_nacc, sizeof(unsigned long long) * nr, cudaMemcpyDeviceToHost));
+      RFINV_CUDA_CHECK(cudaMemcpy(base.data(), d.rs_base, sizeof(unsigned long long) * nr, cudaMemcpyDeviceToHost));
+      for (size_t i = 0; i < nr; ++i) lt[1 + i] = (int64_t)(acc[i] - base[i]);
+    }
+  }
+  hd.n_sections = (uint32_t)(ps.size() + (rs.empty() ? 0 : 1) + (lt.empty() ? 0 : 1));
   size_t total = sizeof(CkHeader) + sizeof(uint64_t);
   for (const Part& p : ps) total += sizeof(CkSection) + (size_t)p.elem * p.count;
   if (!rs.empty()) total += sizeof(CkSection) + sizeof(int64_t) * rs.size();
+  if (!lt.empty()) total += sizeof(CkSection) + sizeof(int64_t) * lt.size();
   std::unique_ptr<uint8_t[]> buf(new (std::nothrow) uint8_t[total]);
   if (!buf) { rfinv_set_error("%s: cannot allocate %zu bytes of host memory", who, total); return RFINV_ERR_IO; }
   size_t off = 0;
@@ -228,6 +246,14 @@ int32_t rfinv_pt_save(rfinv_handle* h, const char* path) {
     sc.elem_size = sizeof(int64_t); sc.count = rs.size();
     std::memcpy(buf.get() + off, &sc, sizeof(sc)); off += sizeof(sc);
     std::memcpy(buf.get() + off, rs.data(), sizeof(int64_t) * rs.size()); off += sizeof(int64_t) * rs.size();
+  }
+  if (!lt.empty()) {
+    CkSection sc;
+    std::memset(&sc, 0, sizeof(sc));
+    std::snprintf(sc.name, sizeof(sc.name), "%s", LT_SECTION);
+    sc.elem_size = sizeof(int64_t); sc.count = lt.size();
+    std::memcpy(buf.get() + off, &sc, sizeof(sc)); off += sizeof(sc);
+    std::memcpy(buf.get() + off, lt.data(), sizeof(int64_t) * lt.size()); off += sizeof(int64_t) * lt.size();
   }
   const uint64_t sum = xxh64(buf.get(), off);
   std::memcpy(buf.get() + off, &sum, sizeof(sum));
@@ -368,6 +394,15 @@ int32_t rfinv_pt_restore(rfinv_handle* h, const char* path) {
   }
   if (rs_it != found.end() && (rs_it->second.second.elem_size != sizeof(int64_t) || rs_it->second.second.count != 1 + 2 * (uint64_t)nl))
     return io_error(who, file, "section 'rank_swaps' is malformed");
+  // the ladder tuning likewise (rfinv_pt_set_ladder_tuning before restoring)
+  const auto lt_it = found.find(LT_SECTION);
+  if ((lt_it != found.end()) != (d.rs_tune != 0)) {
+    rfinv_set_error("%s: %s was written with the ladder tuning %s, this handle has it %s (rfinv_pt_set_ladder_tuning before restore)",
+                    who, path, lt_it != found.end() ? "on" : "off", d.rs_tune ? "on" : "off");
+    return RFINV_ERR_ARG;
+  }
+  if (lt_it != found.end() && (lt_it->second.second.elem_size != sizeof(int64_t) || lt_it->second.second.count != 1 + (uint64_t)d.G * nl))
+    return io_error(who, file, "section 'ladder_tuning' is malformed");
   if (hd.it_done < 0) return io_error(who, file, "negative iteration count");
   const std::vector<Part> ps = parts(h, hd.it_done, n_models);
   for (const Part& p : ps) {
@@ -397,6 +432,13 @@ int32_t rfinv_pt_restore(rfinv_handle* h, const char* path) {
     std::memcpy(rows.data(), rs.data() + 1 + nl, sizeof(int64_t) * nl);
     RFINV_CUDA_CHECK(cudaMemcpy(d.rs_nprop, rs.data() + 1, sizeof(int64_t) * nl, cudaMemcpyHostToDevice));
     RFINV_CUDA_CHECK(cudaMemcpy(d.rs_nacc, rows.data(), sizeof(int64_t) * rows.size(), cudaMemcpyHostToDevice));
+    if (lt_it != found.end()) {   // snapshot = restored row - acceptances of the round (modulo 2^64)
+      std::vector<int64_t> round((size_t)d.G * nl);
+      std::memcpy(round.data(), buf.data() + lt_it->second.first + sizeof(int64_t), sizeof(int64_t) * round.size());
+      std::vector<unsigned long long> base(round.size());
+      for (size_t i = 0; i < base.size(); ++i) base[i] = (unsigned long long)rows[i] - (unsigned long long)round[i];
+      RFINV_CUDA_CHECK(cudaMemcpy(d.rs_base, base.data(), sizeof(unsigned long long) * base.size(), cudaMemcpyHostToDevice));
+    }
   }
   s->it_done = hd.it_done;
   s->n_eval = hd.n_eval_host;

@@ -744,26 +744,84 @@ __device__ __forceinline__ uint64_t philox4x64_w0(uint64_t c0, uint64_t c1, uint
 // exchange their temperatures in temps and in the swap table.  peer: the peer-memory exchange, where pt_finish_kernel has
 // already advanced *it_dev and the table alternates.  DECIDE (single process): the last CTA then takes the global swap
 // decision that pt_finish_kernel<false, true> takes without the sweep.
+// With the ladder tuning on (p.rs_tune), the iterations e - 1 of the tuning points e then retune every rank's ladder
+// (pt_tune_ladder) before the global swap reads the table.
 constexpr int PT_RS_WARPS = 4;
+
+// chain of the rank at each level: its place among the chains c0 .. c0 + n - 1 sorted by (temperature, chain index)
+__device__ __forceinline__ void pt_rank_levels(const PtDev& p, int c0, int n, int lane, int* at) {
+  for (int a = lane; a < n; a += 32) {
+    const double ta = p.temps[c0 + a];
+    int lvl = 0;
+    for (int b = 0; b < n; ++b) { const double tb = p.temps[c0 + b]; lvl += tb < ta || (tb == ta && b < a); }
+    at[lvl] = a;
+  }
+  __syncwarp();
+}
+
+// Ladder tuning of virtual rank r at tuning point e (DESIGN.md 7d; the C reference is lo_tune_rank in tests/ladder_oracle.c):
+// the levels a+1 .. n-2 above the cold anchor a take the inverse temperatures that split the rank's rejection barrier
+// Lambda -- the running sum of the per-pair rejection rates of the round [s, e) -- into equal parts, interpolated linearly in
+// beta between the old levels.  One warp; the levels and the old ladder go to shared memory, lane 0 does the O(n) walk.
+// Every operation is rounded on its own, as in the reference.
+__device__ void pt_tune_ladder(const PtDev& p, double* __restrict__ table, int r, int e, int lane, int* at, double* lt) {
+  const int n = p.nchains, c0 = r * n, nl = n - 1;
+  pt_rank_levels(p, c0, n, lane, at);   // the sweep has just exchanged temperatures
+  for (int l = lane; l < n; l += 32) lt[l] = p.temps[c0 + at[l]];
+  __syncwarp();
+  unsigned long long* acc = p.rs_nacc + (size_t)r * nl;
+  unsigned long long* base = p.rs_base + (size_t)r * nl;
+  if (lane == 0) {
+    const double cold = 1.0 + (double)1.0e-6f;
+    int c = 0;
+    while (c < n && lt[c] <= cold) ++c;   // the cold chains are the lowest levels
+    const int a = c > 0 ? c - 1 : 0, K = nl - a;
+    if (K >= 2) {
+      const int s = e == 64 ? 0 : e / 2;
+      const double P = (double)((e - s) / 2);
+      auto rho = [&](int l) {
+        const double q = __ddiv_rn((double)(acc[l] - base[l]), P);
+        const double x = __dsub_rn(1.0, q);
+        return x < 0x1p-10 ? 0x1p-10 : x;
+      };
+      double LK = 0.0;
+      for (int m = 0; m < K; ++m) LK = __dadd_rn(LK, rho(a + m));
+      // pass 0 checks the guard, pass 1 writes; both walk the same ladder (the new T' are read from the old ladder lt only)
+      for (int pass = 0; pass < 2; ++pass) {
+        int m = 0;
+        double Lm = 0.0, Lm1 = rho(a), prev = lt[a];
+        bool ok = true;
+        for (int k = 1; k < K; ++k) {
+          const double lam = __ddiv_rn(__dmul_rn(LK, (double)k), (double)K);
+          while (m < K - 1 && !(lam < Lm1)) { ++m; Lm = Lm1; Lm1 = __dadd_rn(Lm1, rho(a + m)); }
+          const double f = __ddiv_rn(__dsub_rn(lam, Lm), __dsub_rn(Lm1, Lm));
+          const double bm = __ddiv_rn(1.0, lt[a + m]), bm1 = __ddiv_rn(1.0, lt[a + m + 1]);
+          const double t = __ddiv_rn(1.0, __dadd_rn(bm, __dmul_rn(f, __dsub_rn(bm1, bm))));
+          if (pass == 0) { ok = ok && t > prev && t > cold; prev = t; }
+          else { const int ch = c0 + at[a + k]; p.temps[ch] = t; table[ch] = t; }
+        }
+        if (pass == 0 && !(ok && lt[nl] > prev)) break;   // the guard: this rank keeps its ladder for this round
+      }
+    }
+  }
+  __syncwarp();
+  for (int l = lane; l < nl; l += 32) base[l] = acc[l];
+}
+
 template <bool DECIDE>
 __global__ void __launch_bounds__(32 * PT_RS_WARPS) pt_rank_swap_kernel(const PtDev p, double* __restrict__ table, int table_len,
                                                                         int peer) {
-  extern __shared__ int rs_at[];   // [warps][nchains]: chain at each level
+  // [warps][nchains] chain at each level; with the ladder tuning on, [warps][nchains] doubles of the old ladder first
+  extern __shared__ double rs_smem[];
   __shared__ int s_last;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, n = p.nchains;
   const int r = blockIdx.x * (blockDim.x >> 5) + warp;
   const int it = *p.it_dev - peer;
   if (peer) table += (size_t)(it & 1) * table_len;
   if (r < p.G) {
-    int* at = rs_at + (size_t)warp * n;
+    int* at = (int*)(rs_smem + (p.rs_tune ? (size_t)(blockDim.x >> 5) * n : 0)) + (size_t)warp * n;
     const int c0 = r * n;
-    for (int a = lane; a < n; a += 32) {
-      const double ta = p.temps[c0 + a];
-      int lvl = 0;
-      for (int b = 0; b < n; ++b) { const double tb = p.temps[c0 + b]; lvl += tb < ta || (tb == ta && b < a); }
-      at[lvl] = a;
-    }
-    __syncwarp();
+    pt_rank_levels(p, c0, n, lane, at);
     const uint64_t grank = (uint64_t)(p.rank_begin + r), key = (uint64_t)(uint32_t)p.iseed;
     for (int l = (it & 1) + 2 * lane; l + 1 < n; l += 64) {
       const int a = c0 + at[l], b = c0 + at[l + 1];
@@ -777,6 +835,11 @@ __global__ void __launch_bounds__(32 * PT_RS_WARPS) pt_rank_swap_kernel(const Pt
     }
     if (r == 0 && lane == 0)
       for (int l = it & 1; l + 1 < n; l += 2) p.rs_nprop[l] += (unsigned long long)p.G;
+    const int e = it + 1;   // the iteration count at the end of this iteration: a tuning point?
+    if (p.rs_tune && e >= 64 && e <= p.nburn && (e & (e - 1)) == 0) {
+      __syncwarp();          // the sweep's exchanges and counts are visible to the whole warp
+      pt_tune_ladder(p, table, r, e, lane, at, rs_smem + (size_t)warp * n);
+    }
   }
   if (!DECIDE) return;
   __threadfence();   // this CTA's table entries are ordered before its arrival
@@ -1039,6 +1102,7 @@ void rfinv_handle::free_pt() {
   cudaFree(d.pk); cudaFree(d.pz); cudaFree(d.pdvp); cudaFree(d.pdvs); cudaFree(d.psig); cudaFree(d.pphi); cudaFree(d.log_r);
   cudaFree(d.log_prior12); cudaFree(d.itype); cudaFree(d.pflag); cudaFree(d.active); cudaFree(d.n_active);
   cudaFree(d.nprop); cudaFree(d.naccept); cudaFree(d.n_eval); cudaFree(d.rs_nprop); cudaFree(d.rs_nacc); cudaFree(d.rs_arrived);
+  cudaFree(d.rs_base);
   cudaFree(d.log_flags); cudaFree(d.log_itypes); cudaFree(d.log_swaps);
   cudaFree(d.nk); cudaFree(d.nz); cudaFree(d.nsig); cudaFree(d.namp); cudaFree(d.nvpz); cudaFree(d.nvsz); cudaFree(d.nvpvsz); cudaFree(d.nmod);
   cudaFree(d.vp_mean); cudaFree(d.vs_mean); cudaFree(d.vpvs_mean); cudaFree(d.vp_model); cudaFree(d.vs_model); cudaFree(d.cold_ordinal); cudaFree(d.cold_count); cudaFree(d.ocean_bin);
@@ -1227,6 +1291,53 @@ int32_t rfinv_pt_set_rank_swaps(rfinv_handle* h, int32_t mode) {
   }
   pt_drop_graphs(s);   // the captured launch sequence depends on the mode
   s->rank_swaps = mode;
+  if (mode == 0 && d.rs_tune) {   // the ladder tuning works on the sweep's counters: it goes with it
+    s->tune_points_off = pt_tuning_points(s->it_done, d.nburn);
+    d.rs_tune = 0;
+  }
+  return RFINV_OK;
+}
+
+int32_t rfinv_pt_set_ladder_tuning(rfinv_handle* h, int32_t on) {
+  static const char* who = "rfinv_pt_set_ladder_tuning";
+  int st = pt_require(h, who);
+  if (st != RFINV_OK) return st;
+  PtState* s = h->pt;
+  PtDev& d = s->dev;
+  if (on != 0 && on != 1) { rfinv_set_error("%s: %d (0: off, 1: tune the ladders during the burn-in)", who, on); return RFINV_ERR_ARG; }
+  if (s->step_pending) {
+    rfinv_set_error("%s: an iteration is half done (rfinv_pt_local_step without rfinv_pt_apply_swap)", who);
+    return RFINV_ERR_STATE;
+  }
+  if (s->reduced) { rfinv_set_error("%s: rfinv_pt_reduce_outputs has run", who); return RFINV_ERR_STATE; }
+  if (on && !d.rs_tune) {
+    if (s->it_done > 0) {
+      rfinv_set_error("%s: %d iterations have run; the tuning starts with the run (before its first iteration or a restore)", who, s->it_done);
+      return RFINV_ERR_STATE;
+    }
+    if (s->rank_swaps != 1) { rfinv_set_error("%s: the tuning needs the rank swaps on (rfinv_pt_set_rank_swaps(h, 1) first)", who); return RFINV_ERR_STATE; }
+    // the kernel keeps a rank's ladder and its levels in shared memory
+    if ((sizeof(int) + sizeof(double)) * (size_t)d.nchains > 200 * 1024) {
+      rfinv_set_error("%s: nchains = %d is beyond the %d chains per rank the tuning supports", who, d.nchains, (int)(200 * 1024 / 12));
+      return RFINV_ERR_ARG;
+    }
+  }
+  RFINV_CUDA_CHECK(cudaSetDevice(h->device));
+  RFINV_CUDA_CHECK(cudaStreamSynchronize(h->stream));
+  if (on && d.nchains >= 2 && !d.rs_base)
+    if ((st = dalloc(&d.rs_base, (size_t)d.G * (d.nchains - 1))) != RFINV_OK) return st;
+  if (!on && d.rs_tune) s->tune_points_off = pt_tuning_points(s->it_done, d.nburn);
+  pt_drop_graphs(s);   // the captured launches carry the flag
+  d.rs_tune = on;
+  return RFINV_OK;
+}
+
+int32_t rfinv_pt_get_ladder_tuning(rfinv_handle* h, int32_t* on, int32_t* n_points) {
+  int st = pt_require(h, "rfinv_pt_get_ladder_tuning");
+  if (st != RFINV_OK) return st;
+  const PtState* s = h->pt;
+  if (on) *on = s->dev.rs_tune;
+  if (n_points) *n_points = s->dev.rs_tune ? pt_tuning_points(s->it_done, s->dev.nburn) : s->tune_points_off;
   return RFINV_OK;
 }
 
@@ -1325,7 +1436,7 @@ static int pt_enqueue_local(rfinv_handle* h, bool record, bool peer_exchange = f
   }
   if (sweep) {   // after the bookkeeping (it sees the temperatures at acceptance), before the global swap reads the table
     const int warps = d.nchains <= 3072 ? PT_RS_WARPS : 1;
-    const size_t smem = sizeof(int) * (size_t)d.nchains * warps;
+    const size_t smem = (sizeof(int) + (d.rs_tune ? sizeof(double) : 0)) * (size_t)d.nchains * warps;
     const unsigned nb = (unsigned)((d.G + warps - 1) / warps);
     if (fuse_swap && !peer) {
       RFINV_CUDA_CHECK(rfinv_raise_smem_limit((const void*)pt_rank_swap_kernel<true>, smem));

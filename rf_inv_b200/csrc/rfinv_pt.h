@@ -47,6 +47,9 @@ struct PtDev {
   unsigned long long* rs_nprop;   // [nchains - 1] proposals per level, summed over the local ranks
   unsigned long long* rs_nacc;    // [G][nchains - 1] accepted swaps per rank and level (rows: no same-address atomics)
   int* rs_arrived;                // arrival counter of pt_rank_swap_kernel
+  // ladder tuning during the burn-in (rfinv_pt_set_ladder_tuning, DESIGN.md 7d); allocated by the first switch on
+  unsigned long long* rs_base;    // [G][nchains - 1] rs_nacc at the last tuning point: the acceptances of a round are the difference
+  int rs_tune;                    // 1: pt_rank_swap_kernel retunes the ladders at the tuning points
 };
 
 struct ncclComm;   // NCCL communicator (comm.cu)
@@ -119,7 +122,15 @@ struct PtState {
   bool step_pending = false;   // rfinv_pt_local_step has run, rfinv_pt_apply_swap not yet: no checkpoint in between
   bool reduced = false;        // rfinv_pt_reduce_outputs has run: the bookkeeping may hold job-wide sums
   int rank_swaps = 0;          // rfinv_pt_set_rank_swaps: 0 the reference's global swap only, 1 the rank sweep before it
+  int tune_points_off = 0;     // tuning points passed while the ladder tuning was on, frozen when it is switched off
 };
 
 // does an iteration of this state run the rank sweep?  (nothing to pair with fewer than two chains per rank)
 inline bool pt_sweeps(const PtState* s) { return s->rank_swaps == 1 && s->dev.nchains >= 2; }
+
+// the tuning points e = 2^j, j >= 6, e <= nburn among the first it_done iterations (DESIGN.md 7d)
+inline int pt_tuning_points(int it_done, int nburn) {
+  int n = 0;
+  for (long long e = 64; e <= it_done && e <= nburn; e *= 2) ++n;
+  return n;
+}

@@ -9,7 +9,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
-from typing import Dict, Optional
+from typing import Dict, Optional, Tuple
 
 import numpy as np
 
@@ -132,6 +132,20 @@ class ParallelTempering:
         n_prop = np.zeros(n, dtype=np.int64); n_acc = np.zeros(n, dtype=np.int64)
         capi.check(self._lib.rfinv_pt_get_rank_swaps(self.ev.handle, C.byref(mode), _p(n_prop, capi.i64p), _p(n_acc, capi.i64p)))
         return dict(mode=int(mode.value), n_prop=n_prop, n_acc=n_acc)
+
+    # -- ladder tuning during the burn-in (DESIGN.md 7d) -------------------------------------------------------------
+    def set_ladder_tuning(self, on: bool) -> None:
+        """On top of set_rank_swaps(1), before the first iteration (and before restore()): at the iteration counts 64, 128,
+        256, ... up to N_BURN every virtual rank respaces the temperatures of its levels above the cold ones towards equal
+        neighbour-swap rejection rates.  The ladders stay fixed after the burn-in.  Off is allowed between runs;
+        set_rank_swaps(0) switches it off too."""
+        capi.check(self._lib.rfinv_pt_set_ladder_tuning(self.ev.handle, int(on)))
+
+    def ladder_tuning(self) -> Tuple[bool, int]:
+        """(on, number of tuning points passed with the tuning on)."""
+        on, n = C.c_int32(0), C.c_int32(0)
+        capi.check(self._lib.rfinv_pt_get_ladder_tuning(self.ev.handle, C.byref(on), C.byref(n)))
+        return bool(on.value), int(n.value)
 
     # -- results ----------------------------------------------------------------------------------
     def set_logging(self, cap_iters: int) -> None:

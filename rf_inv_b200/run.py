@@ -16,7 +16,11 @@ params file alone writes.  The stations must agree on N_BURN, N_ITER and N_CORR 
 i % world == r as its group on its own GPU; the processes do not communicate.
 
 ``--rank-swaps`` adds even/odd temperature swaps between neighbouring levels inside every virtual rank (DESIGN.md 7c).  The
-reference's files are written as without it, plus OUT_DIR/rank_swaps with the acceptance of each neighbour pair."""
+reference's files are written as without it, plus OUT_DIR/rank_swaps with the acceptance of each neighbour pair.
+
+``--tune-ladder`` (implies ``--rank-swaps``) also retunes every virtual rank's temperature ladder at the iteration counts 64,
+128, 256, ... up to N_BURN towards equal neighbour-swap rejection rates (DESIGN.md 7d); the ladders are fixed after the
+burn-in.  It adds OUT_DIR/ladder: one line per virtual rank, its temperatures by level (coldest first) at the end of the run."""
 from __future__ import annotations
 
 import argparse
@@ -56,6 +60,20 @@ def write_rank_swaps(out_dir: str, rs) -> None:
             f.write(f"{l:5d} {int(a):12d} {int(n):12d} {a / n if n else 0.0:12.6f}\n")
 
 
+def rank_ladders(pt) -> np.ndarray:
+    """[local ranks][nchains]: each virtual rank's temperatures sorted by (temperature, chain index), coldest first."""
+    t = pt.state()["temps"].reshape(pt.rank_count, pt.cfg.nchains)
+    idx = np.arange(pt.cfg.nchains)
+    return np.take_along_axis(t, np.lexsort((np.broadcast_to(idx, t.shape), t), axis=1), axis=1)
+
+
+def write_ladder(out_dir: str, ladders) -> None:
+    """OUT_DIR/ladder: one line per virtual rank, its temperatures by level."""
+    with open(os.path.join(out_dir, "ladder"), "w") as f:
+        for row in ladders:
+            f.write(" ".join(f"{t:.17g}" for t in row) + "\n")
+
+
 def print_rank_swaps(rs) -> None:
     print(" --- Swaps between neighbouring temperature levels inside the ranks ---")
     for l, (a, n) in enumerate(zip(rs["n_acc"], rs["n_prop"]), start=1):
@@ -63,10 +81,12 @@ def print_rank_swaps(rs) -> None:
 
 
 def run(params_path: str, nproc: int, verbose: bool = True, n_iter: int = None, checkpoint: str = None,
-        checkpoint_every: int = None, resume: bool = False, rank_swaps: bool = False):
+        checkpoint_every: int = None, resume: bool = False, rank_swaps: bool = False, tune_ladder: bool = False):
     """checkpoint: save the state to this path every `checkpoint_every` iterations (rounded up to the progress steps; default:
     every progress step) and at the end.  resume: restore it first if it exists and continue from its iteration count.
-    rank_swaps: the even/odd sweep inside every virtual rank (ParallelTempering.set_rank_swaps(1)); adds OUT_DIR/rank_swaps."""
+    rank_swaps: the even/odd sweep inside every virtual rank (ParallelTempering.set_rank_swaps(1)); adds OUT_DIR/rank_swaps.
+    tune_ladder: implies rank_swaps, plus the ladder tuning during the burn-in (set_ladder_tuning(1)); adds OUT_DIR/ladder."""
+    rank_swaps = rank_swaps or tune_ladder
     if resume and not checkpoint:
         raise ValueError("resume needs a checkpoint path")
     if checkpoint_every is not None and checkpoint_every < 1:
@@ -90,6 +110,8 @@ def run(params_path: str, nproc: int, verbose: bool = True, n_iter: int = None, 
     pt = ParallelTempering(cfg, nproc, device=local_rank, world=world, rank=rank)
     if rank_swaps:                                        # before a restore: the checkpoint holds the sweep's counters
         pt.set_rank_swaps(1)
+    if tune_ladder:
+        pt.set_ladder_tuning(1)
     n_tot = cfg.nburn + cfg.niter if n_iter is None else n_iter
     ck = checkpoint_path(checkpoint, world, rank) if checkpoint else None
     if resume:
@@ -121,6 +143,11 @@ def run(params_path: str, nproc: int, verbose: bool = True, n_iter: int = None, 
         if ck and (done - saved >= every or done == n_tot):   # always at the end
             pt.save(ck)
             saved = done
+    ladders = rank_ladders(pt) if tune_ladder else None
+    if tune_ladder and world > 1:                         # process 0 writes the rows of every process, in rank order
+        rows = [None] * world
+        dist.all_gather_object(rows, ladders)
+        ladders = np.concatenate(rows)
     if world > 1:                                         # the reference's mpi_reduce / mpi_gather (src/mcmc_out.f90:52-93)
         pt.reduce_outputs()                               # ncclReduce / ncclSend+Recv inside the library: process 0 is job-wide now
     hist, cnt = pt.hist(), pt.counters()
@@ -135,6 +162,8 @@ def run(params_path: str, nproc: int, verbose: bool = True, n_iter: int = None, 
         rio.write_outputs(cfg, cfg.out_dir, nproc, hist, lh, vp_model, vs_model)
         if rs:
             write_rank_swaps(cfg.out_dir, rs)
+        if ladders is not None:
+            write_ladder(cfg.out_dir, ladders)
     pt.close()
     if world > 1:
         dist.destroy_process_group()
@@ -166,9 +195,10 @@ def load_stations(params_paths):
 
 
 def run_group(params_paths, nproc: int, verbose: bool = True, n_iter: int = None, checkpoint: str = None,
-              checkpoint_every: int = None, resume: bool = False, rank_swaps: bool = False):
+              checkpoint_every: int = None, resume: bool = False, rank_swaps: bool = False, tune_ladder: bool = False):
     """Several stations (one params file each) as one group on one GPU; arguments as in run().  Under torchrun process r
     takes the stations i with i % world == r.  Returns {station index: (hist, counters)} of this process's stations."""
+    rank_swaps = rank_swaps or tune_ladder
     if resume and not checkpoint:
         raise ValueError("resume needs a checkpoint path")
     if checkpoint_every is not None and checkpoint_every < 1:
@@ -197,6 +227,8 @@ def run_group(params_paths, nproc: int, verbose: bool = True, n_iter: int = None
         if rank_swaps:
             for pt in pts:
                 pt.set_rank_swaps(1)
+                if tune_ladder:
+                    pt.set_ladder_tuning(1)
         if restore:
             for i, pt in zip(mine, pts):
                 pt.restore(cks[i])
@@ -234,6 +266,8 @@ def run_group(params_paths, nproc: int, verbose: bool = True, n_iter: int = None
             rio.write_outputs(cfg, cfg.out_dir, nproc, hist, cnt["likelihood_hist"], vp_model, vs_model)
             if rank_swaps:
                 write_rank_swaps(cfg.out_dir, pt.rank_swaps())
+            if tune_ladder:
+                write_ladder(cfg.out_dir, rank_ladders(pt))
             out[i] = (hist, cnt)
         return out
     finally:
@@ -257,15 +291,18 @@ def main(argv=None):
     ap.add_argument("--rank-swaps", action="store_true",
                     help="also swap temperatures between neighbouring levels inside every virtual rank, even and odd pairs "
                          "in turn (writes OUT_DIR/rank_swaps)")
+    ap.add_argument("--tune-ladder", action="store_true",
+                    help="with --rank-swaps (implied): retune every rank's temperature ladder during the burn-in towards equal "
+                         "swap rejection rates between neighbouring levels (writes OUT_DIR/ladder)")
     a = ap.parse_args(argv)
     if a.resume and not a.checkpoint:
         ap.error("--resume needs --checkpoint")
     if len(a.params) == 1:
         run(a.params[0], a.nproc, n_iter=a.iters, checkpoint=a.checkpoint, checkpoint_every=a.checkpoint_every, resume=a.resume,
-            rank_swaps=a.rank_swaps)
+            rank_swaps=a.rank_swaps, tune_ladder=a.tune_ladder)
     else:
         run_group(a.params, a.nproc, n_iter=a.iters, checkpoint=a.checkpoint, checkpoint_every=a.checkpoint_every,
-                  resume=a.resume, rank_swaps=a.rank_swaps)
+                  resume=a.resume, rank_swaps=a.rank_swaps, tune_ladder=a.tune_ladder)
 
 
 if __name__ == "__main__":

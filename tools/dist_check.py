@@ -5,7 +5,8 @@ rfinv_pt_run_distributed (in-library ncclAllGather, CUDA graph) equal those of O
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29511 tools/dist_check.py
 
 --rank-swaps runs both sides with the even/odd sweep inside every virtual rank (set_rank_swaps(1)) and also compares its
-job-wide counters.
+job-wide counters.  --tune-ladder adds the ladder tuning during the burn-in (set_ladder_tuning(1), implies --rank-swaps), with
+burn-ins and run lengths that pass two or three tuning points, and also compares the number of tuning points passed.
 """
 import faulthandler, hashlib, json, os, signal, sys
 faulthandler.register(signal.SIGTERM, all_threads=True, chain=False)
@@ -19,7 +20,7 @@ from rf_inv_b200.evaluator import Evaluator
 from rf_inv_b200.pt import ParallelTempering
 
 
-def identity_check(cfg, nproc_total, n_iter, world, rank, local_rank, dist, torch, rank_swaps=0):
+def identity_check(cfg, nproc_total, n_iter, world, rank, local_rank, dist, torch, rank_swaps=0, tune_ladder=False):
     """Returns (ok, detail) on every process."""
     dev = torch.device("cuda", local_rank)
     # distributed run
@@ -29,6 +30,8 @@ def identity_check(cfg, nproc_total, n_iter, world, rank, local_rank, dist, torc
     pt.set_logging(n_iter)
     if rank_swaps:
         pt.set_rank_swaps(rank_swaps)
+    if tune_ladder:
+        pt.set_ladder_tuning(1)
     pt.init_comm(dist, torch)
     say("communicator up")
     pt.run_distributed(n_iter, dist, torch)
@@ -36,6 +39,7 @@ def identity_check(cfg, nproc_total, n_iter, world, rank, local_rank, dist, torc
     say("distributed run done (exchange: %s)" % exchange)
     flags, itypes, swaps = pt.log(n_iter)
     st = pt.state()
+    tuning = pt.ladder_tuning()
     pt.reduce_outputs()
     say("outputs reduced")
     cnt = pt.counters()
@@ -50,7 +54,10 @@ def identity_check(cfg, nproc_total, n_iter, world, rank, local_rank, dist, torc
         ref.set_logging(n_iter)
         if rank_swaps:
             ref.set_rank_swaps(rank_swaps)
+        if tune_ladder:
+            ref.set_ladder_tuning(1)
         ref.run(n_iter)
+        rtuning = ref.ladder_tuning()
         rf, ri, rs = ref.log(n_iter)
         rst = ref.state()
         rcnt = ref.counters()
@@ -58,7 +65,7 @@ def identity_check(cfg, nproc_total, n_iter, world, rank, local_rank, dist, torc
         rrsw = ref.rank_swaps() if rank_swaps else None
         ref.close()
         say("reference run done")
-        box = [dict(flags=rf, itypes=ri, swaps=rs, state=rst)]
+        box = [dict(flags=rf, itypes=ri, swaps=rs, state=rst, tuning=rtuning)]
     else:
         box = [None]
     dist.broadcast_object_list(box, src=0)
@@ -70,6 +77,8 @@ def identity_check(cfg, nproc_total, n_iter, world, rank, local_rank, dist, torc
                  swaps=np.array_equal(swaps, r["swaps"]))
     for k in ("k", "z", "dvp", "dvs", "sig", "logl", "temps"):
         parts["state_" + k] = np.array_equal(st[k], r["state"][k][sl])
+    if tune_ladder:
+        parts["ladder_tuning"] = tuning == r["tuning"] and tuning[0] and tuning[1] >= 2
     detail = {}
     if rank == 0:
         parts["nprop"] = np.array_equal(cnt["nprop"], rcnt["nprop"]); parts["naccept"] = np.array_equal(cnt["naccept"], rcnt["naccept"])
@@ -100,9 +109,14 @@ if __name__ == "__main__":
     torch.cuda.set_device(local_rank)
     os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
     dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
-    rank_swaps = 1 if "--rank-swaps" in sys.argv[1:] else 0
+    tune_ladder = "--tune-ladder" in sys.argv[1:]
+    rank_swaps = 1 if "--rank-swaps" in sys.argv[1:] or tune_ladder else 0
     out = {}
-    for name, nproc, iters, kw in (("sample", 4 * world, 300, dict(nburn=100, niter=200)), ("c4", 8 * world, 120, dict()), ("target", 16 * world, 60, dict())):
+    runs = (("sample", 4 * world, 300, dict(nburn=100, niter=200)), ("c4", 8 * world, 120, dict()), ("target", 16 * world, 60, dict()))
+    if tune_ladder:   # tuning points 64, 128, 256 / 64, 128, inside and at the end of the burn-in
+        runs = (("sample", 4 * world, 300, dict(nburn=280, niter=20)), ("c4", 8 * world, 140, dict(nburn=128)),
+                ("target", 16 * world, 130, dict(nburn=200)))
+    for name, nproc, iters, kw in runs:
         cfg = workloads.make_config(name)
         for k_, v_ in kw.items():
             setattr(cfg, k_, v_)
@@ -114,7 +128,7 @@ if __name__ == "__main__":
         with Evaluator(cfg, device=local_rank) as ev:
             _, rft, _ = ev.calc_likelihood(tm["k"], tm["z"], tm["dvp"], tm["dvs"], tm["sig"], want_rft=True)
         cfg.obs = (rft[0, :, :cfg.nsmp] + np.random.default_rng(7).normal(0.0, 0.01, (cfg.ntrc, cfg.nsmp))).astype(np.float32).astype(np.float64)
-        ok, detail = identity_check(cfg, nproc, iters, world, rank, local_rank, dist, torch, rank_swaps)
+        ok, detail = identity_check(cfg, nproc, iters, world, rank, local_rank, dist, torch, rank_swaps, tune_ladder)
         out[name] = dict(identical=ok, world=world, virtual_ranks=nproc, iterations=iters, **detail)
     if rank == 0:
         print(json.dumps(out), flush=True)
