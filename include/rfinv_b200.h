@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define RFINV_ABI_VERSION 7
+#define RFINV_ABI_VERSION 8
 
 /* status codes */
 #define RFINV_OK 0
@@ -318,6 +318,25 @@ int32_t rfinv_pt_get_rank_swaps(rfinv_handle* h, int32_t* mode, int64_t* n_prop,
 int32_t rfinv_pt_set_ladder_tuning(rfinv_handle* h, int32_t on);
 /* The setting and the number of tuning points passed with it on; either pointer may be NULL. */
 int32_t rfinv_pt_get_ladder_tuning(rfinv_handle* h, int32_t* on, int32_t* n_points);
+
+/* ---- random-walk width tuning during the burn-in (ABI version 8, DESIGN.md 7e) ----------------------------------------------
+ * On top of the rank sweep (mode 1), independent of the ladder tuning: the chains at level l of virtual rank r propose the
+ * moves z, dVs, dVp and sigma with width dev_tau * scale[r][l][tau] (scale 1 when switched on); the two chains of the
+ * previous iteration's global swap propose with the params.in widths.  At the tuning points e = 64, 128, 256, ... <= nburn
+ * (inside iteration e - 1, after the sweep and the ladder tuning) every (rank, level, type) with at least 16 proposals since
+ * the previous point multiplies its scale by (acceptance / target) clamped to [1/2, 2], the scale staying in [2^-8, 2^8].
+ * After the burn-in the widths stay fixed.  Off (the default) leaves the mode-1 run bit for bit as it is.  A checkpoint
+ * restores only into a handle with the same setting and target; a distributed run needs it on every process.
+ * on: 0/1; target in (0, 1), e.g. 0.44.
+ * RFINV_ERR_ARG: on other than 0 or 1, a target outside (0, 1), or switching it on with nchains < 2.  RFINV_ERR_STATE:
+ * switching it on without rfinv_pt_init, after an iteration has run, or while the rank swaps are not mode 1; either way
+ * between rfinv_pt_local_step and rfinv_pt_apply_swap or after rfinv_pt_reduce_outputs.  Off returns the widths to the
+ * params.in values; rfinv_pt_set_rank_swaps(h, 0) switches the tuning off as well. */
+int32_t rfinv_pt_set_step_tuning(rfinv_handle* h, int32_t on, double target);
+/* widths[G][nchains][4]: absolute dev_tau * scale in the order z, dvs, dvp, sig (params.in value for a type the run does not
+ * propose); n_prop / n_acc [G][nchains][4] since the last tuning point; any pointer may be NULL */
+int32_t rfinv_pt_get_step_tuning(rfinv_handle* h, int32_t* on, double* target, int32_t* n_points, double* widths,
+                                 int64_t* n_prop, int64_t* n_acc);
 
 /* ---- file formats either side of the path (host only, no CUDA) ---------------------------------------
  * params.in (positional, '#' comment lines; src/params.f90:101-405), SAC traces cut to [T_START, T_END]

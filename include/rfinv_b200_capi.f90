@@ -232,6 +232,24 @@ module rfinv_b200_capi
        integer(c_int32_t), intent(out) :: on, n_points
      end function rfinv_pt_get_ladder_tuning
 
+     ! random-walk width tuning during the burn-in on top of the rank swaps (ABI version 8): on 0 or 1, target in (0, 1)
+     integer(c_int32_t) function rfinv_pt_set_step_tuning(handle, on, target) bind(C, name="rfinv_pt_set_step_tuning")
+       import :: c_int32_t, c_double, c_ptr
+       type(c_ptr), value :: handle
+       integer(c_int32_t), value :: on
+       real(c_double), value :: target
+     end function rfinv_pt_set_step_tuning
+
+     ! the setting, target, tuning points passed; widths / n_prop / n_acc (4, nchains, rank_count) in the order z, dvs, dvp, sig
+     integer(c_int32_t) function rfinv_pt_get_step_tuning(handle, on, target, n_points, widths, n_prop, n_acc) &
+         bind(C, name="rfinv_pt_get_step_tuning")
+       import :: c_int32_t, c_int64_t, c_double, c_ptr
+       type(c_ptr), value :: handle
+       integer(c_int32_t), intent(out) :: on, n_points
+       real(c_double), intent(out) :: target, widths(*)
+       integer(c_int64_t), intent(out) :: n_prop(*), n_acc(*)
+     end function rfinv_pt_get_step_tuning
+
      ! several stations advanced together (ABI version 5): handles(n) are the c_ptr of n handles after rfinv_pt_init
      integer(c_int32_t) function rfinv_pt_group_create(handles, n, group) bind(C, name="rfinv_pt_group_create")
        import :: c_int32_t, c_ptr

@@ -76,6 +76,8 @@ SIGNATURES = {
     "rfinv_pt_get_rank_swaps": (C.c_int32, [C.c_void_p, i32p, i64p, i64p]),
     "rfinv_pt_set_ladder_tuning": (C.c_int32, [C.c_void_p, C.c_int32]),
     "rfinv_pt_get_ladder_tuning": (C.c_int32, [C.c_void_p, i32p, i32p]),
+    "rfinv_pt_set_step_tuning": (C.c_int32, [C.c_void_p, C.c_int32, C.c_double]),
+    "rfinv_pt_get_step_tuning": (C.c_int32, [C.c_void_p, i32p, C.POINTER(C.c_double), i32p, C.POINTER(C.c_double), i64p, i64p]),
     "rfinv_problem_load": (C.c_int32, [C.c_char_p, C.c_char_p, C.POINTER(C.c_void_p)]),
     "rfinv_problem_free": (None, [C.c_void_p]),
     "rfinv_problem_config": (C.POINTER(RfinvConfigC), [C.c_void_p]),

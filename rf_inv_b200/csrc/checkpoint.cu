@@ -147,6 +147,11 @@ std::vector<Part> parts(rfinv_handle* h, int it_done, long long n_models) {
                        {"ocean_bin", d.ocean_bin, 1, nz},
                        {"vp_model", d.vp_model, 8, (uint64_t)n_models * nz}, {"vs_model", d.vs_model, 8, (uint64_t)n_models * nz}});
   }
+  if (d.st_on) {   // the step tuning (rfinv_pt_set_step_tuning), only with it on: a file without it keeps its sections
+    const uint64_t rows = G * d.nchains * 4;
+    v.insert(v.end(), {{"step_scale", d.st_scale, 8, rows}, {"step_nprop", d.st_nprop, 8, rows}, {"step_nacc", d.st_nacc, 8, rows},
+                       {"step_lvl", d.st_lvl, 4, Cl}, {"step_pair", d.st_pair, 4, 2}});
+  }
   return v;
 }
 
@@ -158,6 +163,8 @@ constexpr const char* RS_SECTION = "rank_swaps";
 // restore rebuilds the snapshot rows as (restored rows) - (acceptances of the round): the next tuning point sees the counts
 // of an uninterrupted run.
 constexpr const char* LT_SECTION = "ladder_tuning";
+// The step tuning's setting, written only with it on: double [target].  Its device arrays are sections of parts().
+constexpr const char* ST_SECTION = "step_tuning";
 
 int io_error(const char* who, const std::string& path, const char* what) {
   rfinv_set_error("%s: %s: %s", who, path.c_str(), what);
@@ -220,11 +227,12 @@ int32_t rfinv_pt_save(rfinv_handle* h, const char* path) {
       for (size_t i = 0; i < nr; ++i) lt[1 + i] = (int64_t)(acc[i] - base[i]);
     }
   }
-  hd.n_sections = (uint32_t)(ps.size() + (rs.empty() ? 0 : 1) + (lt.empty() ? 0 : 1));
+  hd.n_sections = (uint32_t)(ps.size() + (rs.empty() ? 0 : 1) + (lt.empty() ? 0 : 1) + (d.st_on ? 1 : 0));
   size_t total = sizeof(CkHeader) + sizeof(uint64_t);
   for (const Part& p : ps) total += sizeof(CkSection) + (size_t)p.elem * p.count;
   if (!rs.empty()) total += sizeof(CkSection) + sizeof(int64_t) * rs.size();
   if (!lt.empty()) total += sizeof(CkSection) + sizeof(int64_t) * lt.size();
+  if (d.st_on) total += sizeof(CkSection) + sizeof(double);
   std::unique_ptr<uint8_t[]> buf(new (std::nothrow) uint8_t[total]);
   if (!buf) { rfinv_set_error("%s: cannot allocate %zu bytes of host memory", who, total); return RFINV_ERR_IO; }
   size_t off = 0;
@@ -254,6 +262,14 @@ int32_t rfinv_pt_save(rfinv_handle* h, const char* path) {
     sc.elem_size = sizeof(int64_t); sc.count = lt.size();
     std::memcpy(buf.get() + off, &sc, sizeof(sc)); off += sizeof(sc);
     std::memcpy(buf.get() + off, lt.data(), sizeof(int64_t) * lt.size()); off += sizeof(int64_t) * lt.size();
+  }
+  if (d.st_on) {
+    CkSection sc;
+    std::memset(&sc, 0, sizeof(sc));
+    std::snprintf(sc.name, sizeof(sc.name), "%s", ST_SECTION);
+    sc.elem_size = sizeof(double); sc.count = 1;
+    std::memcpy(buf.get() + off, &sc, sizeof(sc)); off += sizeof(sc);
+    std::memcpy(buf.get() + off, &d.st_target, sizeof(double)); off += sizeof(double);
   }
   const uint64_t sum = xxh64(buf.get(), off);
   std::memcpy(buf.get() + off, &sum, sizeof(sum));
@@ -403,6 +419,23 @@ int32_t rfinv_pt_restore(rfinv_handle* h, const char* path) {
   }
   if (lt_it != found.end() && (lt_it->second.second.elem_size != sizeof(int64_t) || lt_it->second.second.count != 1 + (uint64_t)d.G * nl))
     return io_error(who, file, "section 'ladder_tuning' is malformed");
+  // the step tuning likewise, and with the same target (rfinv_pt_set_step_tuning before restoring)
+  const auto st_it = found.find(ST_SECTION);
+  if ((st_it != found.end()) != (d.st_on != 0)) {
+    rfinv_set_error("%s: %s was written with the step tuning %s, this handle has it %s (rfinv_pt_set_step_tuning before restore)",
+                    who, path, st_it != found.end() ? "on" : "off", d.st_on ? "on" : "off");
+    return RFINV_ERR_ARG;
+  }
+  if (st_it != found.end()) {
+    if (st_it->second.second.elem_size != sizeof(double) || st_it->second.second.count != 1)
+      return io_error(who, file, "section 'step_tuning' is malformed");
+    double target;
+    std::memcpy(&target, buf.data() + st_it->second.first, sizeof(double));
+    if (target != d.st_target) {
+      rfinv_set_error("%s: %s was written with the step tuning's target %.17g, this handle has %.17g", who, path, target, d.st_target);
+      return RFINV_ERR_ARG;
+    }
+  }
   if (hd.it_done < 0) return io_error(who, file, "negative iteration count");
   const std::vector<Part> ps = parts(h, hd.it_done, n_models);
   for (const Part& p : ps) {

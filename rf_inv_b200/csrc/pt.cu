@@ -282,6 +282,32 @@ __device__ __forceinline__ SwapPlan pt_swap_plan(const PtDev& p, double t1, doub
   return s;
 }
 
+// ---- random-walk width tuning (rfinv_pt_set_step_tuning, DESIGN.md 7e) ----
+// row of proposal type itype in the [4] of a (rank, level): 0 move z, 1 dVs, 2 dVp, 3 sigma; -1 birth and death
+__device__ __forceinline__ int pt_step_type(const PtDev& p, int itype) {
+  return itype == p.it_z ? 0 : itype == p.it_dvs ? 1 : itype == p.it_dvp ? 2 : itype == p.it_sig ? 3 : -1;
+}
+// the width chain c of local rank r proposes type tau with: the params.in width dev, times the scale of the chain's level
+// when the tuning is on -- except for the two chains of the previous iteration's global swap, whose level may depend on that
+// swap's acceptance and so on their own state (the pair rule).  The pair is loaded where it is needed, not held in registers
+// across the proposal loop: PEER, while the swap is still to be applied (px.done[0] < iteration), from its pair slot -- rank 0's
+// warp copies it to st_pair meanwhile, so st_pair is not read then --, otherwise from st_pair.  Never from the swap table,
+// whose pair entries rank 0's warp overwrites during this kernel.
+template <bool PEER>
+__device__ __forceinline__ double pt_step_width(const PtDev& p, const PtPeers& px, double dev, int tau, int r, int c) {
+  if (!p.st_on) return dev;
+  int q1, q2;
+  if (PEER && px.done[0] < *p.it_dev) {
+    const double* pr = pt_pair_slot(px.own_flag, px.world, *p.it_dev - 1);
+    q1 = (int)__ldcg(pr); q2 = (int)__ldcg(pr + 1);
+  } else {
+    q1 = p.st_pair[0]; q2 = p.st_pair[1];
+  }
+  const int gc = p.rank_begin * p.nchains + c;
+  if (gc == q1 || gc == q2) return dev;
+  return __dmul_rn(dev, p.st_scale[((size_t)r * p.nchains + p.st_lvl[c]) * 4 + tau]);
+}
+
 // STAGED: the states of the rank's chains are first brought into shared memory with coalesced loads (the chains of a rank
 // are neighbours in the chain-fastest arrays: one 128-byte line serves 16 of them) and the proposals leave the same way --
 // one memory latency per rank instead of one per chain, a third of the sectors.  Per warp: 2 x nchains x stride doubles
@@ -346,6 +372,8 @@ __global__ void __launch_bounds__(128) pt_propose_kernel(const DevConfig cfg, co
     const double* pr = pt_pair_slot(px.own_flag, px.world, it_now - 1);
     const SwapPlan sp = pt_swap_plan(p, __ldcg(pr), __ldcg(pr + 1));
     if (sp.own1 == px.me && sp.rank1_local == r) shift = 1;   // the stream of rank1 consumed the judge_pt uniform
+    // step tuning: the pair for pt_finish_kernel's counters and, at the end of a run, the next run (pt_drain_kernel otherwise)
+    if (p.st_on && r == 0 && lane == 0) { p.st_pair[0] = sp.i1; p.st_pair[1] = sp.i2; }
   }
   if (PEER) table += (size_t)(it_now & 1) * (2 * Cl + p.G + 2);   // the local table alternates: the previous one is being pushed
   Mt g(p.mt, r, p.mti[r] + shift, /*warp=*/true);
@@ -406,26 +434,26 @@ __global__ void __launch_bounds__(128) pt_propose_kernel(const DevConfig cfg, co
       } else null_flag = true;
     } else if (itype == p.it_z) {
       const int itarget = (int)(g.grnd() * (double)pk) + 1;
-      const double nz = __dadd_rn(lane_get(z0, z1, itarget - 1), __dmul_rn(gauss(g), p.dev_z));
+      const double nz = __dadd_rn(lane_get(z0, z1, itarget - 1), __dmul_rn(gauss(g), pt_step_width<PEER>(p, px, p.dev_z, 0, r, c)));
       lane_set(z0, z1, itarget - 1, nz, lane);
       if (nz < cfg.z_min || nz > cfg.z_max) null_flag = true;
     } else if (itype == p.it_dvs) {
       int itarget = (int)(g.grnd() * (double)(pk + 1)) + 1;
       if (itarget == pk + 1) itarget = km;
       const double old = lane_get(ds0, ds1, itarget - 1);
-      const double nv = __dadd_rn(old, __dmul_rn(gauss(g), p.dev_dvs));
+      const double nv = __dadd_rn(old, __dmul_rn(gauss(g), pt_step_width<PEER>(p, px, p.dev_dvs, 1, r, c)));
       lane_set(ds0, ds1, itarget - 1, nv, lane);
       log_prior12 = log_prior_ratio(nv, old, p.dvs_prior, cfg.prior_mode);
     } else if (itype == p.it_dvp) {
       int itarget = (int)(g.grnd() * (double)(pk + 1)) + 1;
       if (itarget == pk + 1) itarget = km;
       const double old = lane_get(dp0, dp1, itarget - 1);
-      const double nv = __dadd_rn(old, __dmul_rn(gauss(g), p.dev_dvp));
+      const double nv = __dadd_rn(old, __dmul_rn(gauss(g), pt_step_width<PEER>(p, px, p.dev_dvp, 2, r, c)));
       lane_set(dp0, dp1, itarget - 1, nv, lane);
       log_prior12 = log_prior_ratio(nv, old, p.dvp_prior, cfg.prior_mode);
     } else if (itype == p.it_sig) {
       const int itarget = p.isig_trc[(int)(g.grnd() * (double)p.nsig_trc)];
-      const double nv = __dadd_rn(__shfl_sync(0xffffffffu, sg, itarget), __dmul_rn(gauss(g), p.dev_sig));
+      const double nv = __dadd_rn(__shfl_sync(0xffffffffu, sg, itarget), __dmul_rn(gauss(g), pt_step_width<PEER>(p, px, p.dev_sig, 3, r, c)));
       if (lane == itarget) sg = nv;
       if (nv < p.sig_min[itarget] || nv > p.sig_max[itarget]) null_flag = true;
     }
@@ -548,6 +576,7 @@ __device__ void pt_swap_decide(const PtDev& p, const double* gathered, int world
   const double u = __ldcg(ta + 2 * Cl + rank1_local);
   const double del_s = __dmul_rn(__dsub_rn(e2, e1), __dsub_rn(__ddiv_rn(1.0, temp1), __ddiv_rn(1.0, temp2)));
   const int yn = log(u) <= del_s;
+  if (p.st_on) { p.st_pair[0] = i1; p.st_pair[1] = i2; }   // the next iteration's pair rule (step tuning)
   const int me = p.rank_begin / G;
   if (me == own1) {
     p.mti[rank1_local] += 1;  // the stream of rank1 consumed the judge_pt uniform
@@ -639,6 +668,15 @@ __global__ void __launch_bounds__(PT_FIN_THREADS) pt_finish_kernel(const DevConf
           p.k[c] = p.pk[c];
           if (flag == 1) p.slot[c] ^= 1;  // the proposal's RF samples were written to the other slot
           code = flag == 1 ? 3 : 4;
+        }
+      }
+      if (p.st_on) {   // step tuning: the proposal counts against (rank, level, type); lvl is a permutation in each rank
+        const int tau = pt_step_type(p, p.itype[c]);
+        const int gc = p.rank_begin * p.nchains + c;
+        if (tau >= 0 && gc != p.st_pair[0] && gc != p.st_pair[1]) {
+          const size_t row = ((size_t)(c - c % p.nchains) + p.st_lvl[c]) * 4 + tau;
+          p.st_nprop[row] += 1ULL;
+          p.st_nacc[row] += (unsigned long long)yn;
         }
       }
       const bool cold = temp <= 1.0 + (double)1.0e-6f;
@@ -745,7 +783,8 @@ __device__ __forceinline__ uint64_t philox4x64_w0(uint64_t c0, uint64_t c1, uint
 // already advanced *it_dev and the table alternates.  DECIDE (single process): the last CTA then takes the global swap
 // decision that pt_finish_kernel<false, true> takes without the sweep.
 // With the ladder tuning on (p.rs_tune), the iterations e - 1 of the tuning points e then retune every rank's ladder
-// (pt_tune_ladder) before the global swap reads the table.
+// (pt_tune_ladder) before the global swap reads the table.  With the step tuning on (p.st_on), every iteration records the
+// post-sweep levels (st_lvl) for the next iteration's proposals, and the tuning points' iterations tune the widths (pt_tune_steps).
 constexpr int PT_RS_WARPS = 4;
 
 // chain of the rank at each level: its place among the chains c0 .. c0 + n - 1 sorted by (temperature, chain index)
@@ -808,6 +847,27 @@ __device__ void pt_tune_ladder(const PtDev& p, double* __restrict__ table, int r
   for (int l = lane; l < nl; l += 32) base[l] = acc[l];
 }
 
+// Step tuning of virtual rank r at a tuning point (DESIGN.md 7e; the C reference is so_tune_rank in tests/step_oracle.c): every
+// (level, type) the run proposes with at least 16 proposals in the round moves its scale by the factor (acceptance / target),
+// clamped to [1/2, 2], the scale itself to [2^-8, 2^8]; every counter of the rank restarts at zero.  Lanes over the 4n entries.
+__device__ void pt_tune_steps(const PtDev& p, int r, int lane) {
+  const size_t base = (size_t)r * p.nchains * 4;
+  for (int j = lane; j < 4 * p.nchains; j += 32) {
+    const int tau = j & 3;
+    const bool proposed = tau < 2 || (tau == 2 ? p.it_dvp > 0 : p.it_sig > 0);
+    const unsigned long long P = p.st_nprop[base + j], A = p.st_nacc[base + j];
+    if (proposed && P >= 16) {
+      double f = __ddiv_rn(__ddiv_rn((double)A, (double)P), p.st_target);
+      f = f < 0.5 ? 0.5 : (f > 2.0 ? 2.0 : f);
+      double s = __dmul_rn(p.st_scale[base + j], f);
+      s = s < 0x1p-8 ? 0x1p-8 : (s > 0x1p8 ? 0x1p8 : s);
+      p.st_scale[base + j] = s;
+    }
+    p.st_nprop[base + j] = 0ULL;
+    p.st_nacc[base + j] = 0ULL;
+  }
+}
+
 template <bool DECIDE>
 __global__ void __launch_bounds__(32 * PT_RS_WARPS) pt_rank_swap_kernel(const PtDev p, double* __restrict__ table, int table_len,
                                                                         int peer) {
@@ -836,9 +896,16 @@ __global__ void __launch_bounds__(32 * PT_RS_WARPS) pt_rank_swap_kernel(const Pt
     if (r == 0 && lane == 0)
       for (int l = it & 1; l + 1 < n; l += 2) p.rs_nprop[l] += (unsigned long long)p.G;
     const int e = it + 1;   // the iteration count at the end of this iteration: a tuning point?
-    if (p.rs_tune && e >= 64 && e <= p.nburn && (e & (e - 1)) == 0) {
+    const bool tune_point = e >= 64 && e <= p.nburn && (e & (e - 1)) == 0;
+    if (p.rs_tune && tune_point) {
       __syncwarp();          // the sweep's exchanges and counts are visible to the whole warp
       pt_tune_ladder(p, table, r, e, lane, at, rs_smem + (size_t)warp * n);
+    }
+    if (p.st_on) {
+      __syncwarp();          // the sweep's (and the ladder tuning's) exchanges are visible; `at` is free again
+      pt_rank_levels(p, c0, n, lane, at);   // the post-sweep levels (the ladder tuning keeps their order)
+      for (int l = lane; l < n; l += 32) p.st_lvl[c0 + at[l]] = l;
+      if (tune_point) pt_tune_steps(p, r, lane);
     }
   }
   if (!DECIDE) return;
@@ -922,6 +989,7 @@ __global__ void pt_drain_kernel(const PtDev p, const PtPeers px) {
     if (yn) p.temps[sp.l1] = temp2;
   }
   if (sp.own2 == px.me && yn) p.temps[sp.l2] = temp1;
+  if (p.st_on) { p.st_pair[0] = sp.i1; p.st_pair[1] = sp.i2; }   // for the next run's first iteration (step tuning)
   if (p.log_flags) {
     const int ls = it - 1 - p.log_base;
     if (ls >= 0 && ls < p.log_cap) { p.log_swaps[3 * ls] = sp.i1; p.log_swaps[3 * ls + 1] = sp.i2; p.log_swaps[3 * ls + 2] = yn; }
@@ -1102,7 +1170,7 @@ void rfinv_handle::free_pt() {
   cudaFree(d.pk); cudaFree(d.pz); cudaFree(d.pdvp); cudaFree(d.pdvs); cudaFree(d.psig); cudaFree(d.pphi); cudaFree(d.log_r);
   cudaFree(d.log_prior12); cudaFree(d.itype); cudaFree(d.pflag); cudaFree(d.active); cudaFree(d.n_active);
   cudaFree(d.nprop); cudaFree(d.naccept); cudaFree(d.n_eval); cudaFree(d.rs_nprop); cudaFree(d.rs_nacc); cudaFree(d.rs_arrived);
-  cudaFree(d.rs_base);
+  cudaFree(d.rs_base); cudaFree(d.st_scale); cudaFree(d.st_nprop); cudaFree(d.st_nacc); cudaFree(d.st_lvl); cudaFree(d.st_pair);
   cudaFree(d.log_flags); cudaFree(d.log_itypes); cudaFree(d.log_swaps);
   cudaFree(d.nk); cudaFree(d.nz); cudaFree(d.nsig); cudaFree(d.namp); cudaFree(d.nvpz); cudaFree(d.nvsz); cudaFree(d.nvpvsz); cudaFree(d.nmod);
   cudaFree(d.vp_mean); cudaFree(d.vs_mean); cudaFree(d.vpvs_mean); cudaFree(d.vp_model); cudaFree(d.vs_model); cudaFree(d.cold_ordinal); cudaFree(d.cold_count); cudaFree(d.ocean_bin);
@@ -1294,6 +1362,93 @@ int32_t rfinv_pt_set_rank_swaps(rfinv_handle* h, int32_t mode) {
   if (mode == 0 && d.rs_tune) {   // the ladder tuning works on the sweep's counters: it goes with it
     s->tune_points_off = pt_tuning_points(s->it_done, d.nburn);
     d.rs_tune = 0;
+  }
+  if (mode == 0 && d.st_on) {     // the step tuning works on the sweep's levels: likewise
+    s->step_points_off = pt_tuning_points(s->it_done, d.nburn);
+    d.st_on = 0;
+  }
+  return RFINV_OK;
+}
+
+int32_t rfinv_pt_set_step_tuning(rfinv_handle* h, int32_t on, double target) {
+  static const char* who = "rfinv_pt_set_step_tuning";
+  int st = pt_require(h, who);
+  if (st != RFINV_OK) return st;
+  PtState* s = h->pt;
+  PtDev& d = s->dev;
+  if (on != 0 && on != 1) { rfinv_set_error("%s: %d (0: off, 1: tune the random-walk widths during the burn-in)", who, on); return RFINV_ERR_ARG; }
+  if (!(target > 0.0 && target < 1.0)) { rfinv_set_error("%s: target %g is outside (0, 1)", who, target); return RFINV_ERR_ARG; }
+  if (s->step_pending) {
+    rfinv_set_error("%s: an iteration is half done (rfinv_pt_local_step without rfinv_pt_apply_swap)", who);
+    return RFINV_ERR_STATE;
+  }
+  if (s->reduced) { rfinv_set_error("%s: rfinv_pt_reduce_outputs has run", who); return RFINV_ERR_STATE; }
+  if (on) {
+    if (s->it_done > 0) {
+      rfinv_set_error("%s: %d iterations have run; the tuning starts with the run (before its first iteration or a restore)", who, s->it_done);
+      return RFINV_ERR_STATE;
+    }
+    if (d.nchains < 2) { rfinv_set_error("%s: nchains = %d: the tuning needs levels, at least two chains per rank", who, d.nchains); return RFINV_ERR_ARG; }
+    if (s->rank_swaps != 1) { rfinv_set_error("%s: the tuning needs the rank swaps on (rfinv_pt_set_rank_swaps(h, 1) first)", who); return RFINV_ERR_STATE; }
+  }
+  RFINV_CUDA_CHECK(cudaSetDevice(h->device));
+  RFINV_CUDA_CHECK(cudaStreamSynchronize(h->stream));
+  if (on) {   // a fresh start: scales 1, counters zero, no pair yet, the levels of the initial temperatures
+    const size_t rows = (size_t)d.G * d.nchains * 4;
+    if (!d.st_scale) {
+      if ((st = dalloc(&d.st_scale, rows)) != RFINV_OK) return st;
+      if ((st = dalloc(&d.st_nprop, rows)) != RFINV_OK) return st;
+      if ((st = dalloc(&d.st_nacc, rows)) != RFINV_OK) return st;
+      if ((st = dalloc(&d.st_lvl, (size_t)d.Cl)) != RFINV_OK) return st;
+      if ((st = dalloc(&d.st_pair, 2)) != RFINV_OK) return st;
+    }
+    const std::vector<double> ones(rows, 1.0);
+    RFINV_CUDA_CHECK(cudaMemcpy(d.st_scale, ones.data(), sizeof(double) * rows, cudaMemcpyHostToDevice));
+    RFINV_CUDA_CHECK(cudaMemset(d.st_nprop, 0, sizeof(unsigned long long) * rows));
+    RFINV_CUDA_CHECK(cudaMemset(d.st_nacc, 0, sizeof(unsigned long long) * rows));
+    const int none[2] = {-1, -1};
+    RFINV_CUDA_CHECK(cudaMemcpy(d.st_pair, none, sizeof(none), cudaMemcpyHostToDevice));
+    std::vector<double> t((size_t)d.Cl);
+    RFINV_CUDA_CHECK(cudaMemcpy(t.data(), d.temps, sizeof(double) * t.size(), cudaMemcpyDeviceToHost));
+    std::vector<int> lvl((size_t)d.Cl);
+    for (int c0 = 0; c0 < d.Cl; c0 += d.nchains)   // (temperature, chain index) order within each rank
+      for (int a = 0; a < d.nchains; ++a) {
+        int l = 0;
+        for (int b = 0; b < d.nchains; ++b) l += t[c0 + b] < t[c0 + a] || (t[c0 + b] == t[c0 + a] && b < a);
+        lvl[c0 + a] = l;
+      }
+    RFINV_CUDA_CHECK(cudaMemcpy(d.st_lvl, lvl.data(), sizeof(int) * lvl.size(), cudaMemcpyHostToDevice));
+  }
+  if (!on && d.st_on) s->step_points_off = pt_tuning_points(s->it_done, d.nburn);
+  pt_drop_graphs(s);   // the captured launches carry the flag and the target
+  d.st_on = on;
+  if (on) d.st_target = target;
+  return RFINV_OK;
+}
+
+int32_t rfinv_pt_get_step_tuning(rfinv_handle* h, int32_t* on, double* target, int32_t* n_points, double* widths,
+                                 int64_t* n_prop, int64_t* n_acc) {
+  int st = pt_require(h, "rfinv_pt_get_step_tuning");
+  if (st != RFINV_OK) return st;
+  const PtState* s = h->pt;
+  const PtDev& d = s->dev;
+  if (on) *on = d.st_on;
+  if (target) *target = d.st_target;
+  if (n_points) *n_points = d.st_on ? pt_tuning_points(s->it_done, d.nburn) : s->step_points_off;
+  const size_t rows = (size_t)d.G * d.nchains * 4;
+  RFINV_CUDA_CHECK(cudaSetDevice(h->device));
+  RFINV_CUDA_CHECK(cudaStreamSynchronize(h->stream));
+  if (widths) {   // off: the params.in widths
+    const double dev[4] = {d.dev_z, d.dev_dvs, d.dev_dvp, d.dev_sig};
+    std::vector<double> sc(rows, 1.0);
+    if (d.st_on) RFINV_CUDA_CHECK(cudaMemcpy(sc.data(), d.st_scale, sizeof(double) * rows, cudaMemcpyDeviceToHost));
+    for (size_t i = 0; i < rows; ++i) widths[i] = dev[i & 3] * sc[i];
+  }
+  for (int k = 0; k < 2; ++k) {
+    int64_t* out = k ? n_acc : n_prop;
+    if (!out) continue;
+    if (d.st_scale) RFINV_CUDA_CHECK(cudaMemcpy(out, k ? d.st_nacc : d.st_nprop, sizeof(int64_t) * rows, cudaMemcpyDeviceToHost));
+    else std::memset(out, 0, sizeof(int64_t) * rows);
   }
   return RFINV_OK;
 }

@@ -50,6 +50,14 @@ struct PtDev {
   // ladder tuning during the burn-in (rfinv_pt_set_ladder_tuning, DESIGN.md 7d); allocated by the first switch on
   unsigned long long* rs_base;    // [G][nchains - 1] rs_nacc at the last tuning point: the acceptances of a round are the difference
   int rs_tune;                    // 1: pt_rank_swap_kernel retunes the ladders at the tuning points
+  // random-walk width tuning during the burn-in (rfinv_pt_set_step_tuning, DESIGN.md 7e); allocated by the first switch on.
+  // Rows [G][nchains][4]: virtual rank, level, type (0 move z, 1 dVs, 2 dVp, 3 sigma)
+  double* st_scale;               // factor on the params.in width, 1 when switched on
+  unsigned long long *st_nprop, *st_nacc;   // proposals / accepted ones since the last tuning point (one writer per row)
+  int* st_lvl;                    // [Cl] each chain's level after the previous iteration's rank sweep
+  int* st_pair;                   // [2] global chains of the previous iteration's global swap (-1: none yet)
+  double st_target;               // acceptance rate the widths are tuned towards
+  int st_on;                      // 1: proposals use the tuned widths, pt_rank_swap_kernel tunes them at the tuning points
 };
 
 struct ncclComm;   // NCCL communicator (comm.cu)
@@ -123,12 +131,13 @@ struct PtState {
   bool reduced = false;        // rfinv_pt_reduce_outputs has run: the bookkeeping may hold job-wide sums
   int rank_swaps = 0;          // rfinv_pt_set_rank_swaps: 0 the reference's global swap only, 1 the rank sweep before it
   int tune_points_off = 0;     // tuning points passed while the ladder tuning was on, frozen when it is switched off
+  int step_points_off = 0;     // likewise for the step tuning
 };
 
 // does an iteration of this state run the rank sweep?  (nothing to pair with fewer than two chains per rank)
 inline bool pt_sweeps(const PtState* s) { return s->rank_swaps == 1 && s->dev.nchains >= 2; }
 
-// the tuning points e = 2^j, j >= 6, e <= nburn among the first it_done iterations (DESIGN.md 7d)
+// the tuning points e = 2^j, j >= 6, e <= nburn among the first it_done iterations (DESIGN.md 7d, 7e)
 inline int pt_tuning_points(int it_done, int nburn) {
   int n = 0;
   for (long long e = 64; e <= it_done && e <= nburn; e *= 2) ++n;

@@ -147,6 +147,26 @@ class ParallelTempering:
         capi.check(self._lib.rfinv_pt_get_ladder_tuning(self.ev.handle, C.byref(on), C.byref(n)))
         return bool(on.value), int(n.value)
 
+    # -- random-walk width tuning during the burn-in (DESIGN.md 7e) ----------------------------------------------------
+    def set_step_tuning(self, on: bool, target: float = 0.44) -> None:
+        """On top of set_rank_swaps(1), before the first iteration (and before restore()): at the iteration counts 64, 128,
+        256, ... up to N_BURN every virtual rank scales the widths of the moves z, dVs, dVp and sigma of each of its levels
+        towards the acceptance rate `target`.  The widths stay fixed after the burn-in.  Off is allowed between runs and
+        returns the widths to the params.in values; set_rank_swaps(0) switches it off too."""
+        capi.check(self._lib.rfinv_pt_set_step_tuning(self.ev.handle, int(on), float(target)))
+
+    def step_tuning(self) -> Dict[str, object]:
+        """{on, target, n_points, widths, n_prop, n_acc}: widths [local ranks][nchains][4] the absolute widths of the levels
+        in the order z, dVs, dVp, sigma; n_prop / n_acc the same shape, the proposals and acceptances since the last tuning
+        point (after the burn-in: those of the final widths)."""
+        shape = (self.rank_count, self.cfg.nchains, 4)
+        on, n, target = C.c_int32(0), C.c_int32(0), C.c_double(0.0)
+        widths = np.zeros(shape); n_prop = np.zeros(shape, np.int64); n_acc = np.zeros(shape, np.int64)
+        capi.check(self._lib.rfinv_pt_get_step_tuning(self.ev.handle, C.byref(on), C.byref(target), C.byref(n),
+                                                      _p(widths, C.POINTER(C.c_double)), _p(n_prop, capi.i64p), _p(n_acc, capi.i64p)))
+        return dict(on=bool(on.value), target=float(target.value), n_points=int(n.value), widths=widths, n_prop=n_prop,
+                    n_acc=n_acc)
+
     # -- results ----------------------------------------------------------------------------------
     def set_logging(self, cap_iters: int) -> None:
         capi.check(self._lib.rfinv_pt_set_logging(self.ev.handle, int(cap_iters)))

@@ -20,7 +20,13 @@ reference's files are written as without it, plus OUT_DIR/rank_swaps with the ac
 
 ``--tune-ladder`` (implies ``--rank-swaps``) also retunes every virtual rank's temperature ladder at the iteration counts 64,
 128, 256, ... up to N_BURN towards equal neighbour-swap rejection rates (DESIGN.md 7d); the ladders are fixed after the
-burn-in.  It adds OUT_DIR/ladder: one line per virtual rank, its temperatures by level (coldest first) at the end of the run."""
+burn-in.  It adds OUT_DIR/ladder: one line per virtual rank, its temperatures by level (coldest first) at the end of the run.
+
+``--tune-steps`` (implies ``--rank-swaps``) also tunes the random-walk widths of the moves z, dVs, dVp and sigma of every
+virtual rank and level at the same iteration counts towards the acceptance rate ``--step-target`` (default 0.44; DESIGN.md
+7e); the widths are fixed after the burn-in.  It adds OUT_DIR/step_widths: one line per virtual rank and level,
+``rank level w_z w_dvs w_dvp w_sig acc_z acc_dvs acc_dvp acc_sig`` -- the final widths and the acceptance they produced since
+the last tuning point (-1 without proposals)."""
 from __future__ import annotations
 
 import argparse
@@ -74,6 +80,24 @@ def write_ladder(out_dir: str, ladders) -> None:
             f.write(" ".join(f"{t:.17g}" for t in row) + "\n")
 
 
+def step_rows(pt) -> np.ndarray:
+    """[local ranks * nchains][10]: global rank, level, the four widths, the four acceptance rates (-1 without proposals)."""
+    st = pt.step_tuning()
+    nr, nc = pt.rank_count, pt.cfg.nchains
+    acc = np.where(st["n_prop"] > 0, st["n_acc"] / np.maximum(st["n_prop"], 1), -1.0)
+    ranks = np.repeat(np.arange(pt.rank_begin, pt.rank_begin + nr), nc)
+    levels = np.tile(np.arange(nc), nr)
+    return np.column_stack([ranks, levels, st["widths"].reshape(-1, 4), acc.reshape(-1, 4)])
+
+
+def write_step_widths(out_dir: str, rows) -> None:
+    """OUT_DIR/step_widths: one line per virtual rank and level."""
+    with open(os.path.join(out_dir, "step_widths"), "w") as f:
+        for row in rows:
+            f.write(f"{int(row[0]):6d} {int(row[1]):5d} " + " ".join(f"{x:.17g}" for x in row[2:6]) + " "
+                    + " ".join(f"{x:.6f}" for x in row[6:]) + "\n")
+
+
 def print_rank_swaps(rs) -> None:
     print(" --- Swaps between neighbouring temperature levels inside the ranks ---")
     for l, (a, n) in enumerate(zip(rs["n_acc"], rs["n_prop"]), start=1):
@@ -81,12 +105,15 @@ def print_rank_swaps(rs) -> None:
 
 
 def run(params_path: str, nproc: int, verbose: bool = True, n_iter: int = None, checkpoint: str = None,
-        checkpoint_every: int = None, resume: bool = False, rank_swaps: bool = False, tune_ladder: bool = False):
+        checkpoint_every: int = None, resume: bool = False, rank_swaps: bool = False, tune_ladder: bool = False,
+        tune_steps: bool = False, step_target: float = 0.44):
     """checkpoint: save the state to this path every `checkpoint_every` iterations (rounded up to the progress steps; default:
     every progress step) and at the end.  resume: restore it first if it exists and continue from its iteration count.
     rank_swaps: the even/odd sweep inside every virtual rank (ParallelTempering.set_rank_swaps(1)); adds OUT_DIR/rank_swaps.
-    tune_ladder: implies rank_swaps, plus the ladder tuning during the burn-in (set_ladder_tuning(1)); adds OUT_DIR/ladder."""
-    rank_swaps = rank_swaps or tune_ladder
+    tune_ladder: implies rank_swaps, plus the ladder tuning during the burn-in (set_ladder_tuning(1)); adds OUT_DIR/ladder.
+    tune_steps: implies rank_swaps, plus the width tuning during the burn-in towards the acceptance rate step_target
+    (set_step_tuning(1, step_target)); adds OUT_DIR/step_widths."""
+    rank_swaps = rank_swaps or tune_ladder or tune_steps
     if resume and not checkpoint:
         raise ValueError("resume needs a checkpoint path")
     if checkpoint_every is not None and checkpoint_every < 1:
@@ -112,6 +139,8 @@ def run(params_path: str, nproc: int, verbose: bool = True, n_iter: int = None, 
         pt.set_rank_swaps(1)
     if tune_ladder:
         pt.set_ladder_tuning(1)
+    if tune_steps:
+        pt.set_step_tuning(1, step_target)
     n_tot = cfg.nburn + cfg.niter if n_iter is None else n_iter
     ck = checkpoint_path(checkpoint, world, rank) if checkpoint else None
     if resume:
@@ -148,6 +177,11 @@ def run(params_path: str, nproc: int, verbose: bool = True, n_iter: int = None, 
         rows = [None] * world
         dist.all_gather_object(rows, ladders)
         ladders = np.concatenate(rows)
+    widths = step_rows(pt) if tune_steps else None
+    if tune_steps and world > 1:
+        rows = [None] * world
+        dist.all_gather_object(rows, widths)
+        widths = np.concatenate(rows)
     if world > 1:                                         # the reference's mpi_reduce / mpi_gather (src/mcmc_out.f90:52-93)
         pt.reduce_outputs()                               # ncclReduce / ncclSend+Recv inside the library: process 0 is job-wide now
     hist, cnt = pt.hist(), pt.counters()
@@ -164,6 +198,8 @@ def run(params_path: str, nproc: int, verbose: bool = True, n_iter: int = None, 
             write_rank_swaps(cfg.out_dir, rs)
         if ladders is not None:
             write_ladder(cfg.out_dir, ladders)
+        if widths is not None:
+            write_step_widths(cfg.out_dir, widths)
     pt.close()
     if world > 1:
         dist.destroy_process_group()
@@ -195,10 +231,11 @@ def load_stations(params_paths):
 
 
 def run_group(params_paths, nproc: int, verbose: bool = True, n_iter: int = None, checkpoint: str = None,
-              checkpoint_every: int = None, resume: bool = False, rank_swaps: bool = False, tune_ladder: bool = False):
+              checkpoint_every: int = None, resume: bool = False, rank_swaps: bool = False, tune_ladder: bool = False,
+              tune_steps: bool = False, step_target: float = 0.44):
     """Several stations (one params file each) as one group on one GPU; arguments as in run().  Under torchrun process r
     takes the stations i with i % world == r.  Returns {station index: (hist, counters)} of this process's stations."""
-    rank_swaps = rank_swaps or tune_ladder
+    rank_swaps = rank_swaps or tune_ladder or tune_steps
     if resume and not checkpoint:
         raise ValueError("resume needs a checkpoint path")
     if checkpoint_every is not None and checkpoint_every < 1:
@@ -229,6 +266,8 @@ def run_group(params_paths, nproc: int, verbose: bool = True, n_iter: int = None
                 pt.set_rank_swaps(1)
                 if tune_ladder:
                     pt.set_ladder_tuning(1)
+                if tune_steps:
+                    pt.set_step_tuning(1, step_target)
         if restore:
             for i, pt in zip(mine, pts):
                 pt.restore(cks[i])
@@ -268,6 +307,8 @@ def run_group(params_paths, nproc: int, verbose: bool = True, n_iter: int = None
                 write_rank_swaps(cfg.out_dir, pt.rank_swaps())
             if tune_ladder:
                 write_ladder(cfg.out_dir, rank_ladders(pt))
+            if tune_steps:
+                write_step_widths(cfg.out_dir, step_rows(pt))
             out[i] = (hist, cnt)
         return out
     finally:
@@ -294,15 +335,23 @@ def main(argv=None):
     ap.add_argument("--tune-ladder", action="store_true",
                     help="with --rank-swaps (implied): retune every rank's temperature ladder during the burn-in towards equal "
                          "swap rejection rates between neighbouring levels (writes OUT_DIR/ladder)")
+    ap.add_argument("--tune-steps", action="store_true",
+                    help="with --rank-swaps (implied): tune the random-walk widths of every rank's levels during the burn-in "
+                         "towards the acceptance rate --step-target (writes OUT_DIR/step_widths)")
+    ap.add_argument("--step-target", type=float, default=0.44,
+                    help="acceptance rate --tune-steps aims at, in (0, 1) (default 0.44)")
     a = ap.parse_args(argv)
     if a.resume and not a.checkpoint:
         ap.error("--resume needs --checkpoint")
+    if not 0.0 < a.step_target < 1.0:
+        ap.error("--step-target must lie in (0, 1)")
     if len(a.params) == 1:
         run(a.params[0], a.nproc, n_iter=a.iters, checkpoint=a.checkpoint, checkpoint_every=a.checkpoint_every, resume=a.resume,
-            rank_swaps=a.rank_swaps, tune_ladder=a.tune_ladder)
+            rank_swaps=a.rank_swaps, tune_ladder=a.tune_ladder, tune_steps=a.tune_steps, step_target=a.step_target)
     else:
         run_group(a.params, a.nproc, n_iter=a.iters, checkpoint=a.checkpoint, checkpoint_every=a.checkpoint_every,
-                  resume=a.resume, rank_swaps=a.rank_swaps, tune_ladder=a.tune_ladder)
+                  resume=a.resume, rank_swaps=a.rank_swaps, tune_ladder=a.tune_ladder, tune_steps=a.tune_steps,
+                  step_target=a.step_target)
 
 
 if __name__ == "__main__":

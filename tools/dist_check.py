@@ -7,6 +7,8 @@ rfinv_pt_run_distributed (in-library ncclAllGather, CUDA graph) equal those of O
 --rank-swaps runs both sides with the even/odd sweep inside every virtual rank (set_rank_swaps(1)) and also compares its
 job-wide counters.  --tune-ladder adds the ladder tuning during the burn-in (set_ladder_tuning(1), implies --rank-swaps), with
 burn-ins and run lengths that pass two or three tuning points, and also compares the number of tuning points passed.
+--tune-steps adds the width tuning during the burn-in (set_step_tuning(1), implies --rank-swaps) with the same run lengths, and
+also compares each process's widths and width counters with its rows of the single-process run.
 """
 import faulthandler, hashlib, json, os, signal, sys
 faulthandler.register(signal.SIGTERM, all_threads=True, chain=False)
@@ -20,7 +22,8 @@ from rf_inv_b200.evaluator import Evaluator
 from rf_inv_b200.pt import ParallelTempering
 
 
-def identity_check(cfg, nproc_total, n_iter, world, rank, local_rank, dist, torch, rank_swaps=0, tune_ladder=False):
+def identity_check(cfg, nproc_total, n_iter, world, rank, local_rank, dist, torch, rank_swaps=0, tune_ladder=False,
+                   tune_steps=False):
     """Returns (ok, detail) on every process."""
     dev = torch.device("cuda", local_rank)
     # distributed run
@@ -32,6 +35,8 @@ def identity_check(cfg, nproc_total, n_iter, world, rank, local_rank, dist, torc
         pt.set_rank_swaps(rank_swaps)
     if tune_ladder:
         pt.set_ladder_tuning(1)
+    if tune_steps:
+        pt.set_step_tuning(1)
     pt.init_comm(dist, torch)
     say("communicator up")
     pt.run_distributed(n_iter, dist, torch)
@@ -40,6 +45,7 @@ def identity_check(cfg, nproc_total, n_iter, world, rank, local_rank, dist, torc
     flags, itypes, swaps = pt.log(n_iter)
     st = pt.state()
     tuning = pt.ladder_tuning()
+    steps = pt.step_tuning() if tune_steps else None
     pt.reduce_outputs()
     say("outputs reduced")
     cnt = pt.counters()
@@ -56,7 +62,10 @@ def identity_check(cfg, nproc_total, n_iter, world, rank, local_rank, dist, torc
             ref.set_rank_swaps(rank_swaps)
         if tune_ladder:
             ref.set_ladder_tuning(1)
+        if tune_steps:
+            ref.set_step_tuning(1)
         ref.run(n_iter)
+        rsteps = ref.step_tuning() if tune_steps else None
         rtuning = ref.ladder_tuning()
         rf, ri, rs = ref.log(n_iter)
         rst = ref.state()
@@ -65,7 +74,7 @@ def identity_check(cfg, nproc_total, n_iter, world, rank, local_rank, dist, torc
         rrsw = ref.rank_swaps() if rank_swaps else None
         ref.close()
         say("reference run done")
-        box = [dict(flags=rf, itypes=ri, swaps=rs, state=rst, tuning=rtuning)]
+        box = [dict(flags=rf, itypes=ri, swaps=rs, state=rst, tuning=rtuning, steps=rsteps)]
     else:
         box = [None]
     dist.broadcast_object_list(box, src=0)
@@ -79,6 +88,11 @@ def identity_check(cfg, nproc_total, n_iter, world, rank, local_rank, dist, torc
         parts["state_" + k] = np.array_equal(st[k], r["state"][k][sl])
     if tune_ladder:
         parts["ladder_tuning"] = tuning == r["tuning"] and tuning[0] and tuning[1] >= 2
+    if tune_steps:
+        rsl = slice(pt.rank_begin, pt.rank_begin + pt.rank_count)
+        parts["step_tuning"] = (steps["on"] and steps["n_points"] == r["steps"]["n_points"] >= 2
+                                and not np.all(r["steps"]["widths"] == r["steps"]["widths"][0, 0])
+                                and all(np.array_equal(steps[k], r["steps"][k][rsl]) for k in ("widths", "n_prop", "n_acc")))
     detail = {}
     if rank == 0:
         parts["nprop"] = np.array_equal(cnt["nprop"], rcnt["nprop"]); parts["naccept"] = np.array_equal(cnt["naccept"], rcnt["naccept"])
@@ -110,10 +124,11 @@ if __name__ == "__main__":
     os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
     dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
     tune_ladder = "--tune-ladder" in sys.argv[1:]
-    rank_swaps = 1 if "--rank-swaps" in sys.argv[1:] or tune_ladder else 0
+    tune_steps = "--tune-steps" in sys.argv[1:]
+    rank_swaps = 1 if "--rank-swaps" in sys.argv[1:] or tune_ladder or tune_steps else 0
     out = {}
     runs = (("sample", 4 * world, 300, dict(nburn=100, niter=200)), ("c4", 8 * world, 120, dict()), ("target", 16 * world, 60, dict()))
-    if tune_ladder:   # tuning points 64, 128, 256 / 64, 128, inside and at the end of the burn-in
+    if tune_ladder or tune_steps:   # tuning points 64, 128, 256 / 64, 128, inside and at the end of the burn-in
         runs = (("sample", 4 * world, 300, dict(nburn=280, niter=20)), ("c4", 8 * world, 140, dict(nburn=128)),
                 ("target", 16 * world, 130, dict(nburn=200)))
     for name, nproc, iters, kw in runs:
@@ -128,7 +143,8 @@ if __name__ == "__main__":
         with Evaluator(cfg, device=local_rank) as ev:
             _, rft, _ = ev.calc_likelihood(tm["k"], tm["z"], tm["dvp"], tm["dvs"], tm["sig"], want_rft=True)
         cfg.obs = (rft[0, :, :cfg.nsmp] + np.random.default_rng(7).normal(0.0, 0.01, (cfg.ntrc, cfg.nsmp))).astype(np.float32).astype(np.float64)
-        ok, detail = identity_check(cfg, nproc, iters, world, rank, local_rank, dist, torch, rank_swaps, tune_ladder)
+        ok, detail = identity_check(cfg, nproc, iters, world, rank, local_rank, dist, torch, rank_swaps, tune_ladder,
+                                    tune_steps)
         out[name] = dict(identical=ok, world=world, virtual_ranks=nproc, iterations=iters, **detail)
     if rank == 0:
         print(json.dumps(out), flush=True)
