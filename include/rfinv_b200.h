@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define RFINV_ABI_VERSION 8
+#define RFINV_ABI_VERSION 9
 
 /* status codes */
 #define RFINV_OK 0
@@ -337,6 +337,41 @@ int32_t rfinv_pt_set_step_tuning(rfinv_handle* h, int32_t on, double target);
  * propose); n_prop / n_acc [G][nchains][4] since the last tuning point; any pointer may be NULL */
 int32_t rfinv_pt_get_step_tuning(rfinv_handle* h, int32_t* on, double* target, int32_t* n_points, double* widths,
                                  int64_t* n_prop, int64_t* n_acc);
+
+/* ---- convergence diagnostics (ABI version 9, DESIGN.md 7f) ---------------------------------------------------------------
+ * Level 0 of virtual rank r is its chain of lowest (temperature, local chain index), the order of the rank sweep.  With the
+ * diagnostics on, every iteration that records the posterior bookkeeping (it > nburn, it % ncorr == 0) also records, right
+ * after the bookkeeping (the temperatures at acceptance, before the sweep and the global swap), one row per local rank from
+ * its level-0 chain: k, logL, sig[t] of every trace t with sig_mode[t] on (trace order), and the Vs the bookkeeping assigns
+ * to each chosen depth bin b (1-based; vs_min inside the sea layer); and beside it the temperature T0 of that chain.  Layout
+ * trace[sample][local rank][quantity] (fp64), t0[sample][local rank]; the capacity is the number of recording iterations in
+ * [1, nburn + niter]; later samples are not recorded.  In iterations that run the rank sweep (mode 1), each chain also keeps a
+ * round-trip state on the levels the sweep finds before deciding any pair: reaching level 0 sets "came from level 0";
+ * reaching level nchains - 1 from it moves on to "reached the top"; reaching level 0 from there completes one round trip of
+ * the chain's rank, counted during the burn-in (it <= nburn) or after it.  The diagnostics only read: state, counters, logs,
+ * histograms and recorded models stay bit for bit those of the same run without them.
+ * on: 0/1; vs_bins[n_bins], 0 <= n_bins <= 16, each in [1, nbin_z].  Only after rfinv_pt_init and before the first
+ * iteration, or before rfinv_pt_restore (a checkpoint restores only into a handle with the same setting and bins).
+ * RFINV_ERR_ARG: on other than 0 or 1, bad bins or more than 16.  RFINV_ERR_STATE: after an iteration has run, between
+ * rfinv_pt_local_step and rfinv_pt_apply_swap, after rfinv_pt_reduce_outputs, or switching on without the bookkeeping
+ * (niter > 0 and all nbin_* > 0). */
+int32_t rfinv_pt_set_diagnostics(rfinv_handle* h, int32_t on, int32_t n_bins, const int32_t* vs_bins);
+/* The setting, quantities per row (2 + solved sigmas + n_bins), the bins, and the first min(recorded, max_samples) samples of
+ * this process's trace: trace[n][G][n_quantities], t0[n][G]; vs_bins has up to 16 entries.  Any pointer may be NULL. */
+int32_t rfinv_pt_get_cold_trace(rfinv_handle* h, int32_t* on, int32_t* n_quantities, int32_t* n_bins, int32_t* vs_bins,
+                                int64_t max_samples, int64_t* n_samples, double* trace, double* t0);
+/* Statistics of the n recorded samples, computed on the device.  rows[n_ranks][n_quantities][9], one per rank and quantity
+ * from its series alone: mean, variance (n - 1), tau (integrated autocorrelation time: autocovariance with divisor n over
+ * lag 0, tau = 1 + 2 sum rho(t) up to the first m >= 5 tau; NaN for n < 4 or a constant series), ESS = n / tau, the mean and
+ * variance (h - 1) of the halves [0, h) and [n - h, n) with h = n / 2, and the rank's samples with T0 > 1 + 1e-6f.
+ * summary[n_quantities][4] over the ranks in global rank order: split-R-hat (BDA3) over the 2 n_ranks half-chains (NaN for
+ * h < 2 or a zero within-variance), the sum of the ESS and the median tau over the ranks with finite tau, and the share of
+ * (rank, sample) entries whose T0 is tempered.  trips[n_ranks][2]: round trips during the burn-in and after it (zero in
+ * mode 0 and with one chain per rank).  n_ranks is this process's G -- after rfinv_pt_reduce_outputs, on process 0, every
+ * virtual rank of the job, with the same result as one process holding them all.  Any pointer may be NULL.
+ * RFINV_ERR_STATE: the diagnostics are off. */
+int32_t rfinv_pt_get_diagnostics(rfinv_handle* h, int64_t* n_samples, int32_t* n_ranks, int32_t* n_quantities, double* rows,
+                                 double* summary, int64_t* trips);
 
 /* ---- file formats either side of the path (host only, no CUDA) ---------------------------------------
  * params.in (positional, '#' comment lines; src/params.f90:101-405), SAC traces cut to [T_START, T_END]

@@ -250,6 +250,36 @@ module rfinv_b200_capi
        integer(c_int64_t), intent(out) :: n_prop(*), n_acc(*)
      end function rfinv_pt_get_step_tuning
 
+     ! convergence diagnostics (ABI version 9): on 0 or 1, vs_bins(n_bins) 1-based depth bins, before the first iteration
+     integer(c_int32_t) function rfinv_pt_set_diagnostics(handle, on, n_bins, vs_bins) bind(C, name="rfinv_pt_set_diagnostics")
+       import :: c_int32_t, c_ptr
+       type(c_ptr), value :: handle
+       integer(c_int32_t), value :: on, n_bins
+       integer(c_int32_t), intent(in) :: vs_bins(*)
+     end function rfinv_pt_set_diagnostics
+
+     ! the setting, quantities per row, bins (up to 16); trace (n_quantities, rank_count, n_samples), t0 (rank_count, n_samples)
+     integer(c_int32_t) function rfinv_pt_get_cold_trace(handle, on, n_quantities, n_bins, vs_bins, max_samples, n_samples, &
+         trace, t0) bind(C, name="rfinv_pt_get_cold_trace")
+       import :: c_int32_t, c_int64_t, c_double, c_ptr
+       type(c_ptr), value :: handle
+       integer(c_int32_t), intent(out) :: on, n_quantities, n_bins, vs_bins(*)
+       integer(c_int64_t), value :: max_samples
+       integer(c_int64_t), intent(out) :: n_samples
+       real(c_double), intent(out) :: trace(*), t0(*)
+     end function rfinv_pt_get_cold_trace
+
+     ! rows (9, n_quantities, n_ranks), summary (4, n_quantities): R-hat, ESS, median tau, tempered share; trips (2, n_ranks)
+     integer(c_int32_t) function rfinv_pt_get_diagnostics(handle, n_samples, n_ranks, n_quantities, rows, summary, trips) &
+         bind(C, name="rfinv_pt_get_diagnostics")
+       import :: c_int32_t, c_int64_t, c_double, c_ptr
+       type(c_ptr), value :: handle
+       integer(c_int64_t), intent(out) :: n_samples
+       integer(c_int32_t), intent(out) :: n_ranks, n_quantities
+       real(c_double), intent(out) :: rows(*), summary(*)
+       integer(c_int64_t), intent(out) :: trips(*)
+     end function rfinv_pt_get_diagnostics
+
      ! several stations advanced together (ABI version 5): handles(n) are the c_ptr of n handles after rfinv_pt_init
      integer(c_int32_t) function rfinv_pt_group_create(handles, n, group) bind(C, name="rfinv_pt_group_create")
        import :: c_int32_t, c_ptr

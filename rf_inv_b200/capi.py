@@ -78,6 +78,9 @@ SIGNATURES = {
     "rfinv_pt_get_ladder_tuning": (C.c_int32, [C.c_void_p, i32p, i32p]),
     "rfinv_pt_set_step_tuning": (C.c_int32, [C.c_void_p, C.c_int32, C.c_double]),
     "rfinv_pt_get_step_tuning": (C.c_int32, [C.c_void_p, i32p, C.POINTER(C.c_double), i32p, C.POINTER(C.c_double), i64p, i64p]),
+    "rfinv_pt_set_diagnostics": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int32, i32p]),
+    "rfinv_pt_get_cold_trace": (C.c_int32, [C.c_void_p, i32p, i32p, i32p, i32p, C.c_int64, i64p, dp, dp]),
+    "rfinv_pt_get_diagnostics": (C.c_int32, [C.c_void_p, i64p, i32p, i32p, dp, dp, i64p]),
     "rfinv_problem_load": (C.c_int32, [C.c_char_p, C.c_char_p, C.POINTER(C.c_void_p)]),
     "rfinv_problem_free": (None, [C.c_void_p]),
     "rfinv_problem_config": (C.POINTER(RfinvConfigC), [C.c_void_p]),

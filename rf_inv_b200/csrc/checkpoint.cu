@@ -152,6 +152,12 @@ std::vector<Part> parts(rfinv_handle* h, int it_done, long long n_models) {
     v.insert(v.end(), {{"step_scale", d.st_scale, 8, rows}, {"step_nprop", d.st_nprop, 8, rows}, {"step_nacc", d.st_nacc, 8, rows},
                        {"step_lvl", d.st_lvl, 4, Cl}, {"step_pair", d.st_pair, 4, 2}});
   }
+  if (d.dg_on) {   // the diagnostics (rfinv_pt_set_diagnostics), only with them on: the samples recorded so far
+    long long ns = pt_diag_samples(it_done, d.nburn, d.ncorr);
+    if (ns > d.dg_cap) ns = d.dg_cap;
+    v.insert(v.end(), {{"diag_trace", d.dg_trace, 8, (uint64_t)ns * G * d.dg_nq}, {"diag_t0", d.dg_t0, 8, (uint64_t)ns * G},
+                       {"diag_trip_st", d.dg_trip_st, 1, Cl}, {"diag_trips", d.dg_trips, 8, 2 * G}});
+  }
   return v;
 }
 
@@ -165,6 +171,10 @@ constexpr const char* RS_SECTION = "rank_swaps";
 constexpr const char* LT_SECTION = "ladder_tuning";
 // The step tuning's setting, written only with it on: double [target].  Its device arrays are sections of parts().
 constexpr const char* ST_SECTION = "step_tuning";
+// The diagnostics' setting, written only with them on: int64 [number of depth bins | the bins, padded to 16 | trace capacity
+// of the saving handle].  Their device arrays are sections of parts().
+constexpr const char* DG_SECTION = "diagnostics";
+constexpr int DG_WORDS = 1 + 16 + 1;
 
 int io_error(const char* who, const std::string& path, const char* what) {
   rfinv_set_error("%s: %s: %s", who, path.c_str(), what);
@@ -227,12 +237,22 @@ int32_t rfinv_pt_save(rfinv_handle* h, const char* path) {
       for (size_t i = 0; i < nr; ++i) lt[1 + i] = (int64_t)(acc[i] - base[i]);
     }
   }
-  hd.n_sections = (uint32_t)(ps.size() + (rs.empty() ? 0 : 1) + (lt.empty() ? 0 : 1) + (d.st_on ? 1 : 0));
+  std::vector<int64_t> dg;
+  if (d.dg_on) {
+    dg.assign(DG_WORDS, 0);
+    dg[0] = d.dg_nbins;
+    std::vector<int32_t> bins(16, 0);
+    if (d.dg_nbins) RFINV_CUDA_CHECK(cudaMemcpy(bins.data(), d.dg_bins, sizeof(int32_t) * d.dg_nbins, cudaMemcpyDeviceToHost));
+    for (int j = 0; j < 16; ++j) dg[1 + j] = bins[j];
+    dg[17] = d.dg_cap;
+  }
+  hd.n_sections = (uint32_t)(ps.size() + (rs.empty() ? 0 : 1) + (lt.empty() ? 0 : 1) + (d.st_on ? 1 : 0) + (dg.empty() ? 0 : 1));
   size_t total = sizeof(CkHeader) + sizeof(uint64_t);
   for (const Part& p : ps) total += sizeof(CkSection) + (size_t)p.elem * p.count;
   if (!rs.empty()) total += sizeof(CkSection) + sizeof(int64_t) * rs.size();
   if (!lt.empty()) total += sizeof(CkSection) + sizeof(int64_t) * lt.size();
   if (d.st_on) total += sizeof(CkSection) + sizeof(double);
+  if (!dg.empty()) total += sizeof(CkSection) + sizeof(int64_t) * dg.size();
   std::unique_ptr<uint8_t[]> buf(new (std::nothrow) uint8_t[total]);
   if (!buf) { rfinv_set_error("%s: cannot allocate %zu bytes of host memory", who, total); return RFINV_ERR_IO; }
   size_t off = 0;
@@ -270,6 +290,14 @@ int32_t rfinv_pt_save(rfinv_handle* h, const char* path) {
     sc.elem_size = sizeof(double); sc.count = 1;
     std::memcpy(buf.get() + off, &sc, sizeof(sc)); off += sizeof(sc);
     std::memcpy(buf.get() + off, &d.st_target, sizeof(double)); off += sizeof(double);
+  }
+  if (!dg.empty()) {
+    CkSection sc;
+    std::memset(&sc, 0, sizeof(sc));
+    std::snprintf(sc.name, sizeof(sc.name), "%s", DG_SECTION);
+    sc.elem_size = sizeof(int64_t); sc.count = dg.size();
+    std::memcpy(buf.get() + off, &sc, sizeof(sc)); off += sizeof(sc);
+    std::memcpy(buf.get() + off, dg.data(), sizeof(int64_t) * dg.size()); off += sizeof(int64_t) * dg.size();
   }
   const uint64_t sum = xxh64(buf.get(), off);
   std::memcpy(buf.get() + off, &sum, sizeof(sum));
@@ -433,6 +461,34 @@ int32_t rfinv_pt_restore(rfinv_handle* h, const char* path) {
     std::memcpy(&target, buf.data() + st_it->second.first, sizeof(double));
     if (target != d.st_target) {
       rfinv_set_error("%s: %s was written with the step tuning's target %.17g, this handle has %.17g", who, path, target, d.st_target);
+      return RFINV_ERR_ARG;
+    }
+  }
+  // the diagnostics likewise, with the same depth bins (rfinv_pt_set_diagnostics before restoring)
+  const auto dg_it = found.find(DG_SECTION);
+  if ((dg_it != found.end()) != (d.dg_on != 0)) {
+    rfinv_set_error("%s: %s was written with the diagnostics %s, this handle has them %s (rfinv_pt_set_diagnostics before restore)",
+                    who, path, dg_it != found.end() ? "on" : "off", d.dg_on ? "on" : "off");
+    return RFINV_ERR_ARG;
+  }
+  if (dg_it != found.end()) {
+    if (dg_it->second.second.elem_size != sizeof(int64_t) || dg_it->second.second.count != DG_WORDS)
+      return io_error(who, file, "section 'diagnostics' is malformed");
+    int64_t dg[DG_WORDS];
+    std::memcpy(dg, buf.data() + dg_it->second.first, sizeof(dg));
+    std::vector<int32_t> bins(16, 0);
+    if (d.dg_nbins) RFINV_CUDA_CHECK(cudaMemcpy(bins.data(), d.dg_bins, sizeof(int32_t) * d.dg_nbins, cudaMemcpyDeviceToHost));
+    bool same = dg[0] == d.dg_nbins;
+    for (int j = 0; j < 16; ++j) same = same && dg[1 + j] == bins[j];
+    if (!same) {
+      rfinv_set_error("%s: %s was written with %lld diagnostic depth bins that differ from this handle's %d", who, path,
+                      (long long)dg[0], d.dg_nbins);
+      return RFINV_ERR_ARG;
+    }
+    // as for the recorded models: a larger capacity must not open samples the saving handle had no room for
+    if (hd.it_done >= 0 && pt_diag_samples(hd.it_done, d.nburn, d.ncorr) > dg[17] && d.dg_cap > dg[17]) {
+      rfinv_set_error("%s: %s: its trace was full at %lld samples and this configuration has room for %lld: the trace would "
+                      "differ from an uninterrupted run", who, path, (long long)dg[17], d.dg_cap);
       return RFINV_ERR_ARG;
     }
   }

@@ -296,6 +296,43 @@ int32_t rfinv_pt_reduce_outputs(rfinv_handle* h) {
     const int st = rfinv_pt_fix_assigned_bins(h);
     if (st != RFINV_OK) return st;
   }
+  if (d.dg_on) {
+    // convergence diagnostics: every process's per-rank rows (computed from its own trace) and round-trip counters go to
+    // process 0 in process order, i.e. global rank order; the trace itself stays where it is
+    const size_t row = (size_t)d.dg_nq * PT_DG_ROW, G = d.G;
+    double* rows = nullptr;
+    unsigned long long* trips = d.dg_trips;
+    if (h->comm_rank == 0) {
+      cudaFree(s->dg_job_rows); cudaFree(s->dg_job_trips);
+      RFINV_CUDA_CHECK(cudaMalloc((void**)&s->dg_job_rows, sizeof(double) * row * d.nproc_total));
+      RFINV_CUDA_CHECK(cudaMalloc((void**)&s->dg_job_trips, sizeof(unsigned long long) * 2 * d.nproc_total));
+      rows = s->dg_job_rows;
+      trips = s->dg_job_trips;
+      RFINV_CUDA_CHECK(cudaMemcpyAsync(trips, d.dg_trips, sizeof(unsigned long long) * 2 * G, cudaMemcpyDeviceToDevice, q));
+    } else {
+      RFINV_CUDA_CHECK(cudaMalloc((void**)&rows, sizeof(double) * row * G));
+    }
+    int st = rfinv_pt_diag_rows(h, rows);
+    if (st == RFINV_OK) {
+      RFINV_NCCL_CHECK(api, api->GroupStart());
+      if (h->comm_rank == 0) {
+        for (int r = 1; r < h->comm_world; ++r) {
+          RFINV_NCCL_CHECK(api, api->Recv(rows + (size_t)r * G * row, G * row, ncclFloat64, r, comm, q));
+          RFINV_NCCL_CHECK(api, api->Recv(trips + (size_t)r * G * 2, G * 2, ncclUint64, r, comm, q));
+        }
+      } else {
+        RFINV_NCCL_CHECK(api, api->Send(rows, G * row, ncclFloat64, 0, comm, q));
+        RFINV_NCCL_CHECK(api, api->Send(d.dg_trips, G * 2, ncclUint64, 0, comm, q));
+      }
+      RFINV_NCCL_CHECK(api, api->GroupEnd());
+    }
+    if (h->comm_rank != 0) {
+      const cudaError_t e = cudaStreamSynchronize(q);
+      cudaFree(rows);
+      if (st == RFINV_OK && e != cudaSuccess) { rfinv_set_error("rfinv_pt_reduce_outputs: %s", cudaGetErrorString(e)); st = RFINV_ERR_CUDA; }
+    }
+    if (st != RFINV_OK) return st;
+  }
   RFINV_CUDA_CHECK(cudaStreamSynchronize(q));
   return RFINV_OK;
 }

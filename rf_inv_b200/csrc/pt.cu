@@ -13,6 +13,7 @@
 // iseed + r*r*10000 + 23*r.  The number of draws a chain step consumes never depends on the forward result, so
 // per iteration one thread per virtual rank runs the serial proposal pass (draws, proposal, validity, the
 // acceptance uniform), then ALL forward+likelihood evaluations run batched, then acceptance is parallel.
+#include <algorithm>
 #include <vector>
 #include <cstring>
 #include "rfinv_handle.h"
@@ -782,10 +783,18 @@ __device__ __forceinline__ uint64_t philox4x64_w0(uint64_t c0, uint64_t c1, uint
 // exchange their temperatures in temps and in the swap table.  peer: the peer-memory exchange, where pt_finish_kernel has
 // already advanced *it_dev and the table alternates.  DECIDE (single process): the last CTA then takes the global swap
 // decision that pt_finish_kernel<false, true> takes without the sweep.
+// With the diagnostics on (p.dg_on), the levels found before any pair is decided also advance the round-trip states.
 // With the ladder tuning on (p.rs_tune), the iterations e - 1 of the tuning points e then retune every rank's ladder
 // (pt_tune_ladder) before the global swap reads the table.  With the step tuning on (p.st_on), every iteration records the
 // post-sweep levels (st_lvl) for the next iteration's proposals, and the tuning points' iterations tune the widths (pt_tune_steps).
 constexpr int PT_RS_WARPS = 4;
+// Index checks of the diagnostics kernels, compiled in with -DRFINV_KERNEL_ASSERTS (a build for checking, not for speed).
+#ifdef RFINV_KERNEL_ASSERTS
+#include <cassert>
+#define PT_DG_ASSERT(x) assert(x)
+#else
+#define PT_DG_ASSERT(x) ((void)0)
+#endif
 
 // chain of the rank at each level: its place among the chains c0 .. c0 + n - 1 sorted by (temperature, chain index)
 __device__ __forceinline__ void pt_rank_levels(const PtDev& p, int c0, int n, int lane, int* at) {
@@ -882,6 +891,19 @@ __global__ void __launch_bounds__(32 * PT_RS_WARPS) pt_rank_swap_kernel(const Pt
     int* at = (int*)(rs_smem + (p.rs_tune ? (size_t)(blockDim.x >> 5) * n : 0)) + (size_t)warp * n;
     const int c0 = r * n;
     pt_rank_levels(p, c0, n, lane, at);
+    if (p.dg_on) {   // round trips (DESIGN.md 7f) on the levels at acceptance; one lane writes the rank's counters
+      const int phase = it + 1 <= p.nburn ? 0 : 1;
+      if (lane == 0) {
+        PT_DG_ASSERT(at[0] >= 0 && at[0] < n && at[n - 1] >= 0 && at[n - 1] < n && at[0] != at[n - 1]);
+        int8_t* st = p.dg_trip_st + c0 + at[0];
+        if (*st == 2) p.dg_trips[2 * (size_t)r + phase] += 1ULL;
+        *st = 1;
+      }
+      if (lane == (n - 1) % 32) {
+        int8_t* st = p.dg_trip_st + c0 + at[n - 1];
+        if (*st == 1) *st = 2;
+      }
+    }
     const uint64_t grank = (uint64_t)(p.rank_begin + r), key = (uint64_t)(uint32_t)p.iseed;
     for (int l = (it & 1) + 2 * lane; l + 1 < n; l += 64) {
       const int a = c0 + at[l], b = c0 + at[l + 1];
@@ -1023,13 +1045,59 @@ __global__ void pt_coldscan_kernel(const PtDev p) {
   if (tid == 0) *p.cold_count = s_base;
 }
 
+// format_model (src/model.f90:175-290) of chain c's current state as the posterior bookkeeping sees it: layer l has the
+// velocities (alpha[l], beta[l]) and covers the depth bins iz1[l] <= iz < iz1[l + 1] (iz1 has nlay + 1 entries).  Returns nlay.
+// One thread.
+__device__ int pt_format_layers(const DevConfig& cfg, const PtDev& p, int c, double dbin_z, double* alpha, double* beta, int* iz1) {
+  const int km = cfg.k_max, Cl = p.Cl, k = p.k[c];
+  double z[RFINV_MAX_K], dp[RFINV_MAX_K], ds[RFINV_MAX_K];
+  for (int i = 0; i < k; ++i) { z[i] = p.z[(size_t)i * Cl + c]; dp[i] = p.dvp[(size_t)i * Cl + c]; ds[i] = p.dvs[(size_t)i * Cl + c]; }
+  for (int i = 1; i < k; ++i) {
+    const double a = z[i], b = dp[i], d = ds[i];
+    int m = i - 1;
+    while (m >= 0 && z[m] > a) { z[m + 1] = z[m]; dp[m + 1] = dp[m]; ds[m + 1] = ds[m]; --m; }
+    z[m + 1] = a; dp[m + 1] = b; ds[m + 1] = d;
+  }
+  int n = 0;
+  double tmpz = 0.0;
+  if (cfg.sdep > 0.0) {
+    alpha[n] = 1.5; beta[n] = -999.0; iz1[n] = (int)(tmpz / dbin_z) + 1;
+    tmpz = __dadd_rn(tmpz, cfg.sdep); ++n;
+  }
+  for (int l = 0; l <= k; ++l) {
+    double zc, h, dvs_l, dvp_l;
+    if (l == 0) { zc = __dmul_rn(0.5, __dadd_rn(cfg.sdep, z[0])); h = __dsub_rn(z[0], cfg.sdep); dvs_l = ds[0]; dvp_l = dp[0]; }
+    else if (l < k) { zc = __dmul_rn(0.5, __dadd_rn(z[l], z[l - 1])); h = __dsub_rn(z[l], z[l - 1]); dvs_l = ds[l]; dvp_l = dp[l]; }
+    else { zc = __dmul_rn(0.5, __dadd_rn(cfg.z_max, z[k - 1])); h = 999.0;
+           dvs_l = p.dvs[(size_t)(km - 1) * Cl + c]; dvp_l = p.dvp[(size_t)(km - 1) * Cl + c]; }
+    double a, b;
+    layer_velocity(cfg, zc, dvs_l, dvp_l, a, b);
+    alpha[n] = a; beta[n] = b;
+    iz1[n] = (int)(__ddiv_rn(tmpz, dbin_z)) + 1;
+    tmpz = __dadd_rn(tmpz, h);
+    ++n;
+  }
+  iz1[n] = p.nbin_z + 1;   // iz2 of the half space (src/pt_mcmc.f90:243)
+  return n;
+}
+
+// the layer of pt_format_layers that covers depth bin iz (1-based), or -1
+__device__ __forceinline__ int pt_bin_layer(const int* iz1, int nlay, int iz) {
+  int l = 0;
+  while (l + 1 < nlay && iz >= iz1[l + 1]) ++l;
+  return iz < iz1[l] ? -1 : l;
+}
+
+// the Vs the bookkeeping records for a layer of velocity beta: the sea layer (beta <= 0) records vs_min (src/pt_mcmc.f90:260-263)
+__device__ __forceinline__ double pt_recorded_vs(const DevConfig& cfg, double beta) { return beta > 0.0 ? beta : cfg.vs_min; }
+
 // Posterior bookkeeping of one non-tempered chain per CTA (src/pt_mcmc.f90:204-286).
 __global__ void pt_record_kernel(const DevConfig cfg, const PtDev p) {
   const int c = blockIdx.x;
   const int ord = p.cold_ordinal[c];
   if (ord < 0) return;
   const int tid = threadIdx.x, nthr = blockDim.x;
-  const int km = cfg.k_max, Cl = p.Cl, T = cfg.ntrc, S = cfg.nsmp;
+  const int Cl = p.Cl, T = cfg.ntrc, S = cfg.nsmp;
   __shared__ double s_alpha[RFINV_MAX_LAY], s_beta[RFINV_MAX_LAY];
   __shared__ int s_iz1[RFINV_MAX_LAY + 1], s_nlay;
   const double dbin_amp = (p.amp_max - p.amp_min) / p.nbin_amp, dbin_vp = (cfg.vp_max - cfg.vp_min) / p.nbin_vp;
@@ -1049,44 +1117,14 @@ __global__ void pt_record_kernel(const DevConfig cfg, const PtDev p) {
       const int ibin = (int)((p.z[(size_t)(il - 1) * Cl + c] - cfg.z_min) / dbin_z) + 1;
       if (ibin >= 1 && ibin <= p.nbin_z) atomicAdd(&p.nz[ibin - 1], 1ULL);
     }
-    // format_model (src/model.f90:175-290) of the current state
-    double z[RFINV_MAX_K], dp[RFINV_MAX_K], ds[RFINV_MAX_K];
-    for (int i = 0; i < k; ++i) { z[i] = p.z[(size_t)i * Cl + c]; dp[i] = p.dvp[(size_t)i * Cl + c]; ds[i] = p.dvs[(size_t)i * Cl + c]; }
-    for (int i = 1; i < k; ++i) {
-      const double a = z[i], b = dp[i], d = ds[i];
-      int m = i - 1;
-      while (m >= 0 && z[m] > a) { z[m + 1] = z[m]; dp[m + 1] = dp[m]; ds[m + 1] = ds[m]; --m; }
-      z[m + 1] = a; dp[m + 1] = b; ds[m + 1] = d;
-    }
-    int n = 0;
-    double tmpz = 0.0;
-    if (cfg.sdep > 0.0) {
-      s_alpha[n] = 1.5; s_beta[n] = -999.0; s_iz1[n] = (int)(tmpz / dbin_z) + 1;
-      tmpz = __dadd_rn(tmpz, cfg.sdep); ++n;
-    }
-    for (int l = 0; l <= k; ++l) {
-      double zc, h, dvs_l, dvp_l;
-      if (l == 0) { zc = __dmul_rn(0.5, __dadd_rn(cfg.sdep, z[0])); h = __dsub_rn(z[0], cfg.sdep); dvs_l = ds[0]; dvp_l = dp[0]; }
-      else if (l < k) { zc = __dmul_rn(0.5, __dadd_rn(z[l], z[l - 1])); h = __dsub_rn(z[l], z[l - 1]); dvs_l = ds[l]; dvp_l = dp[l]; }
-      else { zc = __dmul_rn(0.5, __dadd_rn(cfg.z_max, z[k - 1])); h = 999.0;
-             dvs_l = p.dvs[(size_t)(km - 1) * Cl + c]; dvp_l = p.dvp[(size_t)(km - 1) * Cl + c]; }
-      double a, b;
-      layer_velocity(cfg, zc, dvs_l, dvp_l, a, b);
-      s_alpha[n] = a; s_beta[n] = b;
-      s_iz1[n] = (int)(__ddiv_rn(tmpz, dbin_z)) + 1;
-      tmpz = __dadd_rn(tmpz, h);
-      ++n;
-    }
-    s_iz1[n] = p.nbin_z + 1;   // iz2 of the half space (src/pt_mcmc.f90:243)
-    s_nlay = n;
+    s_nlay = pt_format_layers(cfg, p, c, dbin_z, s_alpha, s_beta, s_iz1);
   }
   __syncthreads();
   const int nlay = s_nlay;
   // each depth bin belongs to exactly one layer: iz1(l) <= iz < iz1(l+1)
   for (int iz = 1 + tid; iz <= p.nbin_z; iz += nthr) {
-    int l = 0;
-    while (l + 1 < nlay && iz >= s_iz1[l + 1]) ++l;
-    if (iz < s_iz1[l]) continue;
+    const int l = pt_bin_layer(s_iz1, nlay, iz);
+    if (l < 0) continue;
     const double a = s_alpha[l], b = s_beta[l];
     int ivp = (int)((a - cfg.vp_min) / dbin_vp) + 1;
     int ivs = (int)((b - cfg.vs_min) / dbin_vs) + 1;
@@ -1101,16 +1139,14 @@ __global__ void pt_record_kernel(const DevConfig cfg, const PtDev p) {
     atomicAdd(&p.vp_mean[iz - 1], a);
     atomicAdd(&p.nvsz[(size_t)(ivs - 1) * p.nbin_z + iz - 1], 1ULL);
     atomicAdd(&p.nvpvsz[(size_t)(ivpvs - 1) * p.nbin_z + iz - 1], 1ULL);
-    double vs_rec;
+    const double vs_rec = pt_recorded_vs(cfg, b);
     if (b > 0.0) {
       atomicAdd(&p.vpvs_mean[iz - 1], a / b);
       atomicAdd(&p.vs_mean[iz - 1], b);
-      vs_rec = b;
     } else {  // src/pt_mcmc.f90:260-263: assignment, not accumulation (ocean layer)
       p.vpvs_mean[iz - 1] = cfg.vpvs_min;
       p.vs_mean[iz - 1] = cfg.vs_min;
       p.ocean_bin[iz - 1] = 1;
-      vs_rec = cfg.vs_min;
     }
     if (p.vp_model && imod < p.cap_models) {
       p.vp_model[(size_t)imod * p.nbin_z + iz - 1] = a;
@@ -1133,6 +1169,206 @@ __global__ void pt_record_finish_kernel(const PtDev p) { *p.nmod += (unsigned lo
 __global__ void pt_fix_ocean_kernel(const DevConfig cfg, const PtDev p) {
   const int iz = blockIdx.x * blockDim.x + threadIdx.x;
   if (iz < p.nbin_z && p.ocean_bin[iz]) { p.vs_mean[iz] = cfg.vs_min; p.vpvs_mean[iz] = cfg.vpvs_min; }
+}
+
+// ---------------- convergence diagnostics (rfinv_pt_set_diagnostics, DESIGN.md 7f) ----------------
+// Cold-level trace, one WARP per virtual rank, behind the bookkeeping kernels of a recording iteration (the temperatures at
+// acceptance): level 0 of the rank -- its chain of lowest (temperature, chain index) -- writes k, logL, its solved sigmas and
+// the Vs the bookkeeping assigns to each chosen depth bin into row [sample][rank], and its temperature into t0.  peer: the
+// peer-memory exchange, where pt_finish_kernel has already advanced *it_dev.
+constexpr int PT_TR_WARPS = 4;
+__global__ void __launch_bounds__(32 * PT_TR_WARPS) pt_trace_kernel(const DevConfig cfg, const PtDev p, int peer) {
+  __shared__ double s_alpha[PT_TR_WARPS][RFINV_MAX_LAY], s_beta[PT_TR_WARPS][RFINV_MAX_LAY];
+  __shared__ int s_iz1[PT_TR_WARPS][RFINV_MAX_LAY + 1];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, n = p.nchains;
+  const int r = blockIdx.x * PT_TR_WARPS + warp;
+  if (r >= p.G) return;
+  const int it = *p.it_dev - peer + 1;   // this iteration, 1-based: it > nburn, it % ncorr == 0
+  const long long smp = (long long)(it / p.ncorr) - (long long)(p.nburn / p.ncorr) - 1;
+  if (smp < 0 || smp >= p.dg_cap) return;
+  const int c0 = r * n;
+  double tb = 0.0;
+  int ib = n;
+  for (int a = lane; a < n; a += 32) {
+    const double t = p.temps[c0 + a];
+    if (ib == n || t < tb) { tb = t; ib = a; }   // (ascending a: the first of equal temperatures stays)
+  }
+  for (int o = 16; o > 0; o >>= 1) {
+    const double t = __shfl_xor_sync(0xffffffffu, tb, o);
+    const int i = __shfl_xor_sync(0xffffffffu, ib, o);
+    if (i != n && (ib == n || t < tb || (t == tb && i < ib))) { tb = t; ib = i; }
+  }
+  const int c = c0 + ib;
+  PT_DG_ASSERT(ib >= 0 && ib < n && p.dg_nq == 2 + p.nsig_trc + p.dg_nbins);
+  double* row = p.dg_trace + ((size_t)smp * p.G + r) * p.dg_nq;
+  int nlay = 0;
+  if (lane == 0) {
+    row[0] = (double)p.k[c];
+    row[1] = p.logl[c];
+    for (int j = 0; j < p.nsig_trc; ++j) row[2 + j] = p.sig[(size_t)p.isig_trc[j] * p.Cl + c];
+    p.dg_t0[(size_t)smp * p.G + r] = tb;
+    if (p.dg_nbins > 0) nlay = pt_format_layers(cfg, p, c, (cfg.z_max - 0.0) / p.nbin_z, s_alpha[warp], s_beta[warp], s_iz1[warp]);
+  }
+  nlay = __shfl_sync(0xffffffffu, nlay, 0);
+  __syncwarp();   // lane 0's layers in shared memory are visible to the warp
+  PT_DG_ASSERT(p.dg_nbins == 0 || (nlay >= 1 && nlay <= RFINV_MAX_LAY));
+  for (int j = lane; j < p.dg_nbins; j += 32) {
+    PT_DG_ASSERT(p.dg_bins[j] >= 1 && p.dg_bins[j] <= p.nbin_z);
+    const int l = pt_bin_layer(s_iz1[warp], nlay, p.dg_bins[j]);
+    PT_DG_ASSERT(l < nlay);
+    row[2 + p.nsig_trc + j] = l < 0 ? __longlong_as_double(0x7ff8000000000000LL) : pt_recorded_vs(cfg, s_beta[warp][l]);
+  }
+}
+
+// Statistics of the sample series, one CTA per (rank, quantity).  Every sum is taken in an order that depends only on the
+// number of samples n -- thread t adds the elements t, t + 256, ... in order, then a fixed tree -- so a row does not depend on
+// the number of ranks, the launch shape or the split over processes.
+constexpr int PT_DG_THREADS = 256;
+constexpr int PT_DG_SMEM_MAX = 192 * 1024;   // series up to this many bytes are centred into shared memory, longer ones re-read
+
+// sum over the CTA of one value per thread (thread 0 gets it), fixed order
+__device__ double pt_dg_block_sum(double v, double* s_red) {
+  const int tid = threadIdx.x;
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
+  __syncthreads();   // (s_red is reused)
+  if ((tid & 31) == 0) s_red[tid >> 5] = v;
+  __syncthreads();
+  double acc = 0.0;
+  if (tid == 0) for (int w = 0; w < PT_DG_THREADS / 32; ++w) acc += s_red[w];
+  return acc;
+}
+
+// x[i] = trace[(i * G + r) * nq + q]; row: mean (x[lo] + sum(x - x[lo]) / len), variance (n - 1), tau (Sokal, c = 5), ESS = n / tau, mean and variance (h - 1)
+// of [0, h) and of [n - h, n) with h = n / 2, and the count of samples whose t0 is tempered
+__global__ void __launch_bounds__(PT_DG_THREADS) pt_diag_kernel(const double* __restrict__ trace, const double* __restrict__ t0,
+                                                                int G, int nq, int n, int use_smem, double* __restrict__ rows) {
+  extern __shared__ double dg_smem[];
+  __shared__ double s_red[PT_DG_THREADS / 32], s_lag[PT_DG_THREADS / 32], s_bc[2];
+  __shared__ int s_stop;
+  const int r = blockIdx.x / nq, q = blockIdx.x - r * nq, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const size_t stride = (size_t)G * nq;
+  const double* x = trace + (size_t)r * nq + q;
+  const double nan = __longlong_as_double(0x7ff8000000000000LL);
+  auto sum_of = [&](auto f, int lo, int hi) {   // sum of f(i) over [lo, hi)
+    double v = 0.0;
+    for (int i = lo + tid; i < hi; i += PT_DG_THREADS) v += f(i);
+    return pt_dg_block_sum(v, s_red);
+  };
+  auto xi = [&](int i) { return __ldg(x + (size_t)i * stride); };
+  auto mean_var = [&](int lo, int hi, double& m, double& v) {   // (every thread gets them)
+    // shifted by the first element: a constant stretch has its value as mean and variance 0 exactly
+    const int len = hi - lo;
+    const double x0 = len > 0 ? xi(lo) : 0.0;
+    const double s = sum_of([&](int i) { return xi(i) - x0; }, lo, hi);
+    if (tid == 0) s_bc[0] = x0 + s / len;
+    __syncthreads();
+    const double mu = s_bc[0];
+    const double ss = sum_of([&](int i) { const double d = xi(i) - mu; return d * d; }, lo, hi);
+    if (tid == 0) s_bc[1] = len > 1 ? ss / (len - 1) : nan;
+    __syncthreads();
+    m = len > 0 ? mu : nan;
+    v = s_bc[1];
+    __syncthreads();
+  };
+  double mean, var, m1, v1, m2, v2;
+  mean_var(0, n, mean, var);
+  const int h = n / 2;
+  mean_var(0, h, m1, v1);
+  mean_var(n - h, n, m2, v2);
+  PT_DG_ASSERT(r < G && q < nq && (!use_smem || (size_t)n * sizeof(double) <= (size_t)PT_DG_SMEM_MAX));
+  const double tempered = sum_of([&](int i) { return __ldg(t0 + (size_t)i * G + r) > 1.0 + (double)1.0e-6f ? 1.0 : 0.0; }, 0, n);
+  // tau: NaN for n < 4 or a constant series
+  const double x0 = n > 0 ? xi(0) : 0.0;
+  const double differ = sum_of([&](int i) { return xi(i) != x0 ? 1.0 : 0.0; }, 0, n);
+  if (tid == 0) s_stop = n < 4 || differ == 0.0;
+  __syncthreads();
+  double tau = nan;
+  if (!s_stop) {
+    double* d = dg_smem;
+    if (use_smem) {
+      for (int i = tid; i < n; i += PT_DG_THREADS) d[i] = xi(i) - mean;
+      __syncthreads();
+    }
+    auto di = [&](int i) { return use_smem ? d[i] : xi(i) - mean; };
+    // lags in batches of one per warp: warp w sums d[i] d[i + t] over i = lane, lane + 32, ... and its tree; thread 0 walks the
+    // batch in lag order and stops at the first m >= 5 tau
+    double S0 = 0.0, acc = 1.0;
+    for (int t0l = 0; t0l < n; t0l += PT_DG_THREADS / 32) {
+      const int t = t0l + warp;
+      double v = 0.0;
+      if (t < n)
+        for (int i = lane; i < n - t; i += 32) v += di(i) * di(i + t);
+      for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
+      if (lane == 0) s_lag[warp] = v;
+      __syncthreads();
+      if (tid == 0) {
+        for (int w = 0; w < PT_DG_THREADS / 32 && !s_stop; ++w) {
+          const int m = t0l + w;
+          if (m == 0) { S0 = s_lag[w]; continue; }
+          if (m >= n) { s_stop = 1; break; }
+          acc += 2.0 * (s_lag[w] / S0);
+          if (m >= 5.0 * acc) s_stop = 1;
+        }
+        if (t0l + PT_DG_THREADS / 32 >= n) s_stop = 1;
+      }
+      __syncthreads();
+      if (s_stop) break;
+    }
+    tau = acc;   // (thread 0's)
+  }
+  if (tid == 0) {
+    double* o = rows + (size_t)blockIdx.x * PT_DG_ROW;
+    o[0] = mean; o[1] = var; o[2] = tau; o[3] = n / tau; o[4] = m1; o[5] = v1; o[6] = m2; o[7] = v2; o[8] = tempered;
+  }
+}
+
+// Across ranks, one CTA per quantity, in global rank order: split-R-hat over the 2G half-chains (BDA3), the sum of the ESS and
+// the median tau over the ranks with finite tau, and the tempered share (from the rows of quantity 0).
+// out[q]: R-hat, ESS, median tau, tempered share.
+__global__ void __launch_bounds__(PT_DG_THREADS) pt_diag_combine_kernel(const double* __restrict__ rows, int G, int nq, int n,
+                                                                        double* __restrict__ out) {
+  __shared__ double s_med[2];
+  const int q = blockIdx.x, tid = threadIdx.x;
+  const double nan = __longlong_as_double(0x7ff8000000000000LL);
+  auto row = [&](int r) { return rows + ((size_t)r * nq + q) * PT_DG_ROW; };
+  // median: the finite taus ranked by (value, rank) through counting
+  int m = 0;
+  for (int r = 0; r < G; ++r) m += isfinite(row(r)[2]) ? 1 : 0;
+  if (tid < 2) s_med[tid] = nan;
+  __syncthreads();
+  for (int r = tid; r < G; r += PT_DG_THREADS) {
+    const double t = row(r)[2];
+    if (!isfinite(t)) continue;
+    int pos = 0;
+    for (int j = 0; j < G; ++j) { const double u = row(j)[2]; pos += isfinite(u) && (u < t || (u == t && j < r)); }
+    if (pos == (m - 1) / 2) s_med[0] = t;
+    if (pos == m / 2) s_med[1] = t;
+  }
+  __syncthreads();
+  if (tid != 0) return;
+  const int h = n / 2;
+  double sw = 0.0, sm = 0.0, ess = 0.0, tmp = 0.0;
+  for (int r = 0; r < G; ++r) {
+    const double* o = row(r);
+    sw += o[5]; sw += o[7]; sm += o[4]; sm += o[6];
+    if (isfinite(o[2])) ess += o[3];
+    tmp += rows[(size_t)r * nq * PT_DG_ROW + 8];
+  }
+  const double W = sw / (2.0 * G), mbar = sm / (2.0 * G);
+  double sb = 0.0;
+  for (int r = 0; r < G; ++r) {
+    const double* o = row(r);
+    const double a = o[4] - mbar, b = o[6] - mbar;
+    sb += a * a; sb += b * b;
+  }
+  const double B_h = sb / (2.0 * G - 1.0);
+  double rhat = nan;
+  if (h >= 2 && W != 0.0) rhat = sqrt(((double)(h - 1) / h * W + B_h) / W);
+  double* o = out + (size_t)q * 4;
+  o[0] = rhat;
+  o[1] = ess;
+  o[2] = m > 0 ? (s_med[0] + s_med[1]) / 2.0 : nan;
+  o[3] = n > 0 ? tmp / ((double)G * n) : nan;
 }
 
 template <typename T>
@@ -1172,6 +1408,8 @@ void rfinv_handle::free_pt() {
   cudaFree(d.nprop); cudaFree(d.naccept); cudaFree(d.n_eval); cudaFree(d.rs_nprop); cudaFree(d.rs_nacc); cudaFree(d.rs_arrived);
   cudaFree(d.rs_base); cudaFree(d.st_scale); cudaFree(d.st_nprop); cudaFree(d.st_nacc); cudaFree(d.st_lvl); cudaFree(d.st_pair);
   cudaFree(d.log_flags); cudaFree(d.log_itypes); cudaFree(d.log_swaps);
+  cudaFree(d.dg_bins); cudaFree(d.dg_trace); cudaFree(d.dg_t0); cudaFree(d.dg_trip_st); cudaFree(d.dg_trips);
+  cudaFree(pt->dg_job_rows); cudaFree(pt->dg_job_trips);
   cudaFree(d.nk); cudaFree(d.nz); cudaFree(d.nsig); cudaFree(d.namp); cudaFree(d.nvpz); cudaFree(d.nvsz); cudaFree(d.nvpvsz); cudaFree(d.nmod);
   cudaFree(d.vp_mean); cudaFree(d.vs_mean); cudaFree(d.vpvs_mean); cudaFree(d.vp_model); cudaFree(d.vs_model); cudaFree(d.cold_ordinal); cudaFree(d.cold_count); cudaFree(d.ocean_bin);
   cudaFree(pt->d_lhist); cudaFree(pt->d_lh_part); cudaFree(pt->d_lh_cnt); cudaFree(pt->d_table); cudaFree(pt->d_gather); cudaFree(d.it_dev);
@@ -1519,6 +1757,114 @@ int32_t rfinv_pt_get_rank_swaps(rfinv_handle* h, int32_t* mode, int64_t* n_prop,
   return RFINV_OK;
 }
 
+int32_t rfinv_pt_set_diagnostics(rfinv_handle* h, int32_t on, int32_t n_bins, const int32_t* vs_bins) {
+  static const char* who = "rfinv_pt_set_diagnostics";
+  int st = pt_require(h, who);
+  if (st != RFINV_OK) return st;
+  PtState* s = h->pt;
+  PtDev& d = s->dev;
+  if (on != 0 && on != 1) { rfinv_set_error("%s: %d (0: off, 1: record the cold-level trace and the round trips)", who, on); return RFINV_ERR_ARG; }
+  if (n_bins < 0 || n_bins > 16 || (n_bins > 0 && !vs_bins)) {
+    rfinv_set_error("%s: %d depth bins (0 to 16, and the list must not be NULL)", who, n_bins);
+    return RFINV_ERR_ARG;
+  }
+  for (int j = 0; j < n_bins; ++j)
+    if (vs_bins[j] < 1 || vs_bins[j] > d.nbin_z) {
+      rfinv_set_error("%s: depth bin %d is outside [1, nbin_z = %d]", who, vs_bins[j], d.nbin_z);
+      return RFINV_ERR_ARG;
+    }
+  if (s->step_pending) {
+    rfinv_set_error("%s: an iteration is half done (rfinv_pt_local_step without rfinv_pt_apply_swap)", who);
+    return RFINV_ERR_STATE;
+  }
+  if (s->reduced) { rfinv_set_error("%s: rfinv_pt_reduce_outputs has run", who); return RFINV_ERR_STATE; }
+  if (s->it_done > 0) {
+    rfinv_set_error("%s: %d iterations have run; the diagnostics start with the run (before its first iteration or a restore)", who, s->it_done);
+    return RFINV_ERR_STATE;
+  }
+  if (on && !s->record) {
+    rfinv_set_error("%s: the diagnostics record with the posterior bookkeeping, which is off (needs niter > 0 and all nbin_* > 0)", who);
+    return RFINV_ERR_STATE;
+  }
+  RFINV_CUDA_CHECK(cudaSetDevice(h->device));
+  RFINV_CUDA_CHECK(cudaStreamSynchronize(h->stream));
+  cudaFree(d.dg_bins); cudaFree(d.dg_trace); cudaFree(d.dg_t0); cudaFree(d.dg_trip_st); cudaFree(d.dg_trips);
+  d.dg_bins = nullptr; d.dg_trace = nullptr; d.dg_t0 = nullptr; d.dg_trip_st = nullptr; d.dg_trips = nullptr;
+  d.dg_nq = d.dg_nbins = 0; d.dg_cap = 0;
+  pt_drop_graphs(s);   // the captured launches carry the flag and the pointers
+  d.dg_on = 0;
+  if (!on) return RFINV_OK;
+  const long long cap = pt_diag_samples(h->cfg.nburn + h->cfg.niter, d.nburn, d.ncorr);
+  const int nq = 2 + d.nsig_trc + n_bins;
+  if ((st = dalloc(&d.dg_bins, (size_t)n_bins)) != RFINV_OK) return st;
+  if ((st = dalloc(&d.dg_trace, (size_t)cap * d.G * nq)) != RFINV_OK) return st;
+  if ((st = dalloc(&d.dg_t0, (size_t)cap * d.G)) != RFINV_OK) return st;
+  if ((st = dalloc(&d.dg_trip_st, (size_t)d.Cl)) != RFINV_OK) return st;
+  if ((st = dalloc(&d.dg_trips, (size_t)d.G * 2)) != RFINV_OK) return st;
+  if (n_bins) RFINV_CUDA_CHECK(cudaMemcpy(d.dg_bins, vs_bins, sizeof(int32_t) * n_bins, cudaMemcpyHostToDevice));
+  d.dg_nq = nq; d.dg_nbins = n_bins; d.dg_cap = cap;
+  d.dg_on = 1;
+  return RFINV_OK;
+}
+
+int32_t rfinv_pt_get_cold_trace(rfinv_handle* h, int32_t* on, int32_t* n_quantities, int32_t* n_bins, int32_t* vs_bins,
+                                int64_t max_samples, int64_t* n_samples, double* trace, double* t0) {
+  int st = pt_require(h, "rfinv_pt_get_cold_trace");
+  if (st != RFINV_OK) return st;
+  PtState* s = h->pt;
+  PtDev& d = s->dev;
+  RFINV_CUDA_CHECK(cudaSetDevice(h->device));
+  RFINV_CUDA_CHECK(cudaStreamSynchronize(h->stream));
+  if (on) *on = d.dg_on;
+  if (n_quantities) *n_quantities = d.dg_nq;
+  if (n_bins) *n_bins = d.dg_nbins;
+  if (vs_bins && d.dg_nbins) RFINV_CUDA_CHECK(cudaMemcpy(vs_bins, d.dg_bins, sizeof(int32_t) * d.dg_nbins, cudaMemcpyDeviceToHost));
+  long long n = d.dg_on ? std::min(pt_diag_samples(s->it_done, d.nburn, d.ncorr), d.dg_cap) : 0;
+  if (n > max_samples) n = max_samples < 0 ? 0 : max_samples;
+  if (n_samples) *n_samples = n;
+  if (n > 0 && trace) RFINV_CUDA_CHECK(cudaMemcpy(trace, d.dg_trace, sizeof(double) * (size_t)n * d.G * d.dg_nq, cudaMemcpyDeviceToHost));
+  if (n > 0 && t0) RFINV_CUDA_CHECK(cudaMemcpy(t0, d.dg_t0, sizeof(double) * (size_t)n * d.G, cudaMemcpyDeviceToHost));
+  return RFINV_OK;
+}
+
+int32_t rfinv_pt_get_diagnostics(rfinv_handle* h, int64_t* n_samples, int32_t* n_ranks, int32_t* n_quantities, double* rows,
+                                 double* summary, int64_t* trips) {
+  static const char* who = "rfinv_pt_get_diagnostics";
+  int st = pt_require(h, who);
+  if (st != RFINV_OK) return st;
+  PtState* s = h->pt;
+  PtDev& d = s->dev;
+  if (!d.dg_on) { rfinv_set_error("%s: the diagnostics are off (rfinv_pt_set_diagnostics)", who); return RFINV_ERR_STATE; }
+  const bool job = s->dg_job_rows != nullptr;
+  const int G = job ? d.nproc_total : d.G, nq = d.dg_nq;
+  const long long n = std::min(pt_diag_samples(s->it_done, d.nburn, d.ncorr), d.dg_cap);
+  if (n_samples) *n_samples = n;
+  if (n_ranks) *n_ranks = G;
+  if (n_quantities) *n_quantities = nq;
+  RFINV_CUDA_CHECK(cudaSetDevice(h->device));
+  if (trips) {
+    RFINV_CUDA_CHECK(cudaStreamSynchronize(h->stream));
+    RFINV_CUDA_CHECK(cudaMemcpy(trips, job ? s->dg_job_trips : d.dg_trips, sizeof(int64_t) * 2 * (size_t)G, cudaMemcpyDeviceToHost));
+  }
+  if (!rows && !summary) return RFINV_OK;
+  const size_t nrow = (size_t)G * nq * PT_DG_ROW;
+  double *d_rows = nullptr, *d_sum = nullptr;
+  RFINV_CUDA_CHECK(cudaMalloc((void**)&d_rows, sizeof(double) * (nrow + (size_t)nq * 4)));
+  d_sum = d_rows + nrow;
+  if (job) st = cudaMemcpyAsync(d_rows, s->dg_job_rows, sizeof(double) * nrow, cudaMemcpyDeviceToDevice, h->stream) == cudaSuccess ? RFINV_OK : RFINV_ERR_CUDA;
+  else st = rfinv_pt_diag_rows(h, d_rows);
+  if (st == RFINV_OK) {
+    pt_diag_combine_kernel<<<nq, PT_DG_THREADS, 0, h->stream>>>(d_rows, G, nq, (int)n, d_sum);
+    cudaError_t e = cudaGetLastError();
+    if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
+    if (e == cudaSuccess && rows) e = cudaMemcpy(rows, d_rows, sizeof(double) * nrow, cudaMemcpyDeviceToHost);
+    if (e == cudaSuccess && summary) e = cudaMemcpy(summary, d_sum, sizeof(double) * nq * 4, cudaMemcpyDeviceToHost);
+    if (e != cudaSuccess) { rfinv_set_error("%s: %s", who, cudaGetErrorString(e)); st = RFINV_ERR_CUDA; }
+  }
+  cudaFree(d_rows);
+  return st;
+}
+
 // room in the likelihood history for iterations [0, upto); never called while a launch sequence is being captured
 static int pt_reserve_lhist(rfinv_handle* h, int upto) {
   PtState* s = h->pt;
@@ -1588,6 +1934,7 @@ static int pt_enqueue_local(rfinv_handle* h, bool record, bool peer_exchange = f
     pt_coldscan_kernel<<<1, 1024, 0, q>>>(d);
     pt_record_kernel<<<d.Cl, 128, 0, q>>>(h->dc, d);
     pt_record_finish_kernel<<<1, 1, 0, q>>>(d);
+    if (d.dg_on) pt_trace_kernel<<<(d.G + PT_TR_WARPS - 1) / PT_TR_WARPS, 32 * PT_TR_WARPS, 0, q>>>(h->dc, d, peer ? 1 : 0);
   }
   if (sweep) {   // after the bookkeeping (it sees the temperatures at acceptance), before the global swap reads the table
     const int warps = d.nchains <= 3072 ? PT_RS_WARPS : 1;
@@ -1884,6 +2231,20 @@ int32_t rfinv_pt_get_log(rfinv_handle* h, int8_t* flags, int8_t* itypes, int32_t
 }  // extern "C"
 
 int rfinv_pt_reserve_lhist(rfinv_handle* h, int upto) { return pt_reserve_lhist(h, upto); }
+
+int rfinv_pt_diag_rows(rfinv_handle* h, double* rows) {
+  const PtState* s = h->pt;
+  const PtDev& d = s->dev;
+  const long long n = std::min(pt_diag_samples(s->it_done, d.nburn, d.ncorr), d.dg_cap);
+  if (d.G * d.dg_nq == 0) return RFINV_OK;
+  const size_t bytes = sizeof(double) * (size_t)n;
+  const int use_smem = bytes <= (size_t)PT_DG_SMEM_MAX;
+  const size_t smem = use_smem ? bytes : 0;
+  RFINV_CUDA_CHECK(rfinv_raise_smem_limit((const void*)pt_diag_kernel, smem));
+  pt_diag_kernel<<<d.G * d.dg_nq, PT_DG_THREADS, smem, h->stream>>>(d.dg_trace, d.dg_t0, d.G, d.dg_nq, (int)n, use_smem, rows);
+  RFINV_CUDA_CHECK(cudaGetLastError());
+  return RFINV_OK;
+}
 
 // ---------------- several single-process runs advanced together (rfinv_pt_group_*) ----------------
 // One iteration of every member is ONE graph: the group's stream forks to the members' capture streams, each member's own

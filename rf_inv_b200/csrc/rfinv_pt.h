@@ -58,6 +58,15 @@ struct PtDev {
   int* st_pair;                   // [2] global chains of the previous iteration's global swap (-1: none yet)
   double st_target;               // acceptance rate the widths are tuned towards
   int st_on;                      // 1: proposals use the tuned widths, pt_rank_swap_kernel tunes them at the tuning points
+  // convergence diagnostics (rfinv_pt_set_diagnostics, DESIGN.md 7f); allocated by the switch on
+  int dg_on;                      // 1: pt_trace_kernel records level 0 of every rank, pt_rank_swap_kernel counts round trips
+  int dg_nq, dg_nbins;            // quantities per trace row (k, logL, the solved sigmas, the Vs bins) and Vs bins among them
+  int* dg_bins;                   // [dg_nbins] 1-based depth bins
+  long long dg_cap;               // samples the trace holds (recording iterations in [1, nburn + niter])
+  double* dg_trace;               // [dg_cap][G][dg_nq]
+  double* dg_t0;                  // [dg_cap][G] temperature of level 0
+  int8_t* dg_trip_st;             // [Cl] 0 none, 1 came from level 0, 2 reached level nchains - 1 after level 0
+  unsigned long long* dg_trips;   // [G][2] round trips completed during the burn-in / after it (one writer per row)
 };
 
 struct ncclComm;   // NCCL communicator (comm.cu)
@@ -132,10 +141,26 @@ struct PtState {
   int rank_swaps = 0;          // rfinv_pt_set_rank_swaps: 0 the reference's global swap only, 1 the rank sweep before it
   int tune_points_off = 0;     // tuning points passed while the ladder tuning was on, frozen when it is switched off
   int step_points_off = 0;     // likewise for the step tuning
+  // convergence diagnostics after rfinv_pt_reduce_outputs, on process 0: the per-rank rows and round trips of the job, in
+  // global rank order (nullptr: the getter works on this process's ranks)
+  double* dg_job_rows = nullptr;                 // [nproc_total][dg_nq][PT_DG_ROW]
+  unsigned long long* dg_job_trips = nullptr;    // [nproc_total][2]
 };
 
 // does an iteration of this state run the rank sweep?  (nothing to pair with fewer than two chains per rank)
 inline bool pt_sweeps(const PtState* s) { return s->rank_swaps == 1 && s->dev.nchains >= 2; }
+
+// recording iterations (it > nburn, it % ncorr == 0) among the first it_done iterations: samples of the cold-level trace
+inline long long pt_diag_samples(int it_done, int nburn, int ncorr) {
+  const long long n = (long long)(it_done / ncorr) - (long long)(nburn / ncorr);
+  return n > 0 ? n : 0;
+}
+// one row of per-rank statistics (rfinv_pt_get_diagnostics): mean, variance, tau, ESS, the two halves' means and variances,
+// tempered samples of the rank
+constexpr int PT_DG_ROW = 9;
+// rows of this process's ranks from its trace: rows[G][nq][PT_DG_ROW], device memory, on the handle's stream
+struct rfinv_handle;
+int rfinv_pt_diag_rows(rfinv_handle* h, double* rows);
 
 // the tuning points e = 2^j, j >= 6, e <= nburn among the first it_done iterations (DESIGN.md 7d, 7e)
 inline int pt_tuning_points(int it_done, int nburn) {

@@ -167,6 +167,60 @@ class ParallelTempering:
         return dict(on=bool(on.value), target=float(target.value), n_points=int(n.value), widths=widths, n_prop=n_prop,
                     n_acc=n_acc)
 
+    # -- convergence diagnostics (DESIGN.md 7f) -------------------------------------------------------------------------
+    def set_diagnostics(self, on: bool, vs_bins=()) -> None:
+        """Before the first iteration (and before restore()), with the posterior bookkeeping on: every recording iteration
+        also records level 0 of every virtual rank -- k, logL, the solved sigmas and the Vs of each 1-based depth bin in
+        `vs_bins` (at most 16) -- and, in mode 1, every rank counts the round trips of its chains between the coldest and the
+        hottest level.  The run itself is unchanged bit for bit."""
+        bins = np.ascontiguousarray(vs_bins, dtype=np.int32).reshape(-1)
+        capi.check(self._lib.rfinv_pt_set_diagnostics(self.ev.handle, int(on), len(bins), _p(bins, capi.i32p)))
+
+    def quantity_names(self, vs_bins=None):
+        """k, logL, sig_<t> (1-based trace number of every solved sigma), vs_bin<b> -- the order of a trace row."""
+        if vs_bins is None:
+            vs_bins = self.diagnostics_setting()[1]
+        return (["k", "logL"] + [f"sig_{t + 1}" for t, m in enumerate(self.cfg.sig_mode) if m]
+                + [f"vs_bin{int(b)}" for b in vs_bins])
+
+    def diagnostics_setting(self) -> Tuple[bool, np.ndarray]:
+        """(on, depth bins), without copying the trace."""
+        on, nb = C.c_int32(0), C.c_int32(0)
+        bins = np.zeros(16, np.int32)
+        capi.check(self._lib.rfinv_pt_get_cold_trace(self.ev.handle, C.byref(on), None, C.byref(nb), _p(bins, capi.i32p), 0,
+                                                     None, None, None))
+        return bool(on.value), bins[:nb.value].copy()
+
+    def cold_trace(self) -> Dict[str, object]:
+        """{on, vs_bins, trace [samples][local ranks][quantities], t0 [samples][local ranks]}: this process's recorded samples."""
+        on, nq, nb, ns = C.c_int32(0), C.c_int32(0), C.c_int32(0), C.c_int64(0)
+        bins = np.zeros(16, np.int32)
+        capi.check(self._lib.rfinv_pt_get_cold_trace(self.ev.handle, C.byref(on), C.byref(nq), C.byref(nb), _p(bins, capi.i32p),
+                                                     2 ** 62, C.byref(ns), None, None))
+        cap = int(ns.value)
+        trace = np.zeros((cap, self.rank_count, nq.value)); t0 = np.zeros((cap, self.rank_count))
+        capi.check(self._lib.rfinv_pt_get_cold_trace(self.ev.handle, None, None, None, None, cap, C.byref(ns),
+                                                     _p(trace, capi.dp), _p(t0, capi.dp)))
+        return dict(on=bool(on.value), vs_bins=bins[:nb.value].copy(), trace=trace[:ns.value], t0=t0[:ns.value])
+
+    def diagnostics(self) -> Dict[str, object]:
+        """Statistics of the recorded samples, computed on the device (rfinv_pt_get_diagnostics): n_samples, n_ranks, names,
+        per-rank arrays [ranks][quantities] mean, var, tau, ess, mean_1, var_1, mean_2, var_2 (the two halves), tempered (the
+        rank's samples with a tempered level 0); per quantity rhat, ess_total, tau_median, tempered_share; trips [ranks][2]
+        (during the burn-in, after it).  Over this process's ranks, over the job on process 0 after reduce_outputs()."""
+        ns, nr, nq = C.c_int64(0), C.c_int32(0), C.c_int32(0)
+        capi.check(self._lib.rfinv_pt_get_diagnostics(self.ev.handle, C.byref(ns), C.byref(nr), C.byref(nq), None, None, None))
+        rows = np.zeros((nr.value, nq.value, 9)); summary = np.zeros((nq.value, 4)); trips = np.zeros((nr.value, 2), np.int64)
+        capi.check(self._lib.rfinv_pt_get_diagnostics(self.ev.handle, C.byref(ns), C.byref(nr), C.byref(nq), _p(rows, capi.dp),
+                                                      _p(summary, capi.dp), _p(trips, capi.i64p)))
+        out = dict(n_samples=int(ns.value), n_ranks=int(nr.value), names=self.quantity_names(), trips=trips)
+        for i, key in enumerate(("mean", "var", "tau", "ess", "mean_1", "var_1", "mean_2", "var_2")):
+            out[key] = rows[:, :, i]
+        out["tempered"] = rows[:, 0, 8].astype(np.int64)
+        for i, key in enumerate(("rhat", "ess_total", "tau_median", "tempered_share")):
+            out[key] = summary[:, i]
+        return out
+
     # -- results ----------------------------------------------------------------------------------
     def set_logging(self, cap_iters: int) -> None:
         capi.check(self._lib.rfinv_pt_set_logging(self.ev.handle, int(cap_iters)))

@@ -26,7 +26,13 @@ burn-in.  It adds OUT_DIR/ladder: one line per virtual rank, its temperatures by
 virtual rank and level at the same iteration counts towards the acceptance rate ``--step-target`` (default 0.44; DESIGN.md
 7e); the widths are fixed after the burn-in.  It adds OUT_DIR/step_widths: one line per virtual rank and level,
 ``rank level w_z w_dvs w_dvp w_sig acc_z acc_dvs acc_dvp acc_sig`` -- the final widths and the acceptance they produced since
-the last tuning point (-1 without proposals)."""
+the last tuning point (-1 without proposals).
+
+``--diagnostics`` records level 0 of every virtual rank (its coldest chain) at every recording iteration and reports whether the
+run has converged (DESIGN.md 7f): OUT_DIR/convergence has one line per quantity -- ``name samples ranks R-hat ESS tau_median
+tempered_share`` for k, logL, every solved sigma (``sig_<trace>``) and the Vs at each depth of ``--diag-depths KM,KM,...``
+(``vs_<km>``).  With the rank swaps it adds OUT_DIR/round_trips: ``rank trips_burn_in trips_after`` per virtual rank.  The
+reference's files are written as without it."""
 from __future__ import annotations
 
 import argparse
@@ -98,6 +104,55 @@ def write_step_widths(out_dir: str, rows) -> None:
                     + " ".join(f"{x:.6f}" for x in row[6:]) + "\n")
 
 
+def depth_bins(cfg, depths):
+    """The bookkeeping's depth bins int(z / dbin_z) + 1 of depths in km, the bottom z_max in the last bin nbin_z; a depth
+    outside [0, z_max] or inside the sea layer is refused."""
+    dbin_z = (cfg.z_max - 0.0) / cfg.nbin_z
+    sea = int(cfg.sdep / dbin_z) + 1 if cfg.sdep > 0.0 else 1     # the first bin below the sea layer
+    bins = []
+    for z in depths:
+        if not 0.0 <= z <= cfg.z_max:
+            raise ValueError(f"diagnostic depth {z} km is outside [0, Z_MAX = {cfg.z_max}] km")
+        b = min(int(z / dbin_z) + 1, cfg.nbin_z)   # (z_max itself, or a depth rounded past the last bin's bottom)
+        if b < sea:
+            raise ValueError(f"diagnostic depth {z} km lies inside the sea layer (SEA_DEP = {cfg.sdep} km)")
+        bins.append(b)
+    if len(bins) > 16:
+        raise ValueError(f"{len(bins)} diagnostic depths: at most 16")
+    return bins
+
+
+def convergence_rows(diag, depths):
+    """[(name, samples, ranks, R-hat, ESS, median tau, tempered share)] with the Vs quantities named by their depths."""
+    names = diag["names"]
+    nv = len(depths)
+    if nv:
+        names = names[:-nv] + [f"vs_{z:g}" for z in depths]
+    return [(n, diag["n_samples"], diag["n_ranks"], diag["rhat"][q], diag["ess_total"][q], diag["tau_median"][q],
+             diag["tempered_share"][q]) for q, n in enumerate(names)]
+
+
+def write_convergence(out_dir: str, rows) -> None:
+    """OUT_DIR/convergence: one line per quantity."""
+    with open(os.path.join(out_dir, "convergence"), "w") as f:
+        for n, ns, nr, rhat, ess, tau, share in rows:
+            f.write(f"{n:12s} {ns:8d} {nr:6d} {rhat:.17g} {ess:.17g} {tau:.17g} {share:.17g}\n")
+
+
+def write_round_trips(out_dir: str, trips) -> None:
+    """OUT_DIR/round_trips: one line per virtual rank: rank, round trips during the burn-in, after it."""
+    with open(os.path.join(out_dir, "round_trips"), "w") as f:
+        for r, (a, b) in enumerate(trips):
+            f.write(f"{r:6d} {int(a):8d} {int(b):8d}\n")
+
+
+def print_convergence(rows) -> None:
+    print(" --- Convergence of the cold level (R-hat, ESS, median IAT, tempered share) ---")
+    for n, ns, nr, rhat, ess, tau, share in rows:
+        print(f" {n}: R-hat {rhat:.4f}, ESS {ess:.1f} of {ns * nr} samples over {nr} ranks, median IAT {tau:.2f}, "
+              f"tempered {share:.4f}")
+
+
 def print_rank_swaps(rs) -> None:
     print(" --- Swaps between neighbouring temperature levels inside the ranks ---")
     for l, (a, n) in enumerate(zip(rs["n_acc"], rs["n_prop"]), start=1):
@@ -106,19 +161,22 @@ def print_rank_swaps(rs) -> None:
 
 def run(params_path: str, nproc: int, verbose: bool = True, n_iter: int = None, checkpoint: str = None,
         checkpoint_every: int = None, resume: bool = False, rank_swaps: bool = False, tune_ladder: bool = False,
-        tune_steps: bool = False, step_target: float = 0.44):
+        tune_steps: bool = False, step_target: float = 0.44, diagnostics: bool = False, diag_depths=()):
     """checkpoint: save the state to this path every `checkpoint_every` iterations (rounded up to the progress steps; default:
     every progress step) and at the end.  resume: restore it first if it exists and continue from its iteration count.
     rank_swaps: the even/odd sweep inside every virtual rank (ParallelTempering.set_rank_swaps(1)); adds OUT_DIR/rank_swaps.
     tune_ladder: implies rank_swaps, plus the ladder tuning during the burn-in (set_ladder_tuning(1)); adds OUT_DIR/ladder.
     tune_steps: implies rank_swaps, plus the width tuning during the burn-in towards the acceptance rate step_target
-    (set_step_tuning(1, step_target)); adds OUT_DIR/step_widths."""
+    (set_step_tuning(1, step_target)); adds OUT_DIR/step_widths.
+    diagnostics: record the cold level and report convergence (set_diagnostics) at the depths diag_depths (km); adds
+    OUT_DIR/convergence and, with rank_swaps, OUT_DIR/round_trips."""
     rank_swaps = rank_swaps or tune_ladder or tune_steps
     if resume and not checkpoint:
         raise ValueError("resume needs a checkpoint path")
     if checkpoint_every is not None and checkpoint_every < 1:
         raise ValueError("checkpoint_every must be at least 1")
     cfg = rio.load_problem(params_path)
+    bins = depth_bins(cfg, diag_depths) if diagnostics else []
     cfg.r_inv = workloads.lapack_r_inv(cfg)          # init_r_inv: LAPACK dgesvd like the reference
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
@@ -141,6 +199,8 @@ def run(params_path: str, nproc: int, verbose: bool = True, n_iter: int = None, 
         pt.set_ladder_tuning(1)
     if tune_steps:
         pt.set_step_tuning(1, step_target)
+    if diagnostics:
+        pt.set_diagnostics(1, bins)
     n_tot = cfg.nburn + cfg.niter if n_iter is None else n_iter
     ck = checkpoint_path(checkpoint, world, rank) if checkpoint else None
     if resume:
@@ -187,6 +247,7 @@ def run(params_path: str, nproc: int, verbose: bool = True, n_iter: int = None, 
     hist, cnt = pt.hist(), pt.counters()
     vp_model, vs_model = pt.models()
     rs = pt.rank_swaps() if rank_swaps else None
+    diag = pt.diagnostics() if diagnostics else None      # (job-wide on process 0 after reduce_outputs)
     lh = cnt["likelihood_hist"]
     if rank == 0:
         if verbose:
@@ -200,6 +261,13 @@ def run(params_path: str, nproc: int, verbose: bool = True, n_iter: int = None, 
             write_ladder(cfg.out_dir, ladders)
         if widths is not None:
             write_step_widths(cfg.out_dir, widths)
+        if diag is not None:
+            conv = convergence_rows(diag, diag_depths)
+            if verbose:
+                print_convergence(conv)
+            write_convergence(cfg.out_dir, conv)
+            if rank_swaps:
+                write_round_trips(cfg.out_dir, diag["trips"])
     pt.close()
     if world > 1:
         dist.destroy_process_group()
@@ -232,7 +300,7 @@ def load_stations(params_paths):
 
 def run_group(params_paths, nproc: int, verbose: bool = True, n_iter: int = None, checkpoint: str = None,
               checkpoint_every: int = None, resume: bool = False, rank_swaps: bool = False, tune_ladder: bool = False,
-              tune_steps: bool = False, step_target: float = 0.44):
+              tune_steps: bool = False, step_target: float = 0.44, diagnostics: bool = False, diag_depths=()):
     """Several stations (one params file each) as one group on one GPU; arguments as in run().  Under torchrun process r
     takes the stations i with i % world == r.  Returns {station index: (hist, counters)} of this process's stations."""
     rank_swaps = rank_swaps or tune_ladder or tune_steps
@@ -242,6 +310,7 @@ def run_group(params_paths, nproc: int, verbose: bool = True, n_iter: int = None
         raise ValueError("checkpoint_every must be at least 1")
     params_paths = list(params_paths)
     cfgs = load_stations(params_paths)
+    bins = [depth_bins(c, diag_depths) if diagnostics else [] for c in cfgs]
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -268,6 +337,9 @@ def run_group(params_paths, nproc: int, verbose: bool = True, n_iter: int = None
                     pt.set_ladder_tuning(1)
                 if tune_steps:
                     pt.set_step_tuning(1, step_target)
+        if diagnostics:
+            for i, pt in zip(mine, pts):
+                pt.set_diagnostics(1, bins[i])
         if restore:
             for i, pt in zip(mine, pts):
                 pt.restore(cks[i])
@@ -309,6 +381,14 @@ def run_group(params_paths, nproc: int, verbose: bool = True, n_iter: int = None
                 write_ladder(cfg.out_dir, rank_ladders(pt))
             if tune_steps:
                 write_step_widths(cfg.out_dir, step_rows(pt))
+            if diagnostics:
+                diag = pt.diagnostics()
+                conv = convergence_rows(diag, diag_depths)
+                if verbose:
+                    print_convergence(conv)
+                write_convergence(cfg.out_dir, conv)
+                if rank_swaps:
+                    write_round_trips(cfg.out_dir, diag["trips"])
             out[i] = (hist, cnt)
         return out
     finally:
@@ -340,18 +420,30 @@ def main(argv=None):
                          "towards the acceptance rate --step-target (writes OUT_DIR/step_widths)")
     ap.add_argument("--step-target", type=float, default=0.44,
                     help="acceptance rate --tune-steps aims at, in (0, 1) (default 0.44)")
+    ap.add_argument("--diagnostics", action="store_true",
+                    help="record the coldest level of every virtual rank and report convergence: R-hat, ESS, median IAT, "
+                         "tempered share (writes OUT_DIR/convergence; with --rank-swaps also OUT_DIR/round_trips)")
+    ap.add_argument("--diag-depths", default="", metavar="KM,KM,...",
+                    help="with --diagnostics: also follow Vs at these depths in km (at most 16, below the sea layer)")
     a = ap.parse_args(argv)
     if a.resume and not a.checkpoint:
         ap.error("--resume needs --checkpoint")
     if not 0.0 < a.step_target < 1.0:
         ap.error("--step-target must lie in (0, 1)")
+    try:
+        depths = [float(x) for x in a.diag_depths.split(",") if x.strip()]
+    except ValueError:
+        ap.error("--diag-depths takes depths in km separated by commas")
+    if depths and not a.diagnostics:
+        ap.error("--diag-depths needs --diagnostics")
     if len(a.params) == 1:
         run(a.params[0], a.nproc, n_iter=a.iters, checkpoint=a.checkpoint, checkpoint_every=a.checkpoint_every, resume=a.resume,
-            rank_swaps=a.rank_swaps, tune_ladder=a.tune_ladder, tune_steps=a.tune_steps, step_target=a.step_target)
+            rank_swaps=a.rank_swaps, tune_ladder=a.tune_ladder, tune_steps=a.tune_steps, step_target=a.step_target,
+            diagnostics=a.diagnostics, diag_depths=depths)
     else:
         run_group(a.params, a.nproc, n_iter=a.iters, checkpoint=a.checkpoint, checkpoint_every=a.checkpoint_every,
                   resume=a.resume, rank_swaps=a.rank_swaps, tune_ladder=a.tune_ladder, tune_steps=a.tune_steps,
-                  step_target=a.step_target)
+                  step_target=a.step_target, diagnostics=a.diagnostics, diag_depths=depths)
 
 
 if __name__ == "__main__":

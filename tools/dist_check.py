@@ -9,6 +9,9 @@ job-wide counters.  --tune-ladder adds the ladder tuning during the burn-in (set
 burn-ins and run lengths that pass two or three tuning points, and also compares the number of tuning points passed.
 --tune-steps adds the width tuning during the burn-in (set_step_tuning(1), implies --rank-swaps) with the same run lengths, and
 also compares each process's widths and width counters with its rows of the single-process run.
+--diagnostics runs both sides with the convergence diagnostics on (set_diagnostics, in mode 1 with --rank-swaps) and also
+compares each process's cold-level trace with its ranks of the single-process trace and, on process 0 after reduce_outputs,
+the job-wide per-rank rows, summary and round trips with those of the single process, bit for bit.
 """
 import faulthandler, hashlib, json, os, signal, sys
 faulthandler.register(signal.SIGTERM, all_threads=True, chain=False)
@@ -22,8 +25,13 @@ from rf_inv_b200.evaluator import Evaluator
 from rf_inv_b200.pt import ParallelTempering
 
 
+DIAG_BINS = [5, 20, 40]
+DIAG_KEYS = ("mean", "var", "tau", "ess", "mean_1", "var_1", "mean_2", "var_2", "tempered", "rhat", "ess_total", "tau_median",
+             "tempered_share", "trips")
+
+
 def identity_check(cfg, nproc_total, n_iter, world, rank, local_rank, dist, torch, rank_swaps=0, tune_ladder=False,
-                   tune_steps=False):
+                   tune_steps=False, diagnostics=False):
     """Returns (ok, detail) on every process."""
     dev = torch.device("cuda", local_rank)
     # distributed run
@@ -37,6 +45,8 @@ def identity_check(cfg, nproc_total, n_iter, world, rank, local_rank, dist, torc
         pt.set_ladder_tuning(1)
     if tune_steps:
         pt.set_step_tuning(1)
+    if diagnostics:
+        pt.set_diagnostics(1, DIAG_BINS)
     pt.init_comm(dist, torch)
     say("communicator up")
     pt.run_distributed(n_iter, dist, torch)
@@ -46,8 +56,10 @@ def identity_check(cfg, nproc_total, n_iter, world, rank, local_rank, dist, torc
     st = pt.state()
     tuning = pt.ladder_tuning()
     steps = pt.step_tuning() if tune_steps else None
+    trace = pt.cold_trace() if diagnostics else None
     pt.reduce_outputs()
     say("outputs reduced")
+    diag = pt.diagnostics() if diagnostics and rank == 0 else None
     cnt = pt.counters()
     hist = pt.hist() if cfg.niter > 0 else None
     rsw = pt.rank_swaps() if rank_swaps else None
@@ -64,7 +76,11 @@ def identity_check(cfg, nproc_total, n_iter, world, rank, local_rank, dist, torc
             ref.set_ladder_tuning(1)
         if tune_steps:
             ref.set_step_tuning(1)
+        if diagnostics:
+            ref.set_diagnostics(1, DIAG_BINS)
         ref.run(n_iter)
+        rtrace = ref.cold_trace() if diagnostics else None
+        rdiag = ref.diagnostics() if diagnostics else None
         rsteps = ref.step_tuning() if tune_steps else None
         rtuning = ref.ladder_tuning()
         rf, ri, rs = ref.log(n_iter)
@@ -74,7 +90,7 @@ def identity_check(cfg, nproc_total, n_iter, world, rank, local_rank, dist, torc
         rrsw = ref.rank_swaps() if rank_swaps else None
         ref.close()
         say("reference run done")
-        box = [dict(flags=rf, itypes=ri, swaps=rs, state=rst, tuning=rtuning, steps=rsteps)]
+        box = [dict(flags=rf, itypes=ri, swaps=rs, state=rst, tuning=rtuning, steps=rsteps, trace=rtrace)]
     else:
         box = [None]
     dist.broadcast_object_list(box, src=0)
@@ -93,7 +109,15 @@ def identity_check(cfg, nproc_total, n_iter, world, rank, local_rank, dist, torc
         parts["step_tuning"] = (steps["on"] and steps["n_points"] == r["steps"]["n_points"] >= 2
                                 and not np.all(r["steps"]["widths"] == r["steps"]["widths"][0, 0])
                                 and all(np.array_equal(steps[k], r["steps"][k][rsl]) for k in ("widths", "n_prop", "n_acc")))
+    if diagnostics:
+        rsl = slice(pt.rank_begin, pt.rank_begin + pt.rank_count)
+        parts["cold_trace"] = (trace["trace"].shape[0] > 0 and np.array_equal(trace["trace"], r["trace"]["trace"][:, rsl])
+                               and np.array_equal(trace["t0"], r["trace"]["t0"][:, rsl]))
     detail = {}
+    if rank == 0 and diagnostics:
+        parts["diagnostics"] = (diag["n_ranks"] == rdiag["n_ranks"] == nproc_total and diag["n_samples"] == rdiag["n_samples"]
+                                and all(np.asarray(diag[k]).tobytes() == np.asarray(rdiag[k]).tobytes() for k in DIAG_KEYS))
+        parts["round_trips"] = not rank_swaps or int(rdiag["trips"].sum()) > 0
     if rank == 0:
         parts["nprop"] = np.array_equal(cnt["nprop"], rcnt["nprop"]); parts["naccept"] = np.array_equal(cnt["naccept"], rcnt["naccept"])
         # likelihood_hist is a sum over processes of per-process tree sums: equal up to the order of additions
@@ -126,11 +150,15 @@ if __name__ == "__main__":
     tune_ladder = "--tune-ladder" in sys.argv[1:]
     tune_steps = "--tune-steps" in sys.argv[1:]
     rank_swaps = 1 if "--rank-swaps" in sys.argv[1:] or tune_ladder or tune_steps else 0
+    diagnostics = "--diagnostics" in sys.argv[1:]
     out = {}
     runs = (("sample", 4 * world, 300, dict(nburn=100, niter=200)), ("c4", 8 * world, 120, dict()), ("target", 16 * world, 60, dict()))
     if tune_ladder or tune_steps:   # tuning points 64, 128, 256 / 64, 128, inside and at the end of the burn-in
         runs = (("sample", 4 * world, 300, dict(nburn=280, niter=20)), ("c4", 8 * world, 140, dict(nburn=128)),
                 ("target", 16 * world, 130, dict(nburn=200)))
+    if diagnostics:   # every run records (the diagnostics need the bookkeeping), several samples per rank
+        runs = (("sample", 4 * world, 300, dict(nburn=100, niter=200, ncorr=2)), ("c4", 8 * world, 120, dict(nburn=40, niter=80, ncorr=2)),
+                ("target", 16 * world, 60, dict(nburn=20, niter=40, ncorr=2)))
     for name, nproc, iters, kw in runs:
         cfg = workloads.make_config(name)
         for k_, v_ in kw.items():
@@ -144,7 +172,7 @@ if __name__ == "__main__":
             _, rft, _ = ev.calc_likelihood(tm["k"], tm["z"], tm["dvp"], tm["dvs"], tm["sig"], want_rft=True)
         cfg.obs = (rft[0, :, :cfg.nsmp] + np.random.default_rng(7).normal(0.0, 0.01, (cfg.ntrc, cfg.nsmp))).astype(np.float32).astype(np.float64)
         ok, detail = identity_check(cfg, nproc, iters, world, rank, local_rank, dist, torch, rank_swaps, tune_ladder,
-                                    tune_steps)
+                                    tune_steps, diagnostics)
         out[name] = dict(identical=ok, world=world, virtual_ranks=nproc, iterations=iters, **detail)
     if rank == 0:
         print(json.dumps(out), flush=True)
