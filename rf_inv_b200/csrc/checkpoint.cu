@@ -176,6 +176,38 @@ constexpr const char* ST_SECTION = "step_tuning";
 constexpr const char* DG_SECTION = "diagnostics";
 constexpr int DG_WORDS = 1 + 16 + 1;
 
+// The sections of the opt-in settings above, in file order after those of parts().  Each is in a file exactly when the
+// handle that wrote it had the setting on.
+struct Setting {
+  const char* name;        // the section; the setting's setter is rfinv_pt_set_<name>
+  uint32_t elem;
+  uint64_t count;
+  bool on;                 // this handle has the setting on: save writes the section, restore needs it
+  const char* what;        // for restore's message: "... written with <what> <state>, this handle has <them> <state>"
+  const char* them;
+  const char* state[2];    // off, on
+};
+enum { SET_RS, SET_LT, SET_ST, SET_DG, SET_COUNT };
+
+std::vector<Setting> settings(const rfinv_handle* h) {
+  const PtState* s = h->pt;
+  const PtDev& d = s->dev;
+  const uint64_t nl = d.nchains > 1 ? d.nchains - 1 : 0;
+  return {{RS_SECTION, sizeof(int64_t), 1 + 2 * nl, s->rank_swaps == 1, "the rank swaps", "them", {"off (mode 0)", "on (mode 1)"}},
+          {LT_SECTION, sizeof(int64_t), 1 + d.G * nl, d.rs_tune != 0, "the ladder tuning", "it", {"off", "on"}},
+          {ST_SECTION, sizeof(double), 1, d.st_on != 0, "the step tuning", "it", {"off", "on"}},
+          {DG_SECTION, sizeof(int64_t), DG_WORDS, d.dg_on != 0, "the diagnostics", "them", {"off", "on"}}};
+}
+
+// writes a section header at buf + off and advances off past it
+void put_section(uint8_t* buf, size_t& off, const char* name, uint32_t elem, uint64_t count) {
+  CkSection sc;
+  std::memset(&sc, 0, sizeof(sc));
+  std::snprintf(sc.name, sizeof(sc.name), "%s", name);
+  sc.elem_size = elem; sc.count = count;
+  std::memcpy(buf + off, &sc, sizeof(sc)); off += sizeof(sc);
+}
+
 int io_error(const char* who, const std::string& path, const char* what) {
   rfinv_set_error("%s: %s: %s", who, path.c_str(), what);
   return RFINV_ERR_IO;
@@ -190,14 +222,8 @@ int32_t rfinv_pt_save(rfinv_handle* h, const char* path) {
   if (!h || !path || !*path) { rfinv_set_error("%s: handle or path is NULL", who); return RFINV_ERR_ARG; }
   if (!h->pt) { rfinv_set_error("%s: call rfinv_pt_init first", who); return RFINV_ERR_STATE; }
   PtState* s = h->pt;
-  if (s->step_pending) {
-    rfinv_set_error("%s: an iteration is half done (rfinv_pt_local_step without rfinv_pt_apply_swap)", who);
-    return RFINV_ERR_STATE;
-  }
-  if (s->reduced) {
-    rfinv_set_error("%s: rfinv_pt_reduce_outputs has run: process 0 holds job-wide sums, not this process's state", who);
-    return RFINV_ERR_STATE;
-  }
+  int st;
+  if ((st = pt_require_settled(s, who)) != RFINV_OK) return st;
   RFINV_CUDA_CHECK(cudaSetDevice(h->device));
   RFINV_CUDA_CHECK(cudaStreamSynchronize(h->stream));
   PtDev& d = s->dev;
@@ -216,20 +242,20 @@ int32_t rfinv_pt_save(rfinv_handle* h, const char* path) {
   hd.ntrc = h->cfg.ntrc; hd.nsmp = h->cfg.nsmp; hd.k_max = h->cfg.k_max; hd.niter = h->cfg.niter;
   hd.it_done = s->it_done; hd.record = s->record ? 1 : 0; hd.n_eval_host = s->n_eval; hd.cap_models = d.vp_model ? d.cap_models : 0;
   fingerprints(h, hd.fp);
-  std::vector<int64_t> rs;
-  if (s->rank_swaps == 1) {
-    const int nl = d.nchains > 1 ? d.nchains - 1 : 0;
-    rs.assign(1 + 2 * (size_t)nl, 0);
+  // the payloads of the settings' sections that are on, in the order of settings()
+  const std::vector<Setting> ss = settings(h);
+  std::vector<int64_t> rs, lt, dg;
+  if (ss[SET_RS].on) {
+    rs.assign(ss[SET_RS].count, 0);
+    const size_t nl = (rs.size() - 1) / 2;
     int32_t mode = 0;
-    int st;
     if ((st = rfinv_pt_get_rank_swaps(h, &mode, rs.data() + 1, rs.data() + 1 + nl)) != RFINV_OK) return st;
     rs[0] = mode;
   }
-  std::vector<int64_t> lt;
-  if (d.rs_tune) {
-    const size_t nr = d.nchains > 1 ? (size_t)d.G * (d.nchains - 1) : 0;
-    lt.assign(1 + nr, 0);
+  if (ss[SET_LT].on) {
+    lt.assign(ss[SET_LT].count, 0);
     lt[0] = 1;
+    const size_t nr = lt.size() - 1;
     if (nr) {
       std::vector<unsigned long long> acc(nr), base(nr);
       RFINV_CUDA_CHECK(cudaMemcpy(acc.data(), d.rs_nacc, sizeof(unsigned long long) * nr, cudaMemcpyDeviceToHost));
@@ -237,8 +263,7 @@ int32_t rfinv_pt_save(rfinv_handle* h, const char* path) {
       for (size_t i = 0; i < nr; ++i) lt[1 + i] = (int64_t)(acc[i] - base[i]);
     }
   }
-  std::vector<int64_t> dg;
-  if (d.dg_on) {
+  if (ss[SET_DG].on) {
     dg.assign(DG_WORDS, 0);
     dg[0] = d.dg_nbins;
     std::vector<int32_t> bins(16, 0);
@@ -246,58 +271,27 @@ int32_t rfinv_pt_save(rfinv_handle* h, const char* path) {
     for (int j = 0; j < 16; ++j) dg[1 + j] = bins[j];
     dg[17] = d.dg_cap;
   }
-  hd.n_sections = (uint32_t)(ps.size() + (rs.empty() ? 0 : 1) + (lt.empty() ? 0 : 1) + (d.st_on ? 1 : 0) + (dg.empty() ? 0 : 1));
+  const void* const payload[SET_COUNT] = {rs.data(), lt.data(), &d.st_target, dg.data()};
+  hd.n_sections = (uint32_t)ps.size();
   size_t total = sizeof(CkHeader) + sizeof(uint64_t);
   for (const Part& p : ps) total += sizeof(CkSection) + (size_t)p.elem * p.count;
-  if (!rs.empty()) total += sizeof(CkSection) + sizeof(int64_t) * rs.size();
-  if (!lt.empty()) total += sizeof(CkSection) + sizeof(int64_t) * lt.size();
-  if (d.st_on) total += sizeof(CkSection) + sizeof(double);
-  if (!dg.empty()) total += sizeof(CkSection) + sizeof(int64_t) * dg.size();
+  for (const Setting& x : ss)
+    if (x.on) { ++hd.n_sections; total += sizeof(CkSection) + (size_t)x.elem * x.count; }
   std::unique_ptr<uint8_t[]> buf(new (std::nothrow) uint8_t[total]);
   if (!buf) { rfinv_set_error("%s: cannot allocate %zu bytes of host memory", who, total); return RFINV_ERR_IO; }
   size_t off = 0;
   std::memcpy(buf.get(), &hd, sizeof(hd)); off += sizeof(hd);
   for (const Part& p : ps) {
-    CkSection sc;
-    std::memset(&sc, 0, sizeof(sc));
-    std::snprintf(sc.name, sizeof(sc.name), "%s", p.name);
-    sc.elem_size = p.elem; sc.count = p.count;
-    std::memcpy(buf.get() + off, &sc, sizeof(sc)); off += sizeof(sc);
+    put_section(buf.get(), off, p.name, p.elem, p.count);
     const size_t n = (size_t)p.elem * p.count;
     if (n) RFINV_CUDA_CHECK(cudaMemcpy(buf.get() + off, p.dev, n, cudaMemcpyDeviceToHost));
     off += n;
   }
-  if (!rs.empty()) {
-    CkSection sc;
-    std::memset(&sc, 0, sizeof(sc));
-    std::snprintf(sc.name, sizeof(sc.name), "%s", RS_SECTION);
-    sc.elem_size = sizeof(int64_t); sc.count = rs.size();
-    std::memcpy(buf.get() + off, &sc, sizeof(sc)); off += sizeof(sc);
-    std::memcpy(buf.get() + off, rs.data(), sizeof(int64_t) * rs.size()); off += sizeof(int64_t) * rs.size();
-  }
-  if (!lt.empty()) {
-    CkSection sc;
-    std::memset(&sc, 0, sizeof(sc));
-    std::snprintf(sc.name, sizeof(sc.name), "%s", LT_SECTION);
-    sc.elem_size = sizeof(int64_t); sc.count = lt.size();
-    std::memcpy(buf.get() + off, &sc, sizeof(sc)); off += sizeof(sc);
-    std::memcpy(buf.get() + off, lt.data(), sizeof(int64_t) * lt.size()); off += sizeof(int64_t) * lt.size();
-  }
-  if (d.st_on) {
-    CkSection sc;
-    std::memset(&sc, 0, sizeof(sc));
-    std::snprintf(sc.name, sizeof(sc.name), "%s", ST_SECTION);
-    sc.elem_size = sizeof(double); sc.count = 1;
-    std::memcpy(buf.get() + off, &sc, sizeof(sc)); off += sizeof(sc);
-    std::memcpy(buf.get() + off, &d.st_target, sizeof(double)); off += sizeof(double);
-  }
-  if (!dg.empty()) {
-    CkSection sc;
-    std::memset(&sc, 0, sizeof(sc));
-    std::snprintf(sc.name, sizeof(sc.name), "%s", DG_SECTION);
-    sc.elem_size = sizeof(int64_t); sc.count = dg.size();
-    std::memcpy(buf.get() + off, &sc, sizeof(sc)); off += sizeof(sc);
-    std::memcpy(buf.get() + off, dg.data(), sizeof(int64_t) * dg.size()); off += sizeof(int64_t) * dg.size();
+  for (int i = 0; i < SET_COUNT; ++i) {
+    if (!ss[i].on) continue;
+    put_section(buf.get(), off, ss[i].name, ss[i].elem, ss[i].count);
+    const size_t n = (size_t)ss[i].elem * ss[i].count;
+    std::memcpy(buf.get() + off, payload[i], n); off += n;
   }
   const uint64_t sum = xxh64(buf.get(), off);
   std::memcpy(buf.get() + off, &sum, sizeof(sum));
@@ -428,54 +422,30 @@ int32_t rfinv_pt_restore(rfinv_handle* h, const char* path) {
       return RFINV_ERR_ARG;
     }
   }
-  // the rank sweep: the mode is part of the run (set it with rfinv_pt_set_rank_swaps before restoring)
-  const auto rs_it = found.find(RS_SECTION);
+  // the settings are part of the run: each is on in the file exactly when it is on here (set with its setter before restoring)
+  for (const Setting& x : settings(h)) {
+    const auto it = found.find(x.name);
+    const bool in_file = it != found.end();
+    if (in_file != x.on) {
+      rfinv_set_error("%s: %s was written with %s %s, this handle has %s %s (rfinv_pt_set_%s before restore)", who, path, x.what,
+                      x.state[in_file], x.them, x.state[x.on], x.name);
+      return RFINV_ERR_ARG;
+    }
+    if (in_file && (it->second.second.elem_size != x.elem || it->second.second.count != x.count))
+      return io_error(who, file, ("section '" + std::string(x.name) + "' is malformed").c_str());
+  }
   const int nl = d.nchains > 1 ? d.nchains - 1 : 0;
-  if ((rs_it != found.end()) != (s->rank_swaps == 1)) {
-    rfinv_set_error("%s: %s was written with the rank swaps %s, this handle has them %s (rfinv_pt_set_rank_swaps before restore)", who,
-                    path, rs_it != found.end() ? "on (mode 1)" : "off (mode 0)", s->rank_swaps == 1 ? "on (mode 1)" : "off (mode 0)");
-    return RFINV_ERR_ARG;
-  }
-  if (rs_it != found.end() && (rs_it->second.second.elem_size != sizeof(int64_t) || rs_it->second.second.count != 1 + 2 * (uint64_t)nl))
-    return io_error(who, file, "section 'rank_swaps' is malformed");
-  // the ladder tuning likewise (rfinv_pt_set_ladder_tuning before restoring)
-  const auto lt_it = found.find(LT_SECTION);
-  if ((lt_it != found.end()) != (d.rs_tune != 0)) {
-    rfinv_set_error("%s: %s was written with the ladder tuning %s, this handle has it %s (rfinv_pt_set_ladder_tuning before restore)",
-                    who, path, lt_it != found.end() ? "on" : "off", d.rs_tune ? "on" : "off");
-    return RFINV_ERR_ARG;
-  }
-  if (lt_it != found.end() && (lt_it->second.second.elem_size != sizeof(int64_t) || lt_it->second.second.count != 1 + (uint64_t)d.G * nl))
-    return io_error(who, file, "section 'ladder_tuning' is malformed");
-  // the step tuning likewise, and with the same target (rfinv_pt_set_step_tuning before restoring)
-  const auto st_it = found.find(ST_SECTION);
-  if ((st_it != found.end()) != (d.st_on != 0)) {
-    rfinv_set_error("%s: %s was written with the step tuning %s, this handle has it %s (rfinv_pt_set_step_tuning before restore)",
-                    who, path, st_it != found.end() ? "on" : "off", d.st_on ? "on" : "off");
-    return RFINV_ERR_ARG;
-  }
-  if (st_it != found.end()) {
-    if (st_it->second.second.elem_size != sizeof(double) || st_it->second.second.count != 1)
-      return io_error(who, file, "section 'step_tuning' is malformed");
+  if (d.st_on) {   // with the same target
     double target;
-    std::memcpy(&target, buf.data() + st_it->second.first, sizeof(double));
+    std::memcpy(&target, buf.data() + found[ST_SECTION].first, sizeof(double));
     if (target != d.st_target) {
       rfinv_set_error("%s: %s was written with the step tuning's target %.17g, this handle has %.17g", who, path, target, d.st_target);
       return RFINV_ERR_ARG;
     }
   }
-  // the diagnostics likewise, with the same depth bins (rfinv_pt_set_diagnostics before restoring)
-  const auto dg_it = found.find(DG_SECTION);
-  if ((dg_it != found.end()) != (d.dg_on != 0)) {
-    rfinv_set_error("%s: %s was written with the diagnostics %s, this handle has them %s (rfinv_pt_set_diagnostics before restore)",
-                    who, path, dg_it != found.end() ? "on" : "off", d.dg_on ? "on" : "off");
-    return RFINV_ERR_ARG;
-  }
-  if (dg_it != found.end()) {
-    if (dg_it->second.second.elem_size != sizeof(int64_t) || dg_it->second.second.count != DG_WORDS)
-      return io_error(who, file, "section 'diagnostics' is malformed");
+  if (d.dg_on) {   // with the same depth bins
     int64_t dg[DG_WORDS];
-    std::memcpy(dg, buf.data() + dg_it->second.first, sizeof(dg));
+    std::memcpy(dg, buf.data() + found[DG_SECTION].first, sizeof(dg));
     std::vector<int32_t> bins(16, 0);
     if (d.dg_nbins) RFINV_CUDA_CHECK(cudaMemcpy(bins.data(), d.dg_bins, sizeof(int32_t) * d.dg_nbins, cudaMemcpyDeviceToHost));
     bool same = dg[0] == d.dg_nbins;
@@ -514,16 +484,16 @@ int32_t rfinv_pt_restore(rfinv_handle* h, const char* path) {
     const size_t n = (size_t)p.elem * p.count;
     if (n) RFINV_CUDA_CHECK(cudaMemcpy(p.dev, buf.data() + found[p.name].first, n, cudaMemcpyHostToDevice));
   }
-  if (rs_it != found.end() && nl > 0) {   // the per-level sums go into the row of local rank 0, the other rows start at zero
+  if (s->rank_swaps == 1 && nl > 0) {   // the per-level sums go into the row of local rank 0, the other rows start at zero
     std::vector<int64_t> rs(1 + 2 * (size_t)nl);
-    std::memcpy(rs.data(), buf.data() + rs_it->second.first, sizeof(int64_t) * rs.size());
+    std::memcpy(rs.data(), buf.data() + found[RS_SECTION].first, sizeof(int64_t) * rs.size());
     std::vector<int64_t> rows((size_t)d.G * nl, 0);
     std::memcpy(rows.data(), rs.data() + 1 + nl, sizeof(int64_t) * nl);
     RFINV_CUDA_CHECK(cudaMemcpy(d.rs_nprop, rs.data() + 1, sizeof(int64_t) * nl, cudaMemcpyHostToDevice));
     RFINV_CUDA_CHECK(cudaMemcpy(d.rs_nacc, rows.data(), sizeof(int64_t) * rows.size(), cudaMemcpyHostToDevice));
-    if (lt_it != found.end()) {   // snapshot = restored row - acceptances of the round (modulo 2^64)
+    if (d.rs_tune) {   // snapshot = restored row - acceptances of the round (modulo 2^64)
       std::vector<int64_t> round((size_t)d.G * nl);
-      std::memcpy(round.data(), buf.data() + lt_it->second.first + sizeof(int64_t), sizeof(int64_t) * round.size());
+      std::memcpy(round.data(), buf.data() + found[LT_SECTION].first + sizeof(int64_t), sizeof(int64_t) * round.size());
       std::vector<unsigned long long> base(round.size());
       for (size_t i = 0; i < base.size(); ++i) base[i] = (unsigned long long)rows[i] - (unsigned long long)round[i];
       RFINV_CUDA_CHECK(cudaMemcpy(d.rs_base, base.data(), sizeof(unsigned long long) * base.size(), cudaMemcpyHostToDevice));

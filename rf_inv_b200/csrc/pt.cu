@@ -1428,6 +1428,45 @@ static int pt_require(rfinv_handle* h, const char* who) {
   return RFINV_OK;
 }
 
+int pt_require_settled(const PtState* s, const char* who) {
+  if (s->step_pending) {
+    rfinv_set_error("%s: an iteration is half done (rfinv_pt_local_step without rfinv_pt_apply_swap)", who);
+    return RFINV_ERR_STATE;
+  }
+  if (s->reduced) {
+    rfinv_set_error("%s: rfinv_pt_reduce_outputs has run: process 0 holds job-wide sums, not this process's state", who);
+    return RFINV_ERR_STATE;
+  }
+  return RFINV_OK;
+}
+
+// a setting that is part of the run from its start: `what` is "the tuning starts" or the like
+static int pt_require_fresh(const PtState* s, const char* who, const char* what) {
+  if (s->it_done == 0) return RFINV_OK;
+  rfinv_set_error("%s: %d iterations have run; %s with the run (before its first iteration or a restore)", who, s->it_done, what);
+  return RFINV_ERR_STATE;
+}
+
+// the tunings work on the rank sweep's counters and levels
+static int pt_require_rank_swaps(const PtState* s, const char* who) {
+  if (s->rank_swaps == 1) return RFINV_OK;
+  rfinv_set_error("%s: the tuning needs the rank swaps on (rfinv_pt_set_rank_swaps(h, 1) first)", who);
+  return RFINV_ERR_STATE;
+}
+
+// switching a tuning off freezes the count of tuning points it passed (rfinv_pt_get_ladder_tuning, _get_step_tuning)
+static void pt_ladder_tuning_off(PtState* s) {
+  if (!s->dev.rs_tune) return;
+  s->tune_points_off = pt_tuning_points(s->it_done, s->dev.nburn);
+  s->dev.rs_tune = 0;
+}
+
+static void pt_step_tuning_off(PtState* s) {
+  if (!s->dev.st_on) return;
+  s->step_points_off = pt_tuning_points(s->it_done, s->dev.nburn);
+  s->dev.st_on = 0;
+}
+
 // forward + quadratic form for the chains in `active` (or all), proposal or current state
 static int pt_eval(rfinv_handle* h, bool proposal, bool all) {
   PtState* s = h->pt;
@@ -1578,16 +1617,13 @@ int32_t rfinv_pt_set_logging(rfinv_handle* h, int32_t cap_iters) {
 }
 
 int32_t rfinv_pt_set_rank_swaps(rfinv_handle* h, int32_t mode) {
-  int st = pt_require(h, "rfinv_pt_set_rank_swaps");
+  static const char* who = "rfinv_pt_set_rank_swaps";
+  int st = pt_require(h, who);
   if (st != RFINV_OK) return st;
   PtState* s = h->pt;
   PtDev& d = s->dev;
-  if (mode != 0 && mode != 1) { rfinv_set_error("rfinv_pt_set_rank_swaps: mode %d (0: off, 1: even/odd swaps inside every rank)", mode); return RFINV_ERR_ARG; }
-  if (s->step_pending) {
-    rfinv_set_error("rfinv_pt_set_rank_swaps: an iteration is half done (rfinv_pt_local_step without rfinv_pt_apply_swap)");
-    return RFINV_ERR_STATE;
-  }
-  if (s->reduced) { rfinv_set_error("rfinv_pt_set_rank_swaps: rfinv_pt_reduce_outputs has run"); return RFINV_ERR_STATE; }
+  if (mode != 0 && mode != 1) { rfinv_set_error("%s: mode %d (0: off, 1: even/odd swaps inside every rank)", who, mode); return RFINV_ERR_ARG; }
+  if ((st = pt_require_settled(s, who)) != RFINV_OK) return st;
   RFINV_CUDA_CHECK(cudaSetDevice(h->device));
   RFINV_CUDA_CHECK(cudaStreamSynchronize(h->stream));
   if (mode == 1 && d.nchains >= 2 && !d.rs_nprop) {   // counters start at zero and survive later switches
@@ -1597,13 +1633,9 @@ int32_t rfinv_pt_set_rank_swaps(rfinv_handle* h, int32_t mode) {
   }
   pt_drop_graphs(s);   // the captured launch sequence depends on the mode
   s->rank_swaps = mode;
-  if (mode == 0 && d.rs_tune) {   // the ladder tuning works on the sweep's counters: it goes with it
-    s->tune_points_off = pt_tuning_points(s->it_done, d.nburn);
-    d.rs_tune = 0;
-  }
-  if (mode == 0 && d.st_on) {     // the step tuning works on the sweep's levels: likewise
-    s->step_points_off = pt_tuning_points(s->it_done, d.nburn);
-    d.st_on = 0;
+  if (mode == 0) {   // the tunings work on the sweep's counters and levels: they go with it
+    pt_ladder_tuning_off(s);
+    pt_step_tuning_off(s);
   }
   return RFINV_OK;
 }
@@ -1616,18 +1648,11 @@ int32_t rfinv_pt_set_step_tuning(rfinv_handle* h, int32_t on, double target) {
   PtDev& d = s->dev;
   if (on != 0 && on != 1) { rfinv_set_error("%s: %d (0: off, 1: tune the random-walk widths during the burn-in)", who, on); return RFINV_ERR_ARG; }
   if (!(target > 0.0 && target < 1.0)) { rfinv_set_error("%s: target %g is outside (0, 1)", who, target); return RFINV_ERR_ARG; }
-  if (s->step_pending) {
-    rfinv_set_error("%s: an iteration is half done (rfinv_pt_local_step without rfinv_pt_apply_swap)", who);
-    return RFINV_ERR_STATE;
-  }
-  if (s->reduced) { rfinv_set_error("%s: rfinv_pt_reduce_outputs has run", who); return RFINV_ERR_STATE; }
+  if ((st = pt_require_settled(s, who)) != RFINV_OK) return st;
   if (on) {
-    if (s->it_done > 0) {
-      rfinv_set_error("%s: %d iterations have run; the tuning starts with the run (before its first iteration or a restore)", who, s->it_done);
-      return RFINV_ERR_STATE;
-    }
+    if ((st = pt_require_fresh(s, who, "the tuning starts")) != RFINV_OK) return st;
     if (d.nchains < 2) { rfinv_set_error("%s: nchains = %d: the tuning needs levels, at least two chains per rank", who, d.nchains); return RFINV_ERR_ARG; }
-    if (s->rank_swaps != 1) { rfinv_set_error("%s: the tuning needs the rank swaps on (rfinv_pt_set_rank_swaps(h, 1) first)", who); return RFINV_ERR_STATE; }
+    if ((st = pt_require_rank_swaps(s, who)) != RFINV_OK) return st;
   }
   RFINV_CUDA_CHECK(cudaSetDevice(h->device));
   RFINV_CUDA_CHECK(cudaStreamSynchronize(h->stream));
@@ -1657,7 +1682,7 @@ int32_t rfinv_pt_set_step_tuning(rfinv_handle* h, int32_t on, double target) {
       }
     RFINV_CUDA_CHECK(cudaMemcpy(d.st_lvl, lvl.data(), sizeof(int) * lvl.size(), cudaMemcpyHostToDevice));
   }
-  if (!on && d.st_on) s->step_points_off = pt_tuning_points(s->it_done, d.nburn);
+  if (!on) pt_step_tuning_off(s);
   pt_drop_graphs(s);   // the captured launches carry the flag and the target
   d.st_on = on;
   if (on) d.st_target = target;
@@ -1698,17 +1723,10 @@ int32_t rfinv_pt_set_ladder_tuning(rfinv_handle* h, int32_t on) {
   PtState* s = h->pt;
   PtDev& d = s->dev;
   if (on != 0 && on != 1) { rfinv_set_error("%s: %d (0: off, 1: tune the ladders during the burn-in)", who, on); return RFINV_ERR_ARG; }
-  if (s->step_pending) {
-    rfinv_set_error("%s: an iteration is half done (rfinv_pt_local_step without rfinv_pt_apply_swap)", who);
-    return RFINV_ERR_STATE;
-  }
-  if (s->reduced) { rfinv_set_error("%s: rfinv_pt_reduce_outputs has run", who); return RFINV_ERR_STATE; }
+  if ((st = pt_require_settled(s, who)) != RFINV_OK) return st;
   if (on && !d.rs_tune) {
-    if (s->it_done > 0) {
-      rfinv_set_error("%s: %d iterations have run; the tuning starts with the run (before its first iteration or a restore)", who, s->it_done);
-      return RFINV_ERR_STATE;
-    }
-    if (s->rank_swaps != 1) { rfinv_set_error("%s: the tuning needs the rank swaps on (rfinv_pt_set_rank_swaps(h, 1) first)", who); return RFINV_ERR_STATE; }
+    if ((st = pt_require_fresh(s, who, "the tuning starts")) != RFINV_OK) return st;
+    if ((st = pt_require_rank_swaps(s, who)) != RFINV_OK) return st;
     // the kernel keeps a rank's ladder and its levels in shared memory
     if ((sizeof(int) + sizeof(double)) * (size_t)d.nchains > 200 * 1024) {
       rfinv_set_error("%s: nchains = %d is beyond the %d chains per rank the tuning supports", who, d.nchains, (int)(200 * 1024 / 12));
@@ -1719,7 +1737,7 @@ int32_t rfinv_pt_set_ladder_tuning(rfinv_handle* h, int32_t on) {
   RFINV_CUDA_CHECK(cudaStreamSynchronize(h->stream));
   if (on && d.nchains >= 2 && !d.rs_base)
     if ((st = dalloc(&d.rs_base, (size_t)d.G * (d.nchains - 1))) != RFINV_OK) return st;
-  if (!on && d.rs_tune) s->tune_points_off = pt_tuning_points(s->it_done, d.nburn);
+  if (!on) pt_ladder_tuning_off(s);
   pt_drop_graphs(s);   // the captured launches carry the flag
   d.rs_tune = on;
   return RFINV_OK;
@@ -1773,15 +1791,8 @@ int32_t rfinv_pt_set_diagnostics(rfinv_handle* h, int32_t on, int32_t n_bins, co
       rfinv_set_error("%s: depth bin %d is outside [1, nbin_z = %d]", who, vs_bins[j], d.nbin_z);
       return RFINV_ERR_ARG;
     }
-  if (s->step_pending) {
-    rfinv_set_error("%s: an iteration is half done (rfinv_pt_local_step without rfinv_pt_apply_swap)", who);
-    return RFINV_ERR_STATE;
-  }
-  if (s->reduced) { rfinv_set_error("%s: rfinv_pt_reduce_outputs has run", who); return RFINV_ERR_STATE; }
-  if (s->it_done > 0) {
-    rfinv_set_error("%s: %d iterations have run; the diagnostics start with the run (before its first iteration or a restore)", who, s->it_done);
-    return RFINV_ERR_STATE;
-  }
+  if ((st = pt_require_settled(s, who)) != RFINV_OK) return st;
+  if ((st = pt_require_fresh(s, who, "the diagnostics start")) != RFINV_OK) return st;
   if (on && !s->record) {
     rfinv_set_error("%s: the diagnostics record with the posterior bookkeeping, which is off (needs niter > 0 and all nbin_* > 0)", who);
     return RFINV_ERR_STATE;

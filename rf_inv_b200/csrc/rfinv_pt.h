@@ -162,6 +162,10 @@ constexpr int PT_DG_ROW = 9;
 struct rfinv_handle;
 int rfinv_pt_diag_rows(rfinv_handle* h, double* rows);
 
+// RFINV_OK when the state is this process's own and between iterations: not between rfinv_pt_local_step and
+// rfinv_pt_apply_swap, and not after rfinv_pt_reduce_outputs; else RFINV_ERR_STATE with the error set for `who`
+int pt_require_settled(const PtState* s, const char* who);
+
 // the tuning points e = 2^j, j >= 6, e <= nburn among the first it_done iterations (DESIGN.md 7d, 7e)
 inline int pt_tuning_points(int it_done, int nburn) {
   int n = 0;

@@ -38,6 +38,7 @@ from __future__ import annotations
 import argparse
 import os
 import sys
+from collections import namedtuple
 
 import numpy as np
 
@@ -159,6 +160,81 @@ def print_rank_swaps(rs) -> None:
         print(f" # of swaps between levels {l - 1} and {l}: {int(a)} / {int(n)} ({a / n if n else 0.0:.4f})")
 
 
+# the opt-in settings of a run (DESIGN.md 7c-7f), as run() takes them
+Settings = namedtuple("Settings", "rank_swaps tune_ladder tune_steps step_target diagnostics diag_depths")
+
+
+def checked_settings(checkpoint, checkpoint_every, resume, rank_swaps, tune_ladder, tune_steps, step_target, diagnostics,
+                     diag_depths) -> Settings:
+    """run()'s arguments checked, and the settings with the rank swaps that the tunings imply."""
+    if resume and not checkpoint:
+        raise ValueError("resume needs a checkpoint path")
+    if checkpoint_every is not None and checkpoint_every < 1:
+        raise ValueError("checkpoint_every must be at least 1")
+    return Settings(rank_swaps or tune_ladder or tune_steps, tune_ladder, tune_steps, step_target, diagnostics,
+                    tuple(diag_depths))
+
+
+def switch_on(pt, opt: Settings, bins) -> None:
+    """Switches the settings on, before a restore: the checkpoint holds their state.  bins: depth_bins of opt.diag_depths."""
+    if opt.rank_swaps:
+        pt.set_rank_swaps(1)
+    if opt.tune_ladder:
+        pt.set_ladder_tuning(1)
+    if opt.tune_steps:
+        pt.set_step_tuning(1, opt.step_target)
+    if opt.diagnostics:
+        pt.set_diagnostics(1, bins)
+
+
+def iterate(run_step, save, done: int, n_tot: int, ncorr: int, checkpoint_every, verbose: bool) -> None:
+    """Runs iterations done .. n_tot by run_step(n) with a progress line every N_CORR iterations (src/pt_mcmc.f90:489-491);
+    save(), if given, every `checkpoint_every` iterations (rounded up to the progress steps; default: every step) and at the end."""
+    step_len = max(ncorr, 1) * 100
+    every = step_len if checkpoint_every is None else checkpoint_every
+    saved = done
+    while done < n_tot:
+        step = min(step_len - done % step_len, n_tot - done)   # (a resumed run keeps the progress steps of a fresh one)
+        run_step(step)
+        done += step
+        if verbose:
+            print(f" Iteration #: {done} / {n_tot}", flush=True)
+        if save and (done - saved >= every or done == n_tot):   # always at the end
+            save()
+            saved = done
+
+
+def report(pt, cfg, nproc: int, opt: Settings, ladders, widths, write: bool, verbose: bool):
+    """Reads the results of pt (job-wide on process 0 after reduce_outputs) and, with `write`, prints them (verbose) and writes
+    the reference's output files and those of the settings into OUT_DIR.  ladders / widths: the rows of rank_ladders /
+    step_rows with the tunings on, else None.  Returns (hist, counters)."""
+    hist, cnt = pt.hist(), pt.counters()
+    vp_model, vs_model = pt.models()
+    rs = pt.rank_swaps() if opt.rank_swaps else None
+    diag = pt.diagnostics() if opt.diagnostics else None
+    if not write:
+        return hist, cnt
+    if verbose:
+        print_summary(cfg, hist, cnt)
+        if rs:
+            print_rank_swaps(rs)
+    rio.write_outputs(cfg, cfg.out_dir, nproc, hist, cnt["likelihood_hist"], vp_model, vs_model)
+    if rs:
+        write_rank_swaps(cfg.out_dir, rs)
+    if ladders is not None:
+        write_ladder(cfg.out_dir, ladders)
+    if widths is not None:
+        write_step_widths(cfg.out_dir, widths)
+    if diag is not None:
+        conv = convergence_rows(diag, opt.diag_depths)
+        if verbose:
+            print_convergence(conv)
+        write_convergence(cfg.out_dir, conv)
+        if rs:
+            write_round_trips(cfg.out_dir, diag["trips"])
+    return hist, cnt
+
+
 def run(params_path: str, nproc: int, verbose: bool = True, n_iter: int = None, checkpoint: str = None,
         checkpoint_every: int = None, resume: bool = False, rank_swaps: bool = False, tune_ladder: bool = False,
         tune_steps: bool = False, step_target: float = 0.44, diagnostics: bool = False, diag_depths=()):
@@ -170,13 +246,10 @@ def run(params_path: str, nproc: int, verbose: bool = True, n_iter: int = None, 
     (set_step_tuning(1, step_target)); adds OUT_DIR/step_widths.
     diagnostics: record the cold level and report convergence (set_diagnostics) at the depths diag_depths (km); adds
     OUT_DIR/convergence and, with rank_swaps, OUT_DIR/round_trips."""
-    rank_swaps = rank_swaps or tune_ladder or tune_steps
-    if resume and not checkpoint:
-        raise ValueError("resume needs a checkpoint path")
-    if checkpoint_every is not None and checkpoint_every < 1:
-        raise ValueError("checkpoint_every must be at least 1")
+    opt = checked_settings(checkpoint, checkpoint_every, resume, rank_swaps, tune_ladder, tune_steps, step_target, diagnostics,
+                           diag_depths)
     cfg = rio.load_problem(params_path)
-    bins = depth_bins(cfg, diag_depths) if diagnostics else []
+    bins = depth_bins(cfg, opt.diag_depths) if opt.diagnostics else []
     cfg.r_inv = workloads.lapack_r_inv(cfg)          # init_r_inv: LAPACK dgesvd like the reference
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
@@ -193,14 +266,7 @@ def run(params_path: str, nproc: int, verbose: bool = True, n_iter: int = None, 
         os.makedirs(cfg.out_dir, exist_ok=True)
         rio.write_side_copies(params_path, cfg.out_dir, os.path.dirname(os.path.abspath(params_path)))
     pt = ParallelTempering(cfg, nproc, device=local_rank, world=world, rank=rank)
-    if rank_swaps:                                        # before a restore: the checkpoint holds the sweep's counters
-        pt.set_rank_swaps(1)
-    if tune_ladder:
-        pt.set_ladder_tuning(1)
-    if tune_steps:
-        pt.set_step_tuning(1, step_target)
-    if diagnostics:
-        pt.set_diagnostics(1, bins)
+    switch_on(pt, opt, bins)
     n_tot = cfg.nburn + cfg.niter if n_iter is None else n_iter
     ck = checkpoint_path(checkpoint, world, rank) if checkpoint else None
     if resume:
@@ -217,57 +283,20 @@ def run(params_path: str, nproc: int, verbose: bool = True, n_iter: int = None, 
     done = pt.iterations_done
     if done > n_tot:
         raise ValueError(f"the checkpoint is at iteration {done}, beyond the {n_tot} iterations asked for")
-    step_len = max(cfg.ncorr, 1) * 100
-    every = step_len if checkpoint_every is None else checkpoint_every
-    saved = done
-    while done < n_tot:                                   # progress line every N_CORR iterations (src/pt_mcmc.f90:489-491)
-        step = min(step_len - done % step_len, n_tot - done)   # (a resumed run keeps the progress steps of a fresh one)
-        if world == 1:
-            pt.run(step)
-        else:
-            pt.run_distributed(step, dist, torch)
-        done += step
-        if verbose and rank == 0:
-            print(f" Iteration #: {done} / {n_tot}", flush=True)
-        if ck and (done - saved >= every or done == n_tot):   # always at the end
-            pt.save(ck)
-            saved = done
-    ladders = rank_ladders(pt) if tune_ladder else None
-    if tune_ladder and world > 1:                         # process 0 writes the rows of every process, in rank order
-        rows = [None] * world
-        dist.all_gather_object(rows, ladders)
-        ladders = np.concatenate(rows)
-    widths = step_rows(pt) if tune_steps else None
-    if tune_steps and world > 1:
-        rows = [None] * world
-        dist.all_gather_object(rows, widths)
-        widths = np.concatenate(rows)
+    iterate(pt.run if world == 1 else lambda n: pt.run_distributed(n, dist, torch), (lambda: pt.save(ck)) if ck else None,
+            done, n_tot, cfg.ncorr, checkpoint_every, verbose and rank == 0)
+
+    def gathered(rows):                                   # process 0 writes the rows of every process, in rank order
+        if rows is None or world == 1:
+            return rows
+        parts = [None] * world
+        dist.all_gather_object(parts, rows)
+        return np.concatenate(parts)
+    ladders = gathered(rank_ladders(pt) if opt.tune_ladder else None)
+    widths = gathered(step_rows(pt) if opt.tune_steps else None)
     if world > 1:                                         # the reference's mpi_reduce / mpi_gather (src/mcmc_out.f90:52-93)
         pt.reduce_outputs()                               # ncclReduce / ncclSend+Recv inside the library: process 0 is job-wide now
-    hist, cnt = pt.hist(), pt.counters()
-    vp_model, vs_model = pt.models()
-    rs = pt.rank_swaps() if rank_swaps else None
-    diag = pt.diagnostics() if diagnostics else None      # (job-wide on process 0 after reduce_outputs)
-    lh = cnt["likelihood_hist"]
-    if rank == 0:
-        if verbose:
-            print_summary(cfg, hist, cnt)
-            if rs:
-                print_rank_swaps(rs)
-        rio.write_outputs(cfg, cfg.out_dir, nproc, hist, lh, vp_model, vs_model)
-        if rs:
-            write_rank_swaps(cfg.out_dir, rs)
-        if ladders is not None:
-            write_ladder(cfg.out_dir, ladders)
-        if widths is not None:
-            write_step_widths(cfg.out_dir, widths)
-        if diag is not None:
-            conv = convergence_rows(diag, diag_depths)
-            if verbose:
-                print_convergence(conv)
-            write_convergence(cfg.out_dir, conv)
-            if rank_swaps:
-                write_round_trips(cfg.out_dir, diag["trips"])
+    hist, cnt = report(pt, cfg, nproc, opt, ladders, widths, rank == 0, verbose)
     pt.close()
     if world > 1:
         dist.destroy_process_group()
@@ -303,14 +332,11 @@ def run_group(params_paths, nproc: int, verbose: bool = True, n_iter: int = None
               tune_steps: bool = False, step_target: float = 0.44, diagnostics: bool = False, diag_depths=()):
     """Several stations (one params file each) as one group on one GPU; arguments as in run().  Under torchrun process r
     takes the stations i with i % world == r.  Returns {station index: (hist, counters)} of this process's stations."""
-    rank_swaps = rank_swaps or tune_ladder or tune_steps
-    if resume and not checkpoint:
-        raise ValueError("resume needs a checkpoint path")
-    if checkpoint_every is not None and checkpoint_every < 1:
-        raise ValueError("checkpoint_every must be at least 1")
+    opt = checked_settings(checkpoint, checkpoint_every, resume, rank_swaps, tune_ladder, tune_steps, step_target, diagnostics,
+                           diag_depths)
     params_paths = list(params_paths)
     cfgs = load_stations(params_paths)
-    bins = [depth_bins(c, diag_depths) if diagnostics else [] for c in cfgs]
+    bins = [depth_bins(c, opt.diag_depths) if opt.diagnostics else [] for c in cfgs]
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -330,16 +356,8 @@ def run_group(params_paths, nproc: int, verbose: bool = True, n_iter: int = None
         cfgs[i].r_inv = workloads.lapack_r_inv(cfgs[i])
     pts = [ParallelTempering(cfgs[i], nproc, device=local_rank) for i in mine]
     try:
-        if rank_swaps:
-            for pt in pts:
-                pt.set_rank_swaps(1)
-                if tune_ladder:
-                    pt.set_ladder_tuning(1)
-                if tune_steps:
-                    pt.set_step_tuning(1, step_target)
-        if diagnostics:
-            for i, pt in zip(mine, pts):
-                pt.set_diagnostics(1, bins[i])
+        for i, pt in zip(mine, pts):
+            switch_on(pt, opt, bins[i])
         if restore:
             for i, pt in zip(mine, pts):
                 pt.restore(cks[i])
@@ -350,46 +368,18 @@ def run_group(params_paths, nproc: int, verbose: bool = True, n_iter: int = None
         done = pts[0].iterations_done
         if done > n_tot:
             raise ValueError(f"the checkpoints are at iteration {done}, beyond the {n_tot} iterations asked for")
-        step_len = max(cfg0.ncorr, 1) * 100
-        every = step_len if checkpoint_every is None else checkpoint_every
-        saved = done
+
+        def save():
+            for i, pt in zip(mine, pts):
+                pt.save(cks[i])
         with PtGroup(pts) as group:
-            while done < n_tot:                           # the progress steps of run()
-                step = min(step_len - done % step_len, n_tot - done)
-                group.run(step)
-                done += step
-                if verbose:
-                    print(f" Iteration #: {done} / {n_tot}", flush=True)
-                if cks and (done - saved >= every or done == n_tot):
-                    for i, pt in zip(mine, pts):
-                        pt.save(cks[i])
-                    saved = done
+            iterate(group.run, save if cks else None, done, n_tot, cfg0.ncorr, checkpoint_every, verbose)
         out = {}
         for i, pt in zip(mine, pts):
-            cfg = cfgs[i]
-            hist, cnt = pt.hist(), pt.counters()
-            vp_model, vs_model = pt.models()
             if verbose:
                 print(f" === {params_paths[i]} ===")
-                print_summary(cfg, hist, cnt)
-                if rank_swaps:
-                    print_rank_swaps(pt.rank_swaps())
-            rio.write_outputs(cfg, cfg.out_dir, nproc, hist, cnt["likelihood_hist"], vp_model, vs_model)
-            if rank_swaps:
-                write_rank_swaps(cfg.out_dir, pt.rank_swaps())
-            if tune_ladder:
-                write_ladder(cfg.out_dir, rank_ladders(pt))
-            if tune_steps:
-                write_step_widths(cfg.out_dir, step_rows(pt))
-            if diagnostics:
-                diag = pt.diagnostics()
-                conv = convergence_rows(diag, diag_depths)
-                if verbose:
-                    print_convergence(conv)
-                write_convergence(cfg.out_dir, conv)
-                if rank_swaps:
-                    write_round_trips(cfg.out_dir, diag["trips"])
-            out[i] = (hist, cnt)
+            out[i] = report(pt, cfgs[i], nproc, opt, rank_ladders(pt) if opt.tune_ladder else None,
+                            step_rows(pt) if opt.tune_steps else None, True, verbose)
         return out
     finally:
         for pt in pts:
@@ -436,14 +426,13 @@ def main(argv=None):
         ap.error("--diag-depths takes depths in km separated by commas")
     if depths and not a.diagnostics:
         ap.error("--diag-depths needs --diagnostics")
+    kw = dict(n_iter=a.iters, checkpoint=a.checkpoint, checkpoint_every=a.checkpoint_every, resume=a.resume,
+              rank_swaps=a.rank_swaps, tune_ladder=a.tune_ladder, tune_steps=a.tune_steps, step_target=a.step_target,
+              diagnostics=a.diagnostics, diag_depths=depths)
     if len(a.params) == 1:
-        run(a.params[0], a.nproc, n_iter=a.iters, checkpoint=a.checkpoint, checkpoint_every=a.checkpoint_every, resume=a.resume,
-            rank_swaps=a.rank_swaps, tune_ladder=a.tune_ladder, tune_steps=a.tune_steps, step_target=a.step_target,
-            diagnostics=a.diagnostics, diag_depths=depths)
+        run(a.params[0], a.nproc, **kw)
     else:
-        run_group(a.params, a.nproc, n_iter=a.iters, checkpoint=a.checkpoint, checkpoint_every=a.checkpoint_every,
-                  resume=a.resume, rank_swaps=a.rank_swaps, tune_ladder=a.tune_ladder, tune_steps=a.tune_steps,
-                  step_target=a.step_target, diagnostics=a.diagnostics, diag_depths=depths)
+        run_group(a.params, a.nproc, **kw)
 
 
 if __name__ == "__main__":
