@@ -1379,6 +1379,17 @@ __global__ void __launch_bounds__(BMAX, MINB) forward_kernel(const DevConfig cfg
 #endif
     if (general) surface_groups<J, true, MIXED, GEN>(jm, s_rc, wa, wb, jfull, ipha, n, nh, tid, nthr, nullptr, s_buf, s_fr, s_fv, buried, s_tabw, psh, cfg.chirp, nf);
     else surface_groups<J, false, MIXED, GEN>(jm, s_rc, wa, wb, kPruned ? J : jfull, ipha, n, nh, tid, nthr, cfg.flt + (size_t)t0 * nh, s_buf, s_fr, s_fv, false, s_tabw, psh, cfg.chirp, nf);
+    if constexpr (kPruned && (J & 1) && nthr == 256) {
+      // The pruned first FFT stage skips only the legs of n/8 bins that lie wholly above the band limit.  J NT is a leg
+      // boundary at every shape but one: an odd J of 256 threads at nfft 4096 (legs of 512 bins) ends inside leg 1, whose
+      // bins from J NT + 1 to the leg boundary and their mirrors nobody else writes (bin J NT itself: surface_and_pack).
+      const int top = (J * nthr + (n >> 3) - 1) & ~((n >> 3) - 1);
+      if (!general)
+        for (int j = J * nthr + 1 + tid; j <= top; j += nthr) {
+          s_buf[fpad(j, psh)] = make_double2(0.0, 0.0);
+          s_buf[fpad(n - j, psh)] = make_double2(0.0, 0.0);
+        }
+    }
     __syncthreads();
     PHASE_MARK(3);
 
